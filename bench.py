@@ -6,6 +6,7 @@ MAD-shape, device-timed).
     python bench.py --impl reference --steps K --warmup W     # the reference's own eval_epoch on the box's host cores
     python bench.py --gpus N --scaling strong                 # BASELINE.json configs[3]: fixed MAD-test-scale set, LPT-sharded
     python bench.py --gpus N --workload stress                # BASELINE.json configs[4]: one 10-hour video, queries sharded
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also writes the last timed step's outputs as DIR/<name>.npy
 
 A step = one pass of the whole hot path (stages 0-3: adapter + window pre-filter + Moment-DETR on the top-k
 windows + proposal matching + fusion/NMS) over one synthetic MAD-shaped movie with all its queries.  Default
@@ -59,7 +60,15 @@ def parse_args():
                    help="stress: one 180 000-frame video replicated on every rank, --stress-queries queries sharded")
     p.add_argument("--stress-queries", type=int, default=10000)
     p.add_argument("--no-parity-pass", action="store_true", help="skip the fp32 parity-mode pass")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy, "
+                        "so that two builds can be compared output for output on the same seeded inputs")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        p.error("--dump-outputs writes the outputs of this project's path: not available with --impl reference")
+    return a
 
 
 def workload_name(cfg, args, frames):
@@ -270,6 +279,33 @@ def timed_steps(eng, dev_steps, steps, barrier, torch, profile=False):
     return ev0.elapsed_time(ev1), n_queries, out, prof, _lib.launch_count()
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out, path, limit=DUMP_LIMIT_BYTES):
+    """Writes the `GroundingOutput` of one step as `path/<field>.npy`: float32 fields as float32, the fp64 prediction rows
+    and the integer fields as float64 (exact).  Every field has one row per query in packed order; when together they
+    would exceed `limit` bytes, the same fixed seeded sample of rows is written for all of them, and its row indices as
+    `query_index.npy`."""
+    import dataclasses
+    arrays = {}
+    for f in dataclasses.fields(out):
+        t = getattr(out, f.name)
+        if t is not None:
+            a = t.cpu().numpy()
+            arrays[f.name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    n = arrays["nms"].shape[0]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        keep = int(n * limit // (total + 8 * n))
+        idx = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["query_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -336,6 +372,8 @@ def run_ours(args):
         clocks.mark_end()
     finally:
         clocks.__exit__(None, None, None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     ms_max = allreduce(ms, dist.ReduceOp.MAX if world > 1 else None)
     nq_all = allreduce(n_queries, dist.ReduceOp.SUM if world > 1 else None)
     value = nq_all / (ms_max / 1e3)
@@ -562,6 +600,8 @@ def run_strong(args, cfg, world, rank, dev, barrier, allreduce):
     host_nms = g_nms.cpu() if rank == 0 else None
     barrier()
     wall = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0 and host_steps:
+        dump_outputs(o, args.dump_outputs)
     wall_max = allreduce(wall, dist.ReduceOp.MAX if world > 1 else None)
     busy = torch.zeros(world, dtype=torch.float64, device=dev)
     busy[rank] = busy_ms
@@ -630,6 +670,8 @@ def run_stress(args, cfg, world, rank, dev, barrier, allreduce):
     barrier()
     wall_max = allreduce(time.perf_counter() - t0, dist.ReduceOp.MAX if world > 1 else None)
     dev_ms = allreduce(ev0.elapsed_time(ev1), dist.ReduceOp.MAX if world > 1 else None)
+    if args.dump_outputs and rank == 0 and qbs:
+        dump_outputs(o, args.dump_outputs)
     if rank == 0:
         nq_all = len(ds.queries)
         assert host.shape[0] == nq_all
