@@ -16,7 +16,7 @@ PREC_TC_SPLIT = 2  # cone_linear only: 3-product split-fp16 GEMM (fp32-class acc
 
 class ConeDims(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("v_dim", "t_dim", "hidden", "nheads", "ffn", "enc_layers", "dec_layers",
-                                         "num_queries", "max_v_l", "max_q_l")]
+                                         "num_queries", "max_v_l", "max_q_l", "m_dim")]
 
 
 class ConeError(RuntimeError):
@@ -41,6 +41,7 @@ SIGNATURES = {
     "cone_prepare_workspace_bytes": (_sz, [C.POINTER(ConeDims), _i64]),
     "cone_l2_normalize": (C.c_int, [_p, _p, _i64, _i32, _f32, _p]),
     "cone_video_prepare": (C.c_int, [_p, _p, _i64, _p, _p, _p, _sz, C.c_int, _p]),
+    "cone_video_prepare_motion": (C.c_int, [_p, _p, _i64, _p, _p, _sz, C.c_int, _p]),
     "cone_adapter": (C.c_int, [_p, _p, _p, _i64, C.c_int, _p, _sz, C.c_int, _p]),
     "cone_linear": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, C.c_int, _p, _p, _p, _sz, C.c_int, _p]),
     "cone_encoder_tail": (C.c_int, [_p, _i32, _p, _p, _i64, _p, _i32, _p, _sz, _p]),

@@ -12,9 +12,11 @@ import math
 
 @dataclasses.dataclass(frozen=True)
 class ConeConfig:
-    # feature dims (cone/config.py `--v_appear_feat_dim`, `--t_feat_dim`)
+    # feature dims (cone/config.py `--v_appear_feat_dim`, `--t_feat_dim`, `--v_motion_feat_dim`); a motion dim of 0
+    # means one feature source serves both roles (the reference's released configs)
     v_feat_dim: int = 256
     t_feat_dim: int = 768
+    v_motion_feat_dim: int = 0
     # model (cone/config.py:101-125)
     hidden_dim: int = 256
     nheads: int = 8
@@ -34,6 +36,11 @@ class ConeConfig:
     max_before_nms: int = 200
     max_after_nms: int = 5
     name: str = "ego4d"
+
+    @property
+    def motion_dim(self) -> int:
+        """Input width of `input_vid_proj`: the motion feature dim, `v_feat_dim` when no separate stream is set."""
+        return self.v_motion_feat_dim or self.v_feat_dim
 
     @property
     def stride(self) -> int:

@@ -124,9 +124,12 @@ struct cone_weights {
     const float* p(const std::string& name) const { return blob + off.at(name); }
 };
 
+// input width of input_vid_proj: the motion feature dim, which defaults to the appearance dim
+static int motion_dim(const cone_dims& c) { return c.m_dim > 0 ? c.m_dim : c.v_dim; }
+
 // the canonical order of cone_b200/weights.py::state_dict_shapes
 static void layout(const cone_dims& c, std::vector<std::pair<std::string, size_t>>& out) {
-    const size_t d = c.hidden, ff = c.ffn, dv = c.v_dim, dt = c.t_dim;
+    const size_t d = c.hidden, ff = c.ffn, dv = c.v_dim, dt = c.t_dim, dm = motion_dim(c);
     auto attn = [&](const std::string& p) {
         out.push_back({p + ".in_proj_weight", 3 * d * d});
         out.push_back({p + ".in_proj_bias", 3 * d});
@@ -168,7 +171,7 @@ static void layout(const cone_dims& c, std::vector<std::pair<std::string, size_t
     out.push_back({"class_embed.bias", 2});
     out.push_back({"query_embed.weight", (size_t)c.num_queries * d});
     const char* names[2] = {"input_txt_proj", "input_vid_proj"};
-    const size_t din[2] = {dt, dv};
+    const size_t din[2] = {dt, dm};
     for (int t = 0; t < 2; ++t) {
         for (int i = 0; i < 2; ++i) {
             const size_t k = i == 0 ? din[t] : d;
@@ -192,6 +195,7 @@ static int check_dims(const cone_dims* c) {
     CONE_REQUIRE(c->hidden == 256 && c->nheads == 8, "only hidden_dim 256 with 8 heads (head_dim 32) is built");
     CONE_REQUIRE(c->v_dim > 0 && c->v_dim % 16 == 0 && c->t_dim > 0 && c->t_dim % 16 == 0,
                  "feature dims must be positive multiples of 16");
+    CONE_REQUIRE(c->m_dim >= 0 && c->m_dim % 16 == 0, "motion feature dim must be 0 (= v_dim) or a positive multiple of 16");
     CONE_REQUIRE(c->ffn > 0 && c->ffn % 16 == 0, "dim_feedforward must be a multiple of 16");
     CONE_REQUIRE(c->enc_layers >= 1 && c->dec_layers >= 1 && c->enc_layers <= 8 && c->dec_layers <= 8, "1..8 layers");
     CONE_REQUIRE(c->num_queries >= 1 && c->num_queries <= 8, "1..8 moment slots");
@@ -201,7 +205,7 @@ static int check_dims(const cone_dims* c) {
 }
 
 extern "C" const char* cone_last_error(void) { return g_err; }
-extern "C" int cone_version(void) { return 1; }
+extern "C" int cone_version(void) { return 2; }
 extern "C" int64_t cone_launch_count(void) { return g_launches; }
 extern "C" void cone_launch_count_reset(void) { g_launches = 0; }
 
@@ -933,11 +937,23 @@ extern "C" int cone_l2_normalize(const float* x, float* out, int64_t rows, int32
 extern "C" size_t cone_prepare_workspace_bytes(const cone_dims* dims, int64_t n_frames) {
     if (check_dims(dims) != CONE_OK) return 0;
     Arena a(nullptr, 0);
-    a.get<float>(n_frames * dims->v_dim);  // xn
+    const int dm = motion_dim(*dims), dx = dims->v_dim > dm ? dims->v_dim : dm;
+    a.get<float>(n_frames * dx);           // xn: normalised appearance or motion rows
     a.get<float>(n_frames * dims->hidden); // adapter hidden
     a.get<float>(n_frames * dims->v_dim);  // adapted
-    plan_proj(a, n_frames, dims->v_dim, dims->hidden);
-    return a.used + tc_scratch_bytes(n_frames, dims->v_dim > dims->ffn ? dims->v_dim : dims->ffn);
+    plan_proj(a, n_frames, dm, dims->hidden);
+    return a.used + tc_scratch_bytes(n_frames, dx > dims->ffn ? dx : dims->ffn);
+}
+
+// rows per slab of the frame stage: n_frames halved until the slab's buffers fit the workspace
+static int64_t prepare_slab(const cone_dims& dm, int64_t n_frames, size_t workspace_bytes, const char* who) {
+    int64_t slab = n_frames;
+    while (slab > 1 && cone_prepare_workspace_bytes(&dm, slab) > workspace_bytes) slab = (slab + 1) / 2;
+    if (cone_prepare_workspace_bytes(&dm, slab) > workspace_bytes) {
+        set_error("%s: workspace of %zu bytes cannot hold one frame", who, workspace_bytes);
+        return -1;
+    }
+    return slab;
 }
 
 extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw, int64_t n_frames, float* ctx_out,
@@ -945,16 +961,15 @@ extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw
                                   void* stream) {
     CONE_REQUIRE(w && frames_raw, "null argument");
     CONE_TRY(check_prec(precision));
+    const cone_dims& dm = w->dims;
+    CONE_REQUIRE(vidproj_out == nullptr || motion_dim(dm) == dm.v_dim,
+                 "cone_video_prepare: the handle reads %d-d motion features: project them with cone_video_prepare_motion",
+                 motion_dim(dm));
     Ctx c{w, precision, (cudaStream_t)stream};
     CONE_TRY(ensure_tc(w, precision, c.s));
-    const cone_dims& dm = w->dims;
     // frames are processed in slabs sized to the workspace
-    int64_t slab = n_frames;
-    while (slab > 1 && cone_prepare_workspace_bytes(&dm, slab) > workspace_bytes) slab = (slab + 1) / 2;
-    if (cone_prepare_workspace_bytes(&dm, slab) > workspace_bytes) {
-        set_error("cone_video_prepare: workspace of %zu bytes cannot hold one frame", workspace_bytes);
-        return CONE_ERR_WORKSPACE;
-    }
+    const int64_t slab = prepare_slab(dm, n_frames, workspace_bytes, "cone_video_prepare");
+    if (slab < 0) return CONE_ERR_WORKSPACE;
     for (int64_t f0 = 0; f0 < n_frames; f0 += slab) {
         const int64_t n = (n_frames - f0) < slab ? (n_frames - f0) : slab;
         Arena a(workspace, workspace_bytes);
@@ -972,6 +987,31 @@ extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw
             CONE_TRY(l2norm_rows(ad, ctx_out + f0 * dm.v_dim, n, dm.v_dim, 0.f, c.s));
         }
         if (vidproj_out) CONE_TRY(input_proj(c, "input_vid_proj", x, n, dm.v_dim, vidproj_out + f0 * dm.hidden, pb));
+    }
+    return CONE_OK;
+}
+
+extern "C" int cone_video_prepare_motion(const cone_weights* w, const float* motion_raw, int64_t n_frames,
+                                         float* vidproj_out, void* workspace, size_t workspace_bytes, int precision,
+                                         void* stream) {
+    CONE_REQUIRE(w && motion_raw && vidproj_out, "null argument");
+    CONE_REQUIRE(n_frames >= 0, "cone_video_prepare_motion: n_frames=%lld", (long long)n_frames);
+    CONE_TRY(check_prec(precision));
+    Ctx c{w, precision, (cudaStream_t)stream};
+    CONE_TRY(ensure_tc(w, precision, c.s));
+    const cone_dims& dm = w->dims;
+    const int dmot = motion_dim(dm);
+    const int64_t slab = prepare_slab(dm, n_frames, workspace_bytes, "cone_video_prepare_motion");
+    if (slab < 0) return CONE_ERR_WORKSPACE;
+    for (int64_t f0 = 0; f0 < n_frames; f0 += slab) {
+        const int64_t n = (n_frames - f0) < slab ? (n_frames - f0) : slab;
+        Arena a(workspace, workspace_bytes);
+        float* xn = a.get<float>(n * dmot);
+        ProjBuffers pb = plan_proj(a, n, dmot, dm.hidden);
+        tc_set_scratch(w->tc, a.base ? a.base + a.used : nullptr, workspace_bytes > a.used ? workspace_bytes - a.used : 0);
+        // the dataloader normalises motion rows on the host (ego4d_mad_dataloader.py:284-292) before input_vid_proj
+        CONE_TRY(l2norm_rows(motion_raw + f0 * dmot, xn, n, dmot, 1e-5f, c.s));
+        CONE_TRY(input_proj(c, "input_vid_proj", xn, n, dmot, vidproj_out + f0 * dm.hidden, pb));
     }
     return CONE_OK;
 }
@@ -1143,7 +1183,7 @@ extern "C" size_t cone_workspace_bytes(const cone_dims* dims, int64_t n_windows,
     plan_match(a, *dims, n_windows, n_windows);
     a.get<float>(n_windows * lv * dims->hidden);
     a.get<float>(n_windows * lt * dims->hidden);
-    plan_proj(a, n_windows * lv, dims->v_dim, dims->hidden);
+    plan_proj(a, n_windows * lv, motion_dim(*dims), dims->hidden);
     plan_proj(a, n_windows * lt, dims->t_dim, dims->hidden);
     return a.used + tc_scratch_bytes(n_windows * (lv + lt), dims->ffn) + 4096;
 }
@@ -1277,14 +1317,14 @@ extern "C" int cone_forward(const cone_weights* w, const float* src_txt, const i
     CoreBuffers cb = plan_core(a, dm, B, Lv, Lt, precision);
     float* vidproj = a.get<float>((int64_t)B * Lv * dm.hidden);
     float* txtproj = a.get<float>((int64_t)B * Lt * dm.hidden);
-    ProjBuffers pv = plan_proj(a, (int64_t)B * Lv, dm.v_dim, dm.hidden);
+    ProjBuffers pv = plan_proj(a, (int64_t)B * Lv, motion_dim(dm), dm.hidden);
     ProjBuffers pt = plan_proj(a, (int64_t)B * Lt, dm.t_dim, dm.hidden);
     if (!a.fits()) {
         set_error("cone_forward: workspace needs %zu bytes, got %zu", a.used, workspace_bytes);
         return CONE_ERR_WORKSPACE;
     }
     tc_set_scratch(w->tc, a.base + a.used, workspace_bytes - a.used);
-    CONE_TRY(input_proj(c, "input_vid_proj", src_vid, (int64_t)B * Lv, dm.v_dim, vidproj, pv));
+    CONE_TRY(input_proj(c, "input_vid_proj", src_vid, (int64_t)B * Lv, motion_dim(dm), vidproj, pv));
     CONE_TRY(input_proj(c, "input_txt_proj", src_txt, (int64_t)B * Lt, dm.t_dim, txtproj, pt));
     CONE_TRY(fill_window_desc_dense(cb.vid_base, cb.txt_base, cb.qidx, B, Lv, Lt, c.s));
     CONE_CUDA(cudaMemcpyAsync(cb.vlen, vid_len, sizeof(int32_t) * B, cudaMemcpyDeviceToDevice, c.s));

@@ -148,7 +148,8 @@ class ConeEngine:
         self.device = torch.device(device)
         self.precision = {"fp32": _lib.PREC_FP32, "tc": _lib.PREC_TC, "bf16": _lib.PREC_TC}[precision]
         self.dims = _lib.ConeDims(cfg.v_feat_dim, cfg.t_feat_dim, cfg.hidden_dim, cfg.nheads, cfg.dim_feedforward,
-                                  cfg.enc_layers, cfg.dec_layers, cfg.num_queries, cfg.max_v_l, cfg.max_q_l)
+                                  cfg.enc_layers, cfg.dec_layers, cfg.num_queries, cfg.max_v_l, cfg.max_q_l,
+                                  cfg.v_motion_feat_dim)
         self._handle = C.c_void_p(0)
         self._ws = None
         with torch.cuda.device(self.device):
@@ -238,16 +239,37 @@ class ConeEngine:
                                         _ptr(residual), _ptr(y), ws, nb, prec, _stream()), "cone_linear")
         return y
 
-    def video_prepare(self, frames: torch.Tensor, want_ctx=True, want_vidproj=True):
-        """Stage 0 + per-frame `input_vid_proj` over concatenated frames [n, Dv] (raw features)."""
+    def video_prepare(self, frames: torch.Tensor, want_ctx=True, want_vidproj=True, motion: Optional[torch.Tensor] = None):
+        """Stage 0 + per-frame `input_vid_proj` over concatenated frames [n, Dv] (raw appearance features).
+        `motion` [n, Dm]: raw features of a separate motion stream, one row per appearance row; `input_vid_proj` then
+        reads them L2-normalised (ego4d_mad_dataloader.py:284-292).  Without it the appearance rows are projected
+        raw, which is only valid when the model's motion dim is Dv."""
         frames = _need(frames, torch.float32, "frames")
         n = frames.shape[0]
+        if motion is not None:
+            motion = self._check_motion(motion, n)
+        elif want_vidproj and self.cfg.motion_dim != self.cfg.v_feat_dim:
+            raise ValueError(f"the model reads {self.cfg.motion_dim}-d motion features: pass `motion` [n_frames, "
+                             f"{self.cfg.motion_dim}] (appearance rows are {self.cfg.v_feat_dim}-d)")
         ctx = torch.empty_like(frames) if want_ctx else None
         vp = torch.empty((n, self.cfg.hidden_dim), dtype=torch.float32, device=frames.device) if want_vidproj else None
         ws, nb = self._wsargs()
-        _lib.check(self.lib.cone_video_prepare(self._handle, _ptr(frames), n, _ptr(ctx), _ptr(vp), ws, nb,
-                                               self.precision, _stream()), "cone_video_prepare")
+        _lib.check(self.lib.cone_video_prepare(self._handle, _ptr(frames), n, _ptr(ctx),
+                                               _ptr(vp if motion is None else None), ws, nb, self.precision, _stream()),
+                   "cone_video_prepare")
+        if motion is not None and want_vidproj:
+            _lib.check(self.lib.cone_video_prepare_motion(self._handle, _ptr(motion), n, _ptr(vp), ws, nb, self.precision,
+                                                          _stream()), "cone_video_prepare_motion")
         return ctx, vp
+
+    def _check_motion(self, motion: torch.Tensor, n_frames: int) -> torch.Tensor:
+        """Both streams are sliced with the same window bounds (ego4d_mad_dataloader.py:144-159): a motion tensor of
+        another length is refused rather than truncated."""
+        motion = _need(motion, torch.float32, "motion")
+        if motion.dim() != 2 or motion.shape != (n_frames, self.cfg.motion_dim):
+            raise ValueError(f"motion must be [{n_frames}, {self.cfg.motion_dim}] (one row per appearance frame), "
+                             f"got {tuple(motion.shape)}")
+        return motion
 
     def frame_scores(self, ctx: torch.Tensor, qb: QueryBatch, cls_norm: torch.Tensor):
         """`einsum('db,b->d')` of every query against its own video (cone/inference.py:284) as one grouped
@@ -398,12 +420,15 @@ class ConeEngine:
         return hits
 
     # ---- the whole path -------------------------------------------------------------------------
-    def ground(self, frames: torch.Tensor, qb: QueryBatch, want_rows: bool = False, prepared=None) -> GroundingOutput:
+    def ground(self, frames: torch.Tensor, qb: QueryBatch, want_rows: bool = False, prepared=None,
+               motion: Optional[torch.Tensor] = None) -> GroundingOutput:
         """Stages 0-3 for concatenated raw `frames` [n_frames, Dv] and the packed queries `qb` (both on the
         device).  No host synchronisation inside: sizes come from host metadata in `qb`.
-        `prepared` = (ctx, vidproj) from an earlier `video_prepare(frames)`: stage 0 is per VIDEO
+        `motion` [n_frames, Dm]: raw features of a separate motion stream (`--motion_feat_dir`), concatenated like
+        `frames`; stages 0/1 and the matching pool keep reading `frames`, Moment-DETR reads the motion rows.
+        `prepared` = (ctx, vidproj) from an earlier `video_prepare(frames, motion=motion)`: stage 0 is per VIDEO
         (cone/inference.py:241-260 runs it once per video before any query), so a long video whose queries are
-        processed in several calls (BASELINE.json configs[4]) pays for it once."""
+        processed in several calls (BASELINE.json configs[4]) pays for it once; `motion` is then not read."""
         cfg = self.cfg
         frames = _need(frames, torch.float32, "frames")
         dev = frames.device
@@ -411,7 +436,7 @@ class ConeEngine:
         k = cfg.topk_window
         ns = cfg.num_queries
         # stage 0: context features and per-frame video projection
-        ctx, vidproj = prepared if prepared is not None else self.video_prepare(frames)
+        ctx, vidproj = prepared if prepared is not None else self.video_prepare(frames, motion=motion)
         # host-side normalisations of the reference's dataset code, on the device
         cls_norm = self.l2_normalize(qb.cls, 1e-5)  # dataloader:472 / :280
         tok_norm = self.l2_normalize(qb.tokens, 1e-5)  # dataloader:274-276 (zero pad rows stay zero)

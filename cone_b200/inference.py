@@ -21,9 +21,10 @@ class HostStep:
     frames: torch.Tensor  # [n_frames, Dv] fp32 pinned
     qb: QueryBatch  # pinned
     video_ids: List[int]
+    motion: Optional[torch.Tensor] = None  # [n_frames, Dm] fp32 pinned: separate motion stream, None = `frames`
 
     def h2d_bytes(self) -> int:
-        return self.frames.numel() * 4 + self.qb.h2d_bytes()
+        return self.frames.numel() * 4 + self.qb.h2d_bytes() + (self.motion.numel() * 4 if self.motion is not None else 0)
 
 
 def plan_steps(video_lengths: Sequence[int], queries, max_frames_per_step: int) -> List[List[int]]:
@@ -40,18 +41,27 @@ def plan_steps(video_lengths: Sequence[int], queries, max_frames_per_step: int) 
     return steps
 
 
-def stage_step(cfg: ConeConfig, videos: Sequence[np.ndarray], queries, video_ids: Sequence[int], pin: bool = True) -> HostStep:
-    """Concatenate the step's videos and pack its queries (dataset order preserved within the step)."""
+def stage_step(cfg: ConeConfig, videos: Sequence[np.ndarray], queries, video_ids: Sequence[int], pin: bool = True,
+               motion_videos: Optional[Sequence[np.ndarray]] = None) -> HostStep:
+    """Concatenate the step's videos (and their motion features, when a separate motion stream is given) and pack
+    its queries (dataset order preserved within the step)."""
     vid_set = {v: i for i, v in enumerate(video_ids)}
     sel = [(i, q) for i, q in enumerate(queries) if q.video_idx in vid_set]
     local = [dataclasses.replace(q, video_idx=vid_set[q.video_idx]) for _, q in sel]
     lens = [len(videos[v]) for v in video_ids]
     frames = torch.from_numpy(np.concatenate([videos[v] for v in video_ids], axis=0))
+    motion = None
+    if motion_videos is not None:
+        for v in video_ids:  # both streams are sliced with the same window bounds: no silent truncation
+            if len(motion_videos[v]) != len(videos[v]):
+                raise ValueError(f"video {v}: {len(motion_videos[v])} motion rows for {len(videos[v])} appearance rows")
+        motion = torch.from_numpy(np.concatenate([motion_videos[v] for v in video_ids], axis=0))
     qb = pack_queries(cfg, lens, local, dataset_indices=[i for i, _ in sel])
     if pin and torch.cuda.is_available():
         frames = frames.pin_memory()
+        motion = motion.pin_memory() if motion is not None else None
         qb = qb.pin()
-    return HostStep(frames, qb, list(video_ids))
+    return HostStep(frames, qb, list(video_ids), motion)
 
 
 def run_step(engine: ConeEngine, step: HostStep, want_rows: bool = False) -> GroundingOutput:
@@ -59,8 +69,9 @@ def run_step(engine: ConeEngine, step: HostStep, want_rows: bool = False) -> Gro
     dev = engine.device
     with torch.cuda.device(dev):
         frames = step.frames.to(dev, non_blocking=True)
+        motion = step.motion.to(dev, non_blocking=True) if step.motion is not None else None
         qb = step.qb.to(dev)
-        return engine.ground(frames, qb, want_rows=want_rows)
+        return engine.ground(frames, qb, want_rows=want_rows, motion=motion)
 
 
 def output_to_host(cfg: ConeConfig, step: HostStep, out: GroundingOutput, full: bool = True) -> Dict[str, dict]:
@@ -90,20 +101,28 @@ def output_to_host(cfg: ConeConfig, step: HostStep, out: GroundingOutput, full: 
 
 
 def ground_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, max_frames_per_step: int = 1 << 20,
-                   full: bool = True, want_rows: bool = True) -> Dict[str, dict]:
+                   full: bool = True, want_rows: bool = True,
+                   motion_videos: Optional[Sequence[np.ndarray]] = None) -> Dict[str, dict]:
     """Stages 0-3 over a whole in-memory dataset.  Videos are processed in steps of consecutive videos; the
     reference pools proposals over windows padded to the longest window of each `eval_bsz` batch of queries
     (SURVEY.md §8 A9), which is reproduced exactly when a step holds whole eval batches (always true for a
-    single step)."""
+    single step).  `motion_videos[v]` [L_v, Dm]: raw features of a separate motion stream (`--motion_feat_dir`), the
+    input of Moment-DETR; None = the appearance features serve both roles."""
+    _check_streams(videos, motion_videos)
     res: Dict[str, dict] = {}
     lens = [len(v) for v in videos]
     for ids in plan_steps(lens, queries, max_frames_per_step):
-        step = stage_step(engine.cfg, videos, queries, ids)
+        step = stage_step(engine.cfg, videos, queries, ids, motion_videos=motion_videos)
         if step.qb.tok_len.numel() == 0:
             continue
         out = run_step(engine, step, want_rows=want_rows)
         res.update(output_to_host(engine.cfg, step, out, full=full))
     return res
+
+
+def _check_streams(videos, motion_videos) -> None:
+    if motion_videos is not None and len(motion_videos) != len(videos):
+        raise ValueError(f"{len(motion_videos)} motion feature tensors for {len(videos)} videos")
 
 
 def to_submission(results: Dict[str, dict], annotations: Sequence[dict], mode: str = "fusion") -> List[dict]:
@@ -184,8 +203,11 @@ def accumulate_metrics(engine: ConeEngine, counters: MetricCounters, step: HostS
 
 def evaluate_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, gt: Dict[str, Sequence[float]],
                      flavour: str = "mad", topk=(1, 5), thresholds=(0.3, 0.5), window_topk=(1, 5, 10, 30, 50),
-                     max_frames_per_step: int = 1 << 20, video_ids: Optional[Sequence[int]] = None) -> MetricCounters:
-    """Stages 0-3 + metric counters over (this rank's share of) a dataset; only the counters are read back."""
+                     max_frames_per_step: int = 1 << 20, video_ids: Optional[Sequence[int]] = None,
+                     motion_videos: Optional[Sequence[np.ndarray]] = None) -> MetricCounters:
+    """Stages 0-3 + metric counters over (this rank's share of) a dataset; only the counters are read back.
+    `motion_videos` as in `ground_dataset`."""
+    _check_streams(videos, motion_videos)
     counters = new_counters(engine.device, topk, thresholds, window_topk)
     lens = [len(v) for v in videos]
     mine = None if video_ids is None else set(video_ids)
@@ -193,7 +215,7 @@ def evaluate_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, 
         ids = [v for v in ids if mine is None or v in mine]
         if not ids:
             continue
-        step = stage_step(engine.cfg, videos, queries, ids)
+        step = stage_step(engine.cfg, videos, queries, ids, motion_videos=motion_videos)
         if step.qb.tok_len.numel() == 0:
             continue
         out = run_step(engine, step)

@@ -115,8 +115,11 @@ class StagedSteps:
     SURVEY.md §8 A1)."""
 
     def __init__(self, cfg: ConeConfig, video_store, video_ids: Sequence[str], video_lengths: Sequence[int], queries,
-                 max_frames_per_step: int = 1 << 20, depth: int = 2, pin: bool = True):
+                 max_frames_per_step: int = 1 << 20, depth: int = 2, pin: bool = True, motion_store=None):
+        """`motion_store`: records of a separate motion stream under the same keys (`--motion_feat_dir`); None = the
+        appearance records serve both roles."""
         self.cfg, self.store, self.video_ids, self.queries, self.pin = cfg, video_store, list(video_ids), queries, pin
+        self.motion_store = motion_store
         self.plan = plan_steps(video_lengths, queries, max_frames_per_step)
         self._q: "queue.Queue" = queue.Queue(maxsize=max(1, depth))
         self._stop = threading.Event()
@@ -140,7 +143,9 @@ class StagedSteps:
                     return
                 # stage_step only indexes videos[v] for v in ids: a dict of this step's decoded arrays is enough
                 vids: Dict[int, np.ndarray] = {v: decode_video_record(self.store.get(self.video_ids[v])) for v in ids}
-                step = stage_step(self.cfg, vids, self.queries, ids, pin=self.pin)
+                mot = None if self.motion_store is None else \
+                    {v: decode_video_record(self.motion_store.get(self.video_ids[v])) for v in ids}
+                step = stage_step(self.cfg, vids, self.queries, ids, pin=self.pin, motion_videos=mot)
                 if not self._put(step):
                     return
             self._put(None)
@@ -177,10 +182,12 @@ class StagedSteps:
 
 
 def ground_store(engine, video_store, query_store, annotations: Sequence[dict], video_lengths: Optional[Dict[str, int]] = None,
-                 max_frames_per_step: int = 1 << 20, full: bool = False) -> Dict[str, dict]:
+                 max_frames_per_step: int = 1 << 20, full: bool = False, motion_store=None) -> Dict[str, dict]:
     """`eval_epoch` stages 0-3 straight from feature stores: decode -> pinned -> HBM -> kernels, the decoding of the
     next step overlapping the kernels of the current one.  `video_lengths` (frames per clip_id) avoids a first pass
-    over the video records when the annotations do not carry it."""
+    over the video records when the annotations do not carry it.  `motion_store` holds the records of a separate
+    motion stream (`--motion_feat_dir`) under the same clip ids, `features [L, Dm]`; None = the reference's
+    same-directory case."""
     from .inference import output_to_host, run_step
     clip_ids = list(dict.fromkeys(a["clip_id"] for a in annotations))
     index = {c: i for i, c in enumerate(clip_ids)}
@@ -189,7 +196,7 @@ def ground_store(engine, video_store, query_store, annotations: Sequence[dict], 
     queries = load_queries(query_store, annotations, index)
     res: Dict[str, dict] = {}
     steps = StagedSteps(engine.cfg, video_store, clip_ids, [video_lengths[c] for c in clip_ids], queries,
-                        max_frames_per_step)
+                        max_frames_per_step, motion_store=motion_store)
     for step in steps:
         if step.qb.tok_len.numel() == 0:
             continue

@@ -52,6 +52,10 @@ class CONELocalizator:
                  use_cuda_graph: bool = True):
         """`load_checkpoint_path`: a checkpoint file holding {"model": state_dict} as the reference loads it
         (cone_localizator.py:75-76), or the state dict itself."""
+        if cfg.motion_dim != cfg.v_feat_dim:
+            raise NotImplementedError("the single-video front end reads one feature stream for every role "
+                                      "(run_on_video/cone_localizator.py:127-165); a model with a separate motion "
+                                      "stream runs through ConeEngine.ground / inference.ground_dataset")
         if isinstance(load_checkpoint_path, str):
             sd = torch.load(load_checkpoint_path, map_location="cpu")["model"]
         else:

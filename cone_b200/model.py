@@ -100,7 +100,7 @@ class CONE(nn.Module):
     # ---- reference surface ------------------------------------------------------------------------
     @torch.no_grad()
     def forward(self, src_txt, src_txt_mask, src_vid_motion, src_vid_motion_mask):
-        """cone/model.py:82-128.  Returns pred_logits (B,nq,2), pred_spans (B,nq,2), saliency_scores (B,L_vid)
+        """cone/model.py:82-128; `src_vid_motion` is [B, L_vid, v_motion_feat_dim].  Returns pred_logits (B,nq,2), pred_spans (B,nq,2), saliency_scores (B,L_vid)
         and, with aux_loss, aux_outputs."""
         if self.training:
             raise NotImplementedError("cone_b200.CONE is inference-only: call model.eval() first")
@@ -137,7 +137,8 @@ def config_from_opt(opt) -> ConeConfig:
     """The fields `build_model` reads from the argparse namespace (cone/model.py:477-518)."""
     g = lambda k, d: getattr(opt, k, d)
     return ConeConfig(
-        v_feat_dim=opt.v_appear_feat_dim, t_feat_dim=opt.t_feat_dim, hidden_dim=g("hidden_dim", 256),
+        v_feat_dim=opt.v_appear_feat_dim, t_feat_dim=opt.t_feat_dim,
+        v_motion_feat_dim=g("v_motion_feat_dim", 0), hidden_dim=g("hidden_dim", 256),
         nheads=g("nheads", 8), dim_feedforward=g("dim_feedforward", 1024), enc_layers=g("enc_layers", 2),
         dec_layers=g("dec_layers", 2), num_queries=g("num_queries", 5), n_input_proj=g("n_input_proj", 2),
         max_v_l=g("max_v_l", 90), max_q_l=g("max_q_l", 20), clip_length=g("clip_length", 1.0),
@@ -147,9 +148,6 @@ def config_from_opt(opt) -> ConeConfig:
 
 def build_model(args):
     """Same signature and return as the reference `build_model(args) -> (model, criterion)` (cone/model.py:468)."""
-    if getattr(args, "v_motion_feat_dim", args.v_appear_feat_dim) != args.v_appear_feat_dim:
-        raise NotImplementedError("distinct motion/appearance features are not built (the reference's released "
-                                  "configs use one feature for both, ego4d_mad_dataloader.py:62-70)")
     if getattr(args, "span_loss_type", "l1") != "l1" or getattr(args, "use_txt_pos", False) or getattr(args, "pre_norm", False):
         raise NotImplementedError("only span_loss_type='l1', use_txt_pos=False, pre_norm=False are built")
     model = CONE(config_from_opt(args), adapter_module=getattr(args, "adapter_module", "linear"),

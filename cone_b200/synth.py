@@ -8,7 +8,7 @@ per video a raw frame-feature matrix `features [L, Dv]`; per query `token_featur
 from __future__ import annotations
 
 import dataclasses
-from typing import List, Sequence, Tuple, Union
+from typing import List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 
@@ -29,6 +29,7 @@ class SynthDataset:
     cfg: ConeConfig
     videos: List[np.ndarray]  # each [L_v, Dv] float32, raw
     queries: List[SynthQuery]  # grouped by video, in video order
+    motion: Optional[List[np.ndarray]] = None  # each [L_v, Dm] float32, raw: a separate motion stream
 
     @property
     def video_ids(self) -> List[str]:
@@ -45,9 +46,11 @@ class SynthDataset:
 
 def make_dataset(cfg: ConeConfig, n_videos: int, frames: Union[int, Sequence[int], None],
                  queries_per_video: Union[int, Sequence[int]], seed: int = 0, plant: float = 0.5,
-                 id_offset: int = 0, frames_range: Union[Tuple[int, int], None] = None) -> SynthDataset:
+                 id_offset: int = 0, frames_range: Union[Tuple[int, int], None] = None,
+                 motion_dim: Optional[int] = None) -> SynthDataset:
     """`frames`: one L for every video or an explicit per-video list; or `frames_range=(lo, hi)`
-    to draw each video's length uniformly."""
+    to draw each video's length uniformly.  `motion_dim`: also draw a separate motion stream of that width, same
+    lengths, from its own generator (the appearance features and queries do not change)."""
     rng = np.random.default_rng(seed)
     if frames_range is not None:
         lens = [int(x) for x in rng.integers(frames_range[0], frames_range[1] + 1, size=n_videos)]
@@ -81,4 +84,10 @@ def make_dataset(cfg: ConeConfig, n_videos: int, frames: Union[int, Sequence[int
                 x[f0:f1] += np.float32(plant) * cls[None, :]
             queries.append(SynthQuery(f"v{v + id_offset:05d}_{j}", v, tok, cls, (st, ed)))
         videos.append(x)
-    return SynthDataset(cfg, videos, queries)
+    motion = None
+    if motion_dim:
+        mrng = np.random.default_rng([seed, 1])
+        # a per-video offset and scale: the motion rows are not centred like the appearance rows
+        motion = [(mrng.standard_normal((len(x), motion_dim), dtype=np.float32) * np.float32(mrng.uniform(0.5, 3.0))
+                   + np.float32(mrng.uniform(-0.5, 0.5))) for x in videos]
+    return SynthDataset(cfg, videos, queries, motion)

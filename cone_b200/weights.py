@@ -57,7 +57,8 @@ def state_dict_shapes(cfg: ConeConfig) -> "OrderedDict[str, tuple]":
     s["class_embed.weight"] = (2, d)  # model.py:50
     s["class_embed.bias"] = (2,)
     s["query_embed.weight"] = (cfg.num_queries, d)  # model.py:54
-    for name, din in (("input_txt_proj", dt), ("input_vid_proj", dv)):  # model.py:57-72
+    # model.py:57-72; input_vid_proj reads the motion features (`--v_motion_feat_dim`), the adapter the appearance ones
+    for name, din in (("input_txt_proj", dt), ("input_vid_proj", cfg.motion_dim)):
         for i in range(cfg.n_input_proj):
             k = din if i == 0 else d
             s[f"{name}.{i}.LayerNorm.weight"] = (k,)

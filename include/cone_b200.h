@@ -54,6 +54,8 @@ typedef struct cone_dims {
     int32_t num_queries; /* 5 moment slots per window                    --num_queries       */
     int32_t max_v_l;     /* window length in frames                      --max_v_l           */
     int32_t max_q_l;     /* max text tokens                              --max_q_l           */
+    int32_t m_dim;       /* Dm: motion feature dim, the input width of   --v_motion_feat_dim
+                            input_vid_proj; 0 = Dv (one feature source for both roles) */
 } cone_dims;
 
 typedef struct cone_weights cone_weights; /* opaque: packed state dict + derived tables, on device */
@@ -78,7 +80,7 @@ size_t cone_weights_expected_floats(const cone_dims* dims);
 /* ---- workspace sizing ---------------------------------------------------------------------- */
 /* bytes needed by cone_ground_windows / cone_forward for `n_windows` windows in flight */
 size_t cone_workspace_bytes(const cone_dims* dims, int64_t n_windows, int32_t lv, int32_t lt);
-/* bytes needed by cone_video_prepare for `n_frames` rows in flight */
+/* bytes needed by cone_video_prepare / cone_video_prepare_motion for `n_frames` rows in flight */
 size_t cone_prepare_workspace_bytes(const cone_dims* dims, int64_t n_frames);
 
 /* ---- A1  host L2 normalisation: x / (||x|| + eps)  (utils/basic_utils.py:97-99, applied at
@@ -90,9 +92,18 @@ int cone_l2_normalize(const float* x, float* out, int64_t rows, int32_t dim, flo
 /* ---- A2  stage 0 (cone/inference.py:250-260) + per-frame `input_vid_proj` (cone/model.py:100).
  * frames_raw [n_frames, Dv] raw features.  ctx_out [n_frames, Dv] = normalised adapted context
  * features; vidproj_out [n_frames, d] = input_vid_proj(raw) — the reference recomputes this per
- * window (A6); it is row-wise so it is computed once per frame here.  Either output may be NULL. */
+ * window (A6); it is row-wise so it is computed once per frame here.  Either output may be NULL.
+ * Raw appearance rows are the motion input only when one feature source serves both roles: on a handle with
+ * m_dim != v_dim a non-NULL vidproj_out is CONE_ERR_INVALID (use cone_video_prepare_motion). */
 int cone_video_prepare(const cone_weights* w, const float* frames_raw, int64_t n_frames, float* ctx_out,
                        float* vidproj_out, void* workspace, size_t workspace_bytes, int precision, void* stream);
+
+/* Per-frame `input_vid_proj` of a separate motion stream (--motion_feat_dir): motion_raw [n_frames, Dm] raw features
+ * are L2-normalised per frame, x / (||x|| + 1e-5) (cone/ego4d_mad_dataloader.py:284-292), then projected:
+ * vidproj_out [n_frames, d], the `vidproj` of cone_ground_windows.  Frames run in slabs sized to the workspace
+ * (cone_prepare_workspace_bytes); the result does not depend on the slab size. */
+int cone_video_prepare_motion(const cone_weights* w, const float* motion_raw, int64_t n_frames, float* vidproj_out,
+                              void* workspace, size_t workspace_bytes, int precision, void* stream);
 
 /* `adapter_layer(x) + x` on arbitrary rows (cone/model.py:80; inference.py:255): the
  * `model.adapter_layer` attribute of the drop-in surface. `residual` = 1 adds x. */
@@ -154,7 +165,8 @@ int cone_prefilter(const cone_weights* w, const float* frames_raw, int64_t n_fra
 /* ---- A4-A9  stage 2: slice the top-k windows of every query straight out of the frame tensors,
  * run Moment-DETR on them and score the proposals (cone/ego4d_mad_dataloader.py:144-159, 305-358;
  * cone/model.py:82-152; cone/inference.py:46-52).
- *   frames_raw [n_frames, Dv], vidproj [n_frames, d]  (from cone_video_prepare)
+ *   frames_raw [n_frames, Dv] raw appearance rows (pooled for matching), vidproj [n_frames, d] projected motion rows
+ *       (from cone_video_prepare, or cone_video_prepare_motion for a separate motion stream)
  *   q_video_start / q_video_len [n_queries]  frame offset and length of each query's video
  *   ranklist [n_queries, ranklist_stride]    from cone_window_ranklist
  *   tok [n_queries, max_q_l, Dt] L2-normalised tokens, zero padded; tok_len [n_queries]
@@ -174,7 +186,7 @@ int cone_ground_windows(const cone_weights* w, const float* frames_raw, int64_t 
                         void* workspace, size_t workspace_bytes, int precision, void* stream);
 
 /* ---- A6-A8  reference-shaped forward: `model(src_txt, src_txt_mask, src_vid_motion,
- * src_vid_motion_mask)` (cone/model.py:82-128).  src_vid [B, Lv, Dv], src_txt [B, Lt, Dt], valid
+ * src_vid_motion_mask)` (cone/model.py:82-128).  src_vid [B, Lv, Dm] (= src_vid_motion), src_txt [B, Lt, Dt], valid
  * lengths vid_len / txt_len [B] int32.  Outputs: pred_logits [B,nq,2], pred_spans [B,nq,2];
  * nullable: saliency [B,Lv], aux_logits / aux_spans [dec_layers-1, B, nq, 2]. */
 int cone_forward(const cone_weights* w, const float* src_txt, const int32_t* txt_len, const float* src_vid,
