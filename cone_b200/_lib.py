@@ -13,6 +13,11 @@ PREC_FP32 = 0
 PREC_TC = 1
 PREC_TC_SPLIT = 2  # cone_linear only: 3-product split-fp16 GEMM (fp32-class accuracy on the tensor pipe)
 
+# storage type of a raw feature tensor passed to the _ex entry points
+DTYPE_F32 = 0
+DTYPE_F16 = 1
+DTYPE_BF16 = 2
+
 
 class ConeDims(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("v_dim", "t_dim", "hidden", "nheads", "ffn", "enc_layers", "dec_layers",
@@ -40,8 +45,11 @@ SIGNATURES = {
     "cone_workspace_bytes": (_sz, [C.POINTER(ConeDims), _i64, _i32, _i32]),
     "cone_prepare_workspace_bytes": (_sz, [C.POINTER(ConeDims), _i64]),
     "cone_l2_normalize": (C.c_int, [_p, _p, _i64, _i32, _f32, _p]),
+    "cone_l2_normalize_ex": (C.c_int, [_p, _i32, _p, _i64, _i32, _f32, _p]),
     "cone_video_prepare": (C.c_int, [_p, _p, _i64, _p, _p, _p, _sz, C.c_int, _p]),
+    "cone_video_prepare_ex": (C.c_int, [_p, _p, _i32, _i64, _p, _p, _p, _sz, C.c_int, _p]),
     "cone_video_prepare_motion": (C.c_int, [_p, _p, _i64, _p, _p, _sz, C.c_int, _p]),
+    "cone_video_prepare_motion_ex": (C.c_int, [_p, _p, _i32, _i64, _p, _p, _sz, C.c_int, _p]),
     "cone_adapter": (C.c_int, [_p, _p, _p, _i64, C.c_int, _p, _sz, C.c_int, _p]),
     "cone_linear": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, C.c_int, _p, _p, _p, _sz, C.c_int, _p]),
     "cone_encoder_tail": (C.c_int, [_p, _i32, _p, _p, _i64, _p, _i32, _p, _sz, _p]),
@@ -49,8 +57,11 @@ SIGNATURES = {
     "cone_window_ranklist": (C.c_int, [_p, _p, _p, _i32, _i32, _p, _p, _i32, _p]),
     "cone_prefilter_workspace_bytes": (_sz, [_p, _i64, _i32]),
     "cone_prefilter": (C.c_int, [_p, _p, _i64, _p, _i32, _i32, _p, _p, _p, _sz, _p]),
+    "cone_prefilter_ex": (C.c_int, [_p, _p, _i32, _i64, _p, _i32, _i32, _i32, _p, _p, _p, _sz, _p]),
     "cone_ground_windows": (C.c_int, [_p, _p, _i64, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _i32, _i32, _i32,
                                       _p, _p, _p, _p, _p, _p, _sz, C.c_int, _p]),
+    "cone_ground_windows_ex": (C.c_int, [_p, _p, _i32, _i64, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _i32, _i32, _i32,
+                                         _p, _p, _p, _p, _p, _p, _sz, C.c_int, _p]),
     "cone_forward": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _p, _p, _p, _p, _p, _p, _sz, C.c_int, _p]),
     "cone_clip_matching": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _p, _p, _sz, C.c_int, _p]),
     "cone_fuse_nms": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _f32, _f64, _i32, _i32, _p, _p, _p, _p, _p]),

@@ -205,7 +205,7 @@ static int check_dims(const cone_dims* c) {
 }
 
 extern "C" const char* cone_last_error(void) { return g_err; }
-extern "C" int cone_version(void) { return 2; }
+extern "C" int cone_version(void) { return 3; }
 extern "C" int64_t cone_launch_count(void) { return g_launches; }
 extern "C" void cone_launch_count_reset(void) { g_launches = 0; }
 
@@ -490,7 +490,9 @@ ProjBuffers plan_proj(Arena& a, int64_t rows, int din, int d) {
     b.a3 = a.get<uint16_t>(rows * 3 * (din > d ? din : d));
     return b;
 }
-int input_proj(const Ctx& cin, const char* name, const float* x, int64_t rows, int din, float* out, ProjBuffers& b) {
+// x: raw rows of storage type x_dtype (CONE_DTYPE_*), read only by the first LayerNorm
+int input_proj(const Ctx& cin, const char* name, const void* x, int x_dtype, int64_t rows, int din, float* out,
+               ProjBuffers& b) {
     // per-frame / per-query work, a few GFLOP per movie: kept in fp32 in every mode (error budget, DESIGN.md)
     // (measured: plain fp16-operand tensor-core GEMMs here save 0.9 ms per step but raise the end-to-end error by 13-20 %
     // rms and push 0.27 % of the values past 1e-3: profiles/r01_notes.md — hence the split GEMM in tensor-core mode)
@@ -498,13 +500,16 @@ int input_proj(const Ctx& cin, const char* name, const float* x, int64_t rows, i
     const Ctx c{cin.w, split ? CONE_PREC_TC_SPLIT : CONE_PREC_FP32, cin.s, b.a3};
     const int d = c.w->dims.hidden;
     const std::string p0 = std::string(name) + ".0", p1 = std::string(name) + ".1";
-    CONE_TRY(layernorm_rows(x, nullptr, c.w->p(p0 + ".LayerNorm.weight"), c.w->p(p0 + ".LayerNorm.bias"), b.ln_in, rows,
-                            din, 1e-5f, c.s));
+    CONE_TRY(layernorm_rows(x, x_dtype, nullptr, c.w->p(p0 + ".LayerNorm.weight"), c.w->p(p0 + ".LayerNorm.bias"), b.ln_in,
+                            rows, din, 1e-5f, c.s));
     CONE_TRY(linear_named(c, b.ln_in, din, rows, p0 + ".net.1", d, din, b.h1, d, 1));
     CONE_TRY(layernorm_rows(b.h1, nullptr, c.w->p(p1 + ".LayerNorm.weight"), c.w->p(p1 + ".LayerNorm.bias"), b.ln_h1,
                             rows, d, 1e-5f, c.s));
     CONE_TRY(linear_named(c, b.ln_h1, d, rows, p1 + ".net.1", d, d, out, d, 0));
     return CONE_OK;
+}
+int input_proj(const Ctx& c, const char* name, const float* x, int64_t rows, int din, float* out, ProjBuffers& b) {
+    return input_proj(c, name, x, CONE_DTYPE_F32, rows, din, out, b);
 }
 
 // adapter_layer(x) (+ x): MLP(Dv, 256, Dv, 2) (cone/model.py:80, 428-440)
@@ -868,10 +873,10 @@ MatchBuffers plan_match(Arena& a, const cone_dims& c, int64_t B, int64_t n_cls) 
     m.tnorm = a.get<float>(n_cls * c.v_dim);
     return m;
 }
-int match_core(const Ctx& c, const float* frames, int64_t n_frames, const CoreBuffers& b, const float* spans,
-               const float* cls, int64_t n_cls, MatchBuffers& m, float* out, int nq) {
+int match_core(const Ctx& c, const void* frames, int frames_dtype, int64_t n_frames, const CoreBuffers& b,
+               const float* spans, const float* cls, int64_t n_cls, MatchBuffers& m, float* out, int nq) {
     const int dv = c.w->dims.v_dim;
-    CONE_TRY(span_mean_pool(frames, n_frames, b.vid_base, b.vlen, b.pad_len, spans, m.pooled, b.B, nq, dv, c.s));
+    CONE_TRY(span_mean_pool(frames, frames_dtype, n_frames, b.vid_base, b.vlen, b.pad_len, spans, m.pooled, b.B, nq, dv, c.s));
     CONE_TRY(adapter_rows(c, m.pooled, b.B * nq, m.hid, m.adapted, 1));
     CONE_TRY(l2norm_rows(cls, m.tnorm, n_cls, dv, 0.f, c.s));  // text_cls / ||text_cls|| (model.py:142)
     CONE_TRY(norm_dot(m.adapted, m.tnorm, b.qidx, out, b.B, nq, dv, c.s));
@@ -925,13 +930,29 @@ int check_prec(int prec) {
     return CONE_OK;
 }
 
+// a raw feature tensor of an _ex entry point: known storage type; 16-bit rows are read 4 elements (8 bytes) at a time,
+// and a sliced view can start at any element
+int check_feature(const char* who, const char* name, const void* p, int32_t dtype) {
+    CONE_REQUIRE(feature_elem_bytes(dtype) != 0, "%s: unknown dtype %d for %s", who, dtype, name);
+    CONE_REQUIRE(dtype == CONE_DTYPE_F32 || ((uintptr_t)p & 7) == 0,
+                 "%s: %s is a 16-bit feature tensor at %p, which is not 8-byte aligned", who, name, p);
+    return CONE_OK;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------
 // entry points
 // ------------------------------------------------------------------------------------------------
 extern "C" int cone_l2_normalize(const float* x, float* out, int64_t rows, int32_t dim, float eps, void* stream) {
-    return l2norm_rows(x, out, rows, dim, eps, (cudaStream_t)stream);
+    return cone_l2_normalize_ex(x, CONE_DTYPE_F32, out, rows, dim, eps, stream);
+}
+
+extern "C" int cone_l2_normalize_ex(const void* x, int32_t x_dtype, float* out, int64_t rows, int32_t dim, float eps,
+                                    void* stream) {
+    CONE_TRY(check_feature("cone_l2_normalize_ex", "x", x, x_dtype));
+    CONE_REQUIRE(x_dtype == CONE_DTYPE_F32 || x != out, "cone_l2_normalize_ex: in place needs fp32 x");
+    return l2norm_rows(x, x_dtype, out, rows, dim, eps, (cudaStream_t)stream);
 }
 
 extern "C" size_t cone_prepare_workspace_bytes(const cone_dims* dims, int64_t n_frames) {
@@ -959,7 +980,15 @@ static int64_t prepare_slab(const cone_dims& dm, int64_t n_frames, size_t worksp
 extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw, int64_t n_frames, float* ctx_out,
                                   float* vidproj_out, void* workspace, size_t workspace_bytes, int precision,
                                   void* stream) {
+    return cone_video_prepare_ex(w, frames_raw, CONE_DTYPE_F32, n_frames, ctx_out, vidproj_out, workspace, workspace_bytes,
+                                 precision, stream);
+}
+
+extern "C" int cone_video_prepare_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t n_frames,
+                                     float* ctx_out, float* vidproj_out, void* workspace, size_t workspace_bytes,
+                                     int precision, void* stream) {
     CONE_REQUIRE(w && frames_raw, "null argument");
+    CONE_TRY(check_feature("cone_video_prepare", "frames_raw", frames_raw, frames_dtype));
     CONE_TRY(check_prec(precision));
     const cone_dims& dm = w->dims;
     CONE_REQUIRE(vidproj_out == nullptr || motion_dim(dm) == dm.v_dim,
@@ -978,15 +1007,16 @@ extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw
         float* ad = a.get<float>(n * dm.v_dim);
         ProjBuffers pb = plan_proj(a, n, dm.v_dim, dm.hidden);
         tc_set_scratch(w->tc, a.base ? a.base + a.used : nullptr, workspace_bytes > a.used ? workspace_bytes - a.used : 0);
-        const float* x = frames_raw + f0 * dm.v_dim;
+        const void* x = static_cast<const char*>(frames_raw) + f0 * dm.v_dim * feature_elem_bytes(frames_dtype);
         if (ctx_out) {
             // host-side L2 norm of the dataset (dataloader:459), adapter + residual, no-eps norm (inference.py:255-257)
-            CONE_TRY(l2norm_rows(x, xn, n, dm.v_dim, 1e-5f, c.s));
+            CONE_TRY(l2norm_rows(x, frames_dtype, xn, n, dm.v_dim, 1e-5f, c.s));
             const Ctx c32{w, CONE_PREC_FP32, c.s};  // the window ranking must be bit-stable across precisions
             CONE_TRY(adapter_rows(c32, xn, n, hid, ad, 1));
             CONE_TRY(l2norm_rows(ad, ctx_out + f0 * dm.v_dim, n, dm.v_dim, 0.f, c.s));
         }
-        if (vidproj_out) CONE_TRY(input_proj(c, "input_vid_proj", x, n, dm.v_dim, vidproj_out + f0 * dm.hidden, pb));
+        if (vidproj_out)
+            CONE_TRY(input_proj(c, "input_vid_proj", x, frames_dtype, n, dm.v_dim, vidproj_out + f0 * dm.hidden, pb));
     }
     return CONE_OK;
 }
@@ -994,7 +1024,15 @@ extern "C" int cone_video_prepare(const cone_weights* w, const float* frames_raw
 extern "C" int cone_video_prepare_motion(const cone_weights* w, const float* motion_raw, int64_t n_frames,
                                          float* vidproj_out, void* workspace, size_t workspace_bytes, int precision,
                                          void* stream) {
+    return cone_video_prepare_motion_ex(w, motion_raw, CONE_DTYPE_F32, n_frames, vidproj_out, workspace, workspace_bytes,
+                                        precision, stream);
+}
+
+extern "C" int cone_video_prepare_motion_ex(const cone_weights* w, const void* motion_raw, int32_t motion_dtype,
+                                            int64_t n_frames, float* vidproj_out, void* workspace, size_t workspace_bytes,
+                                            int precision, void* stream) {
     CONE_REQUIRE(w && motion_raw && vidproj_out, "null argument");
+    CONE_TRY(check_feature("cone_video_prepare_motion", "motion_raw", motion_raw, motion_dtype));
     CONE_REQUIRE(n_frames >= 0, "cone_video_prepare_motion: n_frames=%lld", (long long)n_frames);
     CONE_TRY(check_prec(precision));
     Ctx c{w, precision, (cudaStream_t)stream};
@@ -1010,7 +1048,8 @@ extern "C" int cone_video_prepare_motion(const cone_weights* w, const float* mot
         ProjBuffers pb = plan_proj(a, n, dmot, dm.hidden);
         tc_set_scratch(w->tc, a.base ? a.base + a.used : nullptr, workspace_bytes > a.used ? workspace_bytes - a.used : 0);
         // the dataloader normalises motion rows on the host (ego4d_mad_dataloader.py:284-292) before input_vid_proj
-        CONE_TRY(l2norm_rows(motion_raw + f0 * dmot, xn, n, dmot, 1e-5f, c.s));
+        CONE_TRY(l2norm_rows(static_cast<const char*>(motion_raw) + f0 * dmot * feature_elem_bytes(motion_dtype), motion_dtype,
+                             xn, n, dmot, 1e-5f, c.s));
         CONE_TRY(input_proj(c, "input_vid_proj", xn, n, dmot, vidproj_out + f0 * dm.hidden, pb));
     }
     return CONE_OK;
@@ -1127,7 +1166,16 @@ extern "C" size_t cone_prefilter_workspace_bytes(const cone_dims* dims, int64_t 
 extern "C" int cone_prefilter(const cone_weights* w, const float* frames_raw, int64_t L, const float* cls_raw,
                               int32_t n_queries, int32_t topk, int32_t* win_idx, float* win_score, void* workspace,
                               size_t workspace_bytes, void* stream) {
+    return cone_prefilter_ex(w, frames_raw, CONE_DTYPE_F32, L, cls_raw, CONE_DTYPE_F32, n_queries, topk, win_idx, win_score,
+                             workspace, workspace_bytes, stream);
+}
+
+extern "C" int cone_prefilter_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t L,
+                                 const void* cls_raw, int32_t cls_dtype, int32_t n_queries, int32_t topk, int32_t* win_idx,
+                                 float* win_score, void* workspace, size_t workspace_bytes, void* stream) {
     CONE_REQUIRE(w && frames_raw && win_idx && (cls_raw || n_queries == 0), "null argument");
+    CONE_TRY(check_feature("cone_prefilter", "frames_raw", frames_raw, frames_dtype));
+    CONE_TRY(check_feature("cone_prefilter", "cls_raw", cls_raw, cls_dtype));
     CONE_REQUIRE(L > 0 && n_queries >= 0 && topk > 0, "cone_prefilter: L=%lld n_queries=%d topk=%d", (long long)L, n_queries, topk);
     if (n_queries == 0) return CONE_OK;
     const cone_dims& dm = w->dims;
@@ -1149,8 +1197,9 @@ extern "C" int cone_prefilter(const cone_weights* w, const float* frames_raw, in
         return CONE_ERR_WORKSPACE;
     }
     // A1 + A2: normalised, adapted context features of every frame (always fp32: the ranking must be bit-stable)
-    CONE_TRY(cone_video_prepare(w, frames_raw, L, ctx, nullptr, a.base + a.used, workspace_bytes - a.used, CONE_PREC_FP32, stream));
-    CONE_TRY(l2norm_rows(cls_raw, cls_n, n_queries, dm.v_dim, 1e-5f, s));  // dataloader:472
+    CONE_TRY(cone_video_prepare_ex(w, frames_raw, frames_dtype, L, ctx, nullptr, a.base + a.used, workspace_bytes - a.used,
+                                   CONE_PREC_FP32, stream));
+    CONE_TRY(l2norm_rows(cls_raw, cls_dtype, cls_n, n_queries, dm.v_dim, 1e-5f, s));  // dataloader:472
     // A3: frame scores, window maxima, full rank-list; the first topk entries leave
     CONE_TRY(prefilter_desc(video_offsets, q_first, score_offsets, frame_count, L, n_queries, s));
     CONE_REQUIRE(L <= INT32_MAX, "cone_prefilter: video too long");
@@ -1195,9 +1244,22 @@ extern "C" int cone_ground_windows(const cone_weights* w, const float* frames_ra
                                    int32_t n_batches, int32_t n_queries, int32_t topk, float* pred_spans,
                                    float* prob_fg, float* match, int32_t* win_start, int32_t* win_len, void* workspace,
                                    size_t workspace_bytes, int precision, void* stream) {
+    return cone_ground_windows_ex(w, frames_raw, CONE_DTYPE_F32, n_frames, vidproj, q_video_start, q_video_len, ranklist,
+                                  ranklist_stride, tok, tok_len, cls_norm, q_batch, n_batches, n_queries, topk, pred_spans,
+                                  prob_fg, match, win_start, win_len, workspace, workspace_bytes, precision, stream);
+}
+
+extern "C" int cone_ground_windows_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t n_frames,
+                                      const float* vidproj, const int64_t* q_video_start, const int32_t* q_video_len,
+                                      const int32_t* ranklist, int32_t ranklist_stride, const float* tok,
+                                      const int32_t* tok_len, const float* cls_norm, const int32_t* q_batch,
+                                      int32_t n_batches, int32_t n_queries, int32_t topk, float* pred_spans,
+                                      float* prob_fg, float* match, int32_t* win_start, int32_t* win_len, void* workspace,
+                                      size_t workspace_bytes, int precision, void* stream) {
     CONE_REQUIRE(w && frames_raw && vidproj && q_video_start && q_video_len && ranklist && tok && tok_len && cls_norm &&
                      pred_spans && prob_fg && match && win_start && win_len && workspace,
                  "null argument");
+    CONE_TRY(check_feature("cone_ground_windows", "frames_raw", frames_raw, frames_dtype));
     CONE_REQUIRE(topk >= 1 && n_batches >= 1 && n_queries >= 0, "bad sizes");
     CONE_TRY(check_prec(precision));
     Ctx c{w, precision, (cudaStream_t)stream};
@@ -1296,7 +1358,7 @@ extern "C" int cone_ground_windows(const cone_weights* w, const float* frames_ra
         }
         float* spans_c = pred_spans + q0 * topk * nq * 2;
         CONE_TRY(transformer_core(c, cb, nullptr, prob_fg + q0 * topk * nq, spans_c, nullptr, nullptr, nullptr));
-        CONE_TRY(match_core(c, frames_raw, n_frames, cb, spans_c, cls_norm + q0 * dm.v_dim, n, mb, match + q0 * topk * nq, nq));
+        CONE_TRY(match_core(c, frames_raw, frames_dtype, n_frames, cb, spans_c, cls_norm + q0 * dm.v_dim, n, mb, match + q0 * topk * nq, nq));
     }
     return CONE_OK;
 }
@@ -1370,7 +1432,7 @@ extern "C" int cone_clip_matching(const cone_weights* w, const float* src_cls_tx
     CONE_TRY(fill_window_desc_dense(cb.vid_base, cb.txt_base, cb.qidx, B, Lv, 0, c.s));
     CONE_CUDA(cudaMemcpyAsync(cb.vlen, vid_len, sizeof(int32_t) * B, cudaMemcpyDeviceToDevice, c.s));
     CONE_TRY(fill_i32(cb.pad_len, B, Lv, c.s));  // the dense tensor is already padded to Lv rows
-    return match_core(c, src_vid_appear, (int64_t)B * Lv, cb, spans, src_cls_txt, B, mb, out, nq);
+    return match_core(c, src_vid_appear, CONE_DTYPE_F32, (int64_t)B * Lv, cb, spans, src_cls_txt, B, mb, out, nq);
 }
 
 extern "C" int cone_fuse_nms(const float* pred_spans, const float* prob_fg, const float* match, const int32_t* win_start,

@@ -4,6 +4,11 @@
 
 namespace cone {
 
+// bytes per element of a raw feature tensor of dtype CONE_DTYPE_*; 0 = unknown code
+inline size_t feature_elem_bytes(int dtype) {
+    return dtype == CONE_DTYPE_F32 ? 4 : (dtype == CONE_DTYPE_F16 || dtype == CONE_DTYPE_BF16) ? 2 : 0;
+}
+
 // ---------------------------------------------------------------- gemm_simt.cu
 // C[M,N] = epi(A[M,K] * W[N,K]^T): both operands K-major (row-major activations x nn.Linear weight).
 struct GemmParams {
@@ -34,9 +39,17 @@ int rowdot_small(const float* x, int64_t ldx, const float* W, const float* bias,
                  int mode, cudaStream_t s, int group_out = 0, int group_in = 0);
 
 // ---------------------------------------------------------------- rowops.cu
-int layernorm_rows(const float* x, const float* residual, const float* gamma, const float* beta, float* out,
+// x_dtype (CONE_DTYPE_*) is the element type of the raw rows x; residual, gamma, beta and out are fp32
+int layernorm_rows(const void* x, int x_dtype, const float* residual, const float* gamma, const float* beta, float* out,
                    int64_t rows, int D, float eps, cudaStream_t s);
-int l2norm_rows(const float* x, float* out, int64_t rows, int D, float eps, cudaStream_t s);
+inline int layernorm_rows(const float* x, const float* residual, const float* gamma, const float* beta, float* out,
+                          int64_t rows, int D, float eps, cudaStream_t s) {
+    return layernorm_rows(x, CONE_DTYPE_F32, residual, gamma, beta, out, rows, D, eps, s);
+}
+int l2norm_rows(const void* x, int x_dtype, float* out, int64_t rows, int D, float eps, cudaStream_t s);
+inline int l2norm_rows(const float* x, float* out, int64_t rows, int D, float eps, cudaStream_t s) {
+    return l2norm_rows(x, CONE_DTYPE_F32, out, rows, D, eps, s);
+}
 int build_pos_table(float* table, int max_v_l, int d, cudaStream_t s);  // [max_v_l+1, max_v_l, d]
 // window rows: src[b*S + r] = r < Lv ? vidproj[min(vid_base[b]+r, n_vid_rows-1)] : txtproj[txt_base[b] + r - Lv]
 int gather_window_rows(const float* vidproj, int64_t n_vid_rows, const int64_t* vid_base, const float* txtproj,
@@ -123,7 +136,8 @@ int fill_window_desc_chunk(const int64_t* q_video_start, const int32_t* win_star
 
 // ---------------------------------------------------------------- pool_match.cu
 // pooled[(b*nq+j), :] = mean of zero-padded window rows [start, min(end, pad_len)) (model.py:186-200)
-int span_mean_pool(const float* frames, int64_t n_frames, const int64_t* vid_base, const int32_t* vlen,
+// frames_dtype (CONE_DTYPE_*): element type of the raw rows; pooled is fp32
+int span_mean_pool(const void* frames, int frames_dtype, int64_t n_frames, const int64_t* vid_base, const int32_t* vlen,
                    const int32_t* pad_len, const float* spans, float* pooled, int64_t B, int nq, int Dv,
                    cudaStream_t s);
 // out[b*nq+j] = (p / ||p||) . t[qidx[b]]

@@ -1,8 +1,13 @@
 // Fine-grained proposal ranking (cone/model.py:130-152, 178-210): span -> [floor, ceil) frame bounds,
 // mean-pool the RAW appearance rows of the zero-padded window, (adapter + residual via the GEMM path),
 // L2-normalise, dot with the normalised CLS vector.  HBM/L2-bound: coalesced float4 row reads.
+// The pooling kernels also read raw rows stored as fp16 / bf16 (features.cuh): 4 columns per thread as in fp32, each
+// column's rows added in row order into its own fp32 accumulator, so the pooled rows are those of the upcast input.
 #include <math_constants.h>
 
+#include <type_traits>
+
+#include "features.cuh"
 #include "kernels.h"
 
 namespace cone {
@@ -14,8 +19,9 @@ namespace {
 //   start = relu(int(floor(x1 * dur))) ; end = int(ceil(x2 * dur))          (model.py:187-192)
 // `feat[start:end]` is a Python slice of the window zero-padded to pad_len rows: `end` clips to pad_len,
 // pad rows inside the slice are averaged in (they are zeros), an empty slice gives NaN.
+template <class T>
 __global__ void __launch_bounds__(256)
-span_mean_pool_kernel(const float* __restrict__ frames, int64_t n_frames, const int64_t* __restrict__ vid_base,
+span_mean_pool_kernel(const T* __restrict__ frames, int64_t n_frames, const int64_t* __restrict__ vid_base,
                       const int32_t* __restrict__ vlen, const int32_t* __restrict__ pad_len,
                       const float* __restrict__ spans, float* __restrict__ pooled, int nq, int Dv) {
     const int64_t p = blockIdx.x;  // window * nq + slot
@@ -44,8 +50,7 @@ span_mean_pool_kernel(const float* __restrict__ frames, int64_t n_frames, const 
             float4 v[8];
 #pragma unroll
             for (int u = 0; u < 8; ++u)
-                v[u] = (r + u < last) ? __ldg(reinterpret_cast<const float4*>(frames + (base + r + u) * Dv) + c)
-                                      : make_float4(0.f, 0.f, 0.f, 0.f);
+                v[u] = (r + u < last) ? ldg_feat4(frames + (base + r + u) * Dv + 4 * c) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
                 if (r + u < last) {
@@ -69,9 +74,9 @@ span_mean_pool_kernel(const float* __restrict__ frames, int64_t n_frames, const 
 // still added in increasing order into its own accumulator, so the result is bit-identical to the per-proposal kernel
 // above; what changes is the traffic: the proposals of a window overlap (ncu: 39 rows per proposal on average, 195 per
 // window, against at most Lv = 125 distinct rows).
-template <int NQ>
+template <int NQ, class T>
 __global__ void __launch_bounds__(256)
-span_mean_pool_window_kernel(const float* __restrict__ frames, int64_t n_frames, const int64_t* __restrict__ vid_base,
+span_mean_pool_window_kernel(const T* __restrict__ frames, int64_t n_frames, const int64_t* __restrict__ vid_base,
                              const int32_t* __restrict__ vlen, const int32_t* __restrict__ pad_len,
                              const float* __restrict__ spans, float* __restrict__ pooled, int nq, int Dv) {
     const int64_t b = blockIdx.x;
@@ -114,8 +119,7 @@ span_mean_pool_window_kernel(const float* __restrict__ frames, int64_t n_frames,
             float4 v[8];
 #pragma unroll
             for (int u = 0; u < 8; ++u)
-                v[u] = (r + u < hi) ? __ldg(reinterpret_cast<const float4*>(frames + (base + r + u) * Dv) + c)
-                                    : make_float4(0.f, 0.f, 0.f, 0.f);
+                v[u] = (r + u < hi) ? ldg_feat4(frames + (base + r + u) * Dv + 4 * c) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
             for (int u = 0; u < 8; ++u) {
 #pragma unroll
@@ -169,25 +173,29 @@ __global__ void norm_dot_kernel(const float* __restrict__ x, const float* __rest
 
 }  // namespace
 
-int span_mean_pool(const float* frames, int64_t n_frames, const int64_t* vid_base, const int32_t* vlen,
+int span_mean_pool(const void* frames_v, int frames_dtype, int64_t n_frames, const int64_t* vid_base, const int32_t* vlen,
                    const int32_t* pad_len, const float* spans, float* pooled, int64_t B, int nq, int Dv,
                    cudaStream_t s) {
-    if (B == 0) return CONE_OK;
-    CONE_REQUIRE((Dv & 3) == 0, "span_mean_pool: Dv must be a multiple of 4");
-    const int threads = (Dv / 4) >= 256 ? 256 : ((Dv / 4 + 31) / 32) * 32;
-    ProfScope ps(s, P_POOL);
-    if (nq <= 5) {
-        span_mean_pool_window_kernel<5><<<(unsigned)B, threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len, spans,
-                                                                     pooled, nq, Dv);
-    } else if (nq <= 8) {
-        span_mean_pool_window_kernel<8><<<(unsigned)B, threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len, spans,
-                                                                     pooled, nq, Dv);
-    } else {  // many proposals per window (cone_clip_matching allows up to 64): one CTA per proposal
-        span_mean_pool_kernel<<<(unsigned)(B * nq), threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len, spans,
-                                                                   pooled, nq, Dv);
-    }
-    CONE_LAUNCH_CHECK("span_mean_pool");
-    return CONE_OK;
+    return dispatch_feature(frames_dtype, [&](auto tag) {
+        using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+        const T* frames = static_cast<const T*>(frames_v);
+        if (B == 0) return CONE_OK;
+        CONE_REQUIRE((Dv & 3) == 0, "span_mean_pool: Dv must be a multiple of 4");
+        const int threads = (Dv / 4) >= 256 ? 256 : ((Dv / 4 + 31) / 32) * 32;
+        ProfScope ps(s, P_POOL);
+        if (nq <= 5) {
+            span_mean_pool_window_kernel<5, T><<<(unsigned)B, threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len,
+                                                                            spans, pooled, nq, Dv);
+        } else if (nq <= 8) {
+            span_mean_pool_window_kernel<8, T><<<(unsigned)B, threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len,
+                                                                            spans, pooled, nq, Dv);
+        } else {  // many proposals per window (cone_clip_matching allows up to 64): one CTA per proposal
+            span_mean_pool_kernel<T><<<(unsigned)(B * nq), threads, 0, s>>>(frames, n_frames, vid_base, vlen, pad_len, spans,
+                                                                          pooled, nq, Dv);
+        }
+        CONE_LAUNCH_CHECK("span_mean_pool");
+        return CONE_OK;
+    });
 }
 
 int norm_dot(const float* p, const float* t, const int32_t* qidx, float* out, int64_t B, int nq, int Dv,

@@ -1,7 +1,12 @@
 // Row-wise fp32 kernels: LayerNorm (+residual), L2 normalisation, sine position table, window row gather.
 // All are HBM/L2-bound: one warp per row, float4 accesses, grid sized from the row count.
+// LayerNorm and L2 normalisation also read raw feature rows stored as fp16 / bf16 (features.cuh): a lane then loads the
+// same 4 elements per step with one 8-byte load, so its partial sums, and the result, are those of the fp32 kernel.
 #include <cuda_fp16.h>
 
+#include <type_traits>
+
+#include "features.cuh"
 #include "kernels.h"
 
 namespace cone {
@@ -11,18 +16,19 @@ namespace {
 constexpr int kWarpsPerBlock = 8;
 
 // out = LayerNorm(x (+ residual)) * gamma + beta     (torch.nn.LayerNorm: biased variance, eps inside sqrt)
-__global__ void layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ res,
+template <class T>
+__global__ void layernorm_rows_kernel(const T* __restrict__ x, const float* __restrict__ res,
                                       const float* __restrict__ gamma, const float* __restrict__ beta,
                                       float* __restrict__ out, int64_t rows, int D, float eps) {
     const int lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
     if (row >= rows) return;
-    const float4* xr = reinterpret_cast<const float4*>(x + row * D);
+    const T* xr = x + row * D;
     const float4* rr = res ? reinterpret_cast<const float4*>(res + row * D) : nullptr;
     const int nv = D >> 2;
     float sum = 0.f;
     for (int i = lane; i < nv; i += 32) {
-        float4 v = xr[i];
+        float4 v = load_feat4(xr + 4 * i);
         if (rr) {
             const float4 r = rr[i];
             v.x += r.x; v.y += r.y; v.z += r.z; v.w += r.w;
@@ -32,7 +38,7 @@ __global__ void layernorm_rows_kernel(const float* __restrict__ x, const float* 
     const float mean = warp_sum(sum) / (float)D;
     float sq = 0.f;
     for (int i = lane; i < nv; i += 32) {
-        float4 v = xr[i];
+        float4 v = load_feat4(xr + 4 * i);
         if (rr) {
             const float4 r = rr[i];
             v.x += r.x; v.y += r.y; v.z += r.z; v.w += r.w;
@@ -43,7 +49,7 @@ __global__ void layernorm_rows_kernel(const float* __restrict__ x, const float* 
     const float rstd = rsqrtf(warp_sum(sq) / (float)D + eps);
     float4* orow = reinterpret_cast<float4*>(out + row * D);
     for (int i = lane; i < nv; i += 32) {
-        float4 v = xr[i];
+        float4 v = load_feat4(xr + 4 * i);
         if (rr) {
             const float4 r = rr[i];
             v.x += r.x; v.y += r.y; v.z += r.z; v.w += r.w;
@@ -60,15 +66,16 @@ __global__ void layernorm_rows_kernel(const float* __restrict__ x, const float* 
 }
 
 // out = x / (||x||_2 + eps)
-__global__ void l2norm_rows_kernel(const float* __restrict__ x, float* __restrict__ out, int64_t rows, int D, float eps) {
+template <class T>
+__global__ void l2norm_rows_kernel(const T* __restrict__ x, float* __restrict__ out, int64_t rows, int D, float eps) {
     const int lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5);
     if (row >= rows) return;
-    const float4* xr = reinterpret_cast<const float4*>(x + row * D);
+    const T* xr = x + row * D;
     const int nv = D >> 2;
     float sq = 0.f;
     for (int i = lane; i < nv; i += 32) {
-        const float4 v = xr[i];
+        const float4 v = load_feat4(xr + 4 * i);
         sq += (v.x * v.x + v.y * v.y) + (v.z * v.z + v.w * v.w);
     }
     // eps >= 0: x / (||x|| + eps) (utils/basic_utils.py:97-99); eps < 0: x / max(||x||, -eps) = torch F.normalize
@@ -77,7 +84,7 @@ __global__ void l2norm_rows_kernel(const float* __restrict__ x, float* __restric
     const float denom = eps >= 0.f ? nrm + eps : fmaxf(nrm, -eps);
     float4* orow = reinterpret_cast<float4*>(out + row * D);
     for (int i = lane; i < nv; i += 32) {
-        const float4 v = xr[i];
+        const float4 v = load_feat4(xr + 4 * i);
         orow[i] = make_float4(v.x / denom, v.y / denom, v.z / denom, v.w / denom);
     }
 }
@@ -317,24 +324,31 @@ inline unsigned grid_for(int64_t total, int block) {
 
 }  // namespace
 
-int layernorm_rows(const float* x, const float* residual, const float* gamma, const float* beta, float* out,
+int layernorm_rows(const void* x, int x_dtype, const float* residual, const float* gamma, const float* beta, float* out,
                    int64_t rows, int D, float eps, cudaStream_t s) {
-    if (rows == 0) return CONE_OK;
-    CONE_REQUIRE((D & 3) == 0, "layernorm: D must be a multiple of 4");
-    ProfScope ps(s, P_LAYERNORM, 0.0, (residual ? 12.0 : 8.0) * (double)rows * D);
-    layernorm_rows_kernel<<<(unsigned)cdiv64(rows, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(x, residual, gamma,
-                                                                                               beta, out, rows, D, eps);
-    CONE_LAUNCH_CHECK("layernorm_rows");
-    return CONE_OK;
+    return dispatch_feature(x_dtype, [&](auto tag) {
+        using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+        if (rows == 0) return CONE_OK;
+        CONE_REQUIRE((D & 3) == 0, "layernorm: D must be a multiple of 4");
+        ProfScope ps(s, P_LAYERNORM, 0.0, ((residual ? 8.0 : 4.0) + sizeof(T)) * (double)rows * D);
+        layernorm_rows_kernel<T><<<(unsigned)cdiv64(rows, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+            static_cast<const T*>(x), residual, gamma, beta, out, rows, D, eps);
+        CONE_LAUNCH_CHECK("layernorm_rows");
+        return CONE_OK;
+    });
 }
 
-int l2norm_rows(const float* x, float* out, int64_t rows, int D, float eps, cudaStream_t s) {
-    if (rows == 0) return CONE_OK;
-    CONE_REQUIRE((D & 3) == 0, "l2norm: D must be a multiple of 4");
-    ProfScope ps(s, P_LAYERNORM, 0.0, 8.0 * (double)rows * D);
-    l2norm_rows_kernel<<<(unsigned)cdiv64(rows, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(x, out, rows, D, eps);
-    CONE_LAUNCH_CHECK("l2norm_rows");
-    return CONE_OK;
+int l2norm_rows(const void* x, int x_dtype, float* out, int64_t rows, int D, float eps, cudaStream_t s) {
+    return dispatch_feature(x_dtype, [&](auto tag) {
+        using T = std::remove_const_t<std::remove_pointer_t<decltype(tag)>>;
+        if (rows == 0) return CONE_OK;
+        CONE_REQUIRE((D & 3) == 0, "l2norm: D must be a multiple of 4");
+        ProfScope ps(s, P_LAYERNORM, 0.0, (4.0 + sizeof(T)) * (double)rows * D);
+        l2norm_rows_kernel<T><<<(unsigned)cdiv64(rows, kWarpsPerBlock), kWarpsPerBlock * 32, 0, s>>>(
+            static_cast<const T*>(x), out, rows, D, eps);
+        CONE_LAUNCH_CHECK("l2norm_rows");
+        return CONE_OK;
+    });
 }
 
 int build_pos_table(float* table, int max_v_l, int d, cudaStream_t s) {

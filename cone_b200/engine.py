@@ -32,6 +32,29 @@ def _need(t: torch.Tensor, dtype, name: str) -> torch.Tensor:
     return t.contiguous()
 
 
+# storage types a raw feature tensor (frames, motion rows, tokens, CLS) may have; results are those of `t.float()`
+FEATURE_DTYPES = {torch.float32: _lib.DTYPE_F32, torch.float16: _lib.DTYPE_F16, torch.bfloat16: _lib.DTYPE_BF16}
+
+
+def _need_feature(t: torch.Tensor, name: str):
+    """(contiguous t, its CONE_DTYPE_* code) for a raw feature tensor."""
+    if not t.is_cuda:
+        raise ValueError(f"{name} must be a CUDA tensor")
+    if t.dtype not in FEATURE_DTYPES:
+        raise TypeError(f"{name} must be float32, float16 or bfloat16, got {t.dtype}")
+    return t.contiguous(), FEATURE_DTYPES[t.dtype]
+
+
+def host_feature_dtype(arrays, what: str) -> np.dtype:
+    """Storage type of a set of host feature arrays that are staged together: float16 when every array is float16,
+    else float32 (other float types are converted as before).  A mix of float16 and other types raises ValueError:
+    concatenating them would silently promote the float16 ones."""
+    kinds = {np.asarray(a).dtype == np.float16 for a in arrays}
+    if len(kinds) > 1:
+        raise ValueError(f"{what} mix float16 and float32 features: cast them to one dtype")
+    return np.dtype(np.float16 if kinds == {True} else np.float32)
+
+
 @dataclasses.dataclass
 class QueryBatch:
     """Queries of a set of videos, grouped by video (the order the kernels run in).  `order[i]` is the
@@ -40,9 +63,9 @@ class QueryBatch:
     q_first: torch.Tensor  # [Nv+1] int32, first packed query of each video
     q_video_start: torch.Tensor  # [Nq] int64
     q_video_len: torch.Tensor  # [Nq] int32
-    tokens: torch.Tensor  # [Nq, max_q_l, Dt] fp32 raw, zero padded (truncated to max_q_l)
+    tokens: torch.Tensor  # [Nq, max_q_l, Dt] raw (fp32, fp16 or bf16), zero padded (truncated to max_q_l)
     tok_len: torch.Tensor  # [Nq] int32
-    cls: torch.Tensor  # [Nq, Dv] fp32 raw
+    cls: torch.Tensor  # [Nq, Dv] raw (fp32, fp16 or bf16)
     q_batch: torch.Tensor  # [Nq] int32 reference eval-batch id (dataset index // eval_bsz)
     n_batches: int
     max_video_frames: int
@@ -96,9 +119,11 @@ def pack_queries(cfg: ConeConfig, video_lengths: Sequence[int], queries, first_d
     offs[1:] = np.cumsum(np.asarray(video_lengths, dtype=np.int64))
     vid = np.asarray([queries[i].video_idx for i in order], dtype=np.int64)
     q_first = np.searchsorted(vid, np.arange(len(video_lengths) + 1)).astype(np.int32)
-    tokens = np.zeros((nq, cfg.max_q_l, cfg.t_feat_dim), dtype=np.float32)
+    # float16 queries stay float16 (zero padded in float16): the device converts them on load
+    fdt = host_feature_dtype([q.tokens for q in queries] + [q.cls for q in queries], "queries")
+    tokens = np.zeros((nq, cfg.max_q_l, cfg.t_feat_dim), dtype=fdt)
     tok_len = np.zeros(nq, dtype=np.int32)
-    cls = np.zeros((nq, cfg.v_feat_dim), dtype=np.float32)
+    cls = np.zeros((nq, cfg.v_feat_dim), dtype=fdt)
     for j, i in enumerate(order):
         q = queries[i]
         t = q.tokens[: cfg.max_q_l]  # `q_feat[:self.max_q_l]` (dataloader:272)
@@ -196,10 +221,12 @@ class ConeEngine:
 
     # ---- stage kernels ------------------------------------------------------------------------
     def l2_normalize(self, x: torch.Tensor, eps: float) -> torch.Tensor:
-        x = _need(x, torch.float32, "x")
-        out = torch.empty_like(x)
+        """x / (||x|| + eps) per row (eps < 0: x / max(||x||, -eps)); x fp32, fp16 or bf16, the result fp32."""
+        x, xt = _need_feature(x, "x")
+        out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
         rows = x.numel() // x.shape[-1]
-        _lib.check(self.lib.cone_l2_normalize(_ptr(x), _ptr(out), rows, x.shape[-1], eps, _stream()), "cone_l2_normalize")
+        _lib.check(self.lib.cone_l2_normalize_ex(_ptr(x), xt, _ptr(out), rows, x.shape[-1], eps, _stream()),
+                   "cone_l2_normalize_ex")
         return out
 
     def encoder_tail(self, layer: int, att: torch.Tensor, res: torch.Tensor, cta_group: int = 0) -> torch.Tensor:
@@ -243,33 +270,34 @@ class ConeEngine:
         """Stage 0 + per-frame `input_vid_proj` over concatenated frames [n, Dv] (raw appearance features).
         `motion` [n, Dm]: raw features of a separate motion stream, one row per appearance row; `input_vid_proj` then
         reads them L2-normalised (ego4d_mad_dataloader.py:284-292).  Without it the appearance rows are projected
-        raw, which is only valid when the model's motion dim is Dv."""
-        frames = _need(frames, torch.float32, "frames")
+        raw, which is only valid when the model's motion dim is Dv.  `frames` and `motion` may each be stored as fp32,
+        fp16 or bf16; the results (fp32) are those of the fp32 upcast."""
+        frames, ft = _need_feature(frames, "frames")
         n = frames.shape[0]
         if motion is not None:
-            motion = self._check_motion(motion, n)
+            motion, mt = self._check_motion(motion, n)
         elif want_vidproj and self.cfg.motion_dim != self.cfg.v_feat_dim:
             raise ValueError(f"the model reads {self.cfg.motion_dim}-d motion features: pass `motion` [n_frames, "
                              f"{self.cfg.motion_dim}] (appearance rows are {self.cfg.v_feat_dim}-d)")
-        ctx = torch.empty_like(frames) if want_ctx else None
+        ctx = torch.empty(frames.shape, dtype=torch.float32, device=frames.device) if want_ctx else None
         vp = torch.empty((n, self.cfg.hidden_dim), dtype=torch.float32, device=frames.device) if want_vidproj else None
         ws, nb = self._wsargs()
-        _lib.check(self.lib.cone_video_prepare(self._handle, _ptr(frames), n, _ptr(ctx),
-                                               _ptr(vp if motion is None else None), ws, nb, self.precision, _stream()),
-                   "cone_video_prepare")
+        _lib.check(self.lib.cone_video_prepare_ex(self._handle, _ptr(frames), ft, n, _ptr(ctx),
+                                                  _ptr(vp if motion is None else None), ws, nb, self.precision, _stream()),
+                   "cone_video_prepare_ex")
         if motion is not None and want_vidproj:
-            _lib.check(self.lib.cone_video_prepare_motion(self._handle, _ptr(motion), n, _ptr(vp), ws, nb, self.precision,
-                                                          _stream()), "cone_video_prepare_motion")
+            _lib.check(self.lib.cone_video_prepare_motion_ex(self._handle, _ptr(motion), mt, n, _ptr(vp), ws, nb,
+                                                             self.precision, _stream()), "cone_video_prepare_motion_ex")
         return ctx, vp
 
-    def _check_motion(self, motion: torch.Tensor, n_frames: int) -> torch.Tensor:
+    def _check_motion(self, motion: torch.Tensor, n_frames: int):
         """Both streams are sliced with the same window bounds (ego4d_mad_dataloader.py:144-159): a motion tensor of
-        another length is refused rather than truncated."""
-        motion = _need(motion, torch.float32, "motion")
+        another length is refused rather than truncated.  Returns (motion, its dtype code)."""
+        motion, mt = _need_feature(motion, "motion")
         if motion.dim() != 2 or motion.shape != (n_frames, self.cfg.motion_dim):
             raise ValueError(f"motion must be [{n_frames}, {self.cfg.motion_dim}] (one row per appearance frame), "
                              f"got {tuple(motion.shape)}")
-        return motion
+        return motion, mt
 
     def frame_scores(self, ctx: torch.Tensor, qb: QueryBatch, cls_norm: torch.Tensor):
         """`einsum('db,b->d')` of every query against its own video (cone/inference.py:284) as one grouped
@@ -304,17 +332,17 @@ class ConeEngine:
         """Stages 0 + 1 for ONE video in one call (`cone_prefilter`): raw frames [L, Dv] and raw CLS [Nq, Dv] -> the first
         `topk` window ids of every query's rank-list (-1 where the video has fewer windows) and their window scores.
         The same pre-filter `compute_window_ranklist` runs (run_on_video/cone_localizator.py:83-100) and the 2D-TAN
-        variant reuses (cone_2dtan/moment_localization/test.py:173-239)."""
-        frames_raw = _need(frames_raw, torch.float32, "frames_raw")
-        cls_raw = _need(cls_raw, torch.float32, "cls_raw")
+        variant reuses (cone_2dtan/moment_localization/test.py:173-239).  Frames and CLS may each be fp32, fp16 or bf16."""
+        frames_raw, ft = _need_feature(frames_raw, "frames_raw")
+        cls_raw, ct = _need_feature(cls_raw, "cls_raw")
         L, nq = frames_raw.shape[0], cls_raw.shape[0]
         topk = topk or self.cfg.topk_window
         idx = torch.empty((nq, topk), dtype=torch.int32, device=frames_raw.device)
         sc = torch.empty((nq, topk), dtype=torch.float32, device=frames_raw.device) if want_scores else None
         need = self.lib.cone_prefilter_workspace_bytes(C.byref(self.dims), L, nq)
         ws, nb = self._wsargs(need)
-        _lib.check(self.lib.cone_prefilter(self._handle, _ptr(frames_raw), L, _ptr(cls_raw), nq, topk, _ptr(idx), _ptr(sc), ws, nb,
-                                           _stream()), "cone_prefilter")
+        _lib.check(self.lib.cone_prefilter_ex(self._handle, _ptr(frames_raw), ft, L, _ptr(cls_raw), ct, nq, topk, _ptr(idx),
+                                              _ptr(sc), ws, nb, _stream()), "cone_prefilter_ex")
         return (idx, sc) if want_scores else idx
 
     def forward(self, src_txt, txt_len, src_vid, vid_len, want_saliency=False, want_aux=False):
@@ -428,9 +456,11 @@ class ConeEngine:
         `frames`; stages 0/1 and the matching pool keep reading `frames`, Moment-DETR reads the motion rows.
         `prepared` = (ctx, vidproj) from an earlier `video_prepare(frames, motion=motion)`: stage 0 is per VIDEO
         (cone/inference.py:241-260 runs it once per video before any query), so a long video whose queries are
-        processed in several calls (BASELINE.json configs[4]) pays for it once; `motion` is then not read."""
+        processed in several calls (BASELINE.json configs[4]) pays for it once; `motion` is then not read.
+        `frames`, `motion`, `qb.tokens` and `qb.cls` may each be stored as fp32, fp16 or bf16: the output is bitwise
+        the one of the same call on their fp32 upcasts (the library converts on load and keeps the fp32 order)."""
         cfg = self.cfg
-        frames = _need(frames, torch.float32, "frames")
+        frames, ft = _need_feature(frames, "frames")
         dev = frames.device
         nq = qb.tok_len.numel()
         k = cfg.topk_window
@@ -452,11 +482,11 @@ class ConeEngine:
         wstart = torch.empty((nq, k), dtype=torch.int32, device=dev)
         wlen = torch.empty((nq, k), dtype=torch.int32, device=dev)
         ws, nb = self._wsargs()
-        _lib.check(self.lib.cone_ground_windows(
-            self._handle, _ptr(frames), frames.shape[0], _ptr(vidproj), _ptr(qb.q_video_start), _ptr(qb.q_video_len),
+        _lib.check(self.lib.cone_ground_windows_ex(
+            self._handle, _ptr(frames), ft, frames.shape[0], _ptr(vidproj), _ptr(qb.q_video_start), _ptr(qb.q_video_len),
             _ptr(ranklist), stride, _ptr(tok_norm), _ptr(qb.tok_len), _ptr(cls_norm), _ptr(qb.q_batch), qb.n_batches,
             nq, k, _ptr(spans), _ptr(prob), _ptr(match), _ptr(wstart), _ptr(wlen), ws, nb, self.precision, _stream()),
-            "cone_ground_windows")
+            "cone_ground_windows_ex")
         # stage 3
         nms, cnt, rows, rcnt = self.fuse_nms(spans, prob, match, wstart, wlen, want_rows=want_rows)
         return GroundingOutput(ranklist, wstart, wlen, spans, prob, match, nms, cnt, rows, rcnt)
@@ -477,8 +507,12 @@ class ConeEngine:
                      cfg: Optional[ConeConfig] = None, want_rows: bool = False) -> GroundingOutput:
         """Per-query part of `predict_moment` (:131-221) for queries of ONE video prepared by `prepare_video`:
         tokens F.normalize'd, CLS used raw, windows zero-padded to max_v_l for pooling, spans scaled by max_v_l,
-        slots in slot order, fusion ranking with the demo's NMS constants (pass them in `cfg`).  No host sync."""
+        slots in slot order, fusion ranking with the demo's NMS constants (pass them in `cfg`).  No host sync.
+        fp32 only, like `prepare_video`."""
         cfg = cfg or self.cfg
+        xn = _need(xn, torch.float32, "xn")
+        _need(qb.tokens, torch.float32, "qb.tokens")
+        _need(qb.cls, torch.float32, "qb.cls")
         dev = xn.device
         nq, k, ns = qb.tok_len.numel(), cfg.topk_window, cfg.num_queries
         tok_norm = self.l2_normalize(qb.tokens, -1e-5)

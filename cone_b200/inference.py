@@ -10,7 +10,7 @@ import numpy as np
 import torch
 
 from .config import ConeConfig
-from .engine import ConeEngine, GroundingOutput, QueryBatch, pack_queries
+from .engine import ConeEngine, GroundingOutput, QueryBatch, host_feature_dtype, pack_queries
 
 MODES = ("fusion", "proposal", "matching")  # order of GroundingOutput.nms[:, m]
 
@@ -18,13 +18,14 @@ MODES = ("fusion", "proposal", "matching")  # order of GroundingOutput.nms[:, m]
 @dataclasses.dataclass
 class HostStep:
     """One step's inputs staged in pinned host memory."""
-    frames: torch.Tensor  # [n_frames, Dv] fp32 pinned
+    frames: torch.Tensor  # [n_frames, Dv] fp32 or fp16 pinned
     qb: QueryBatch  # pinned
     video_ids: List[int]
-    motion: Optional[torch.Tensor] = None  # [n_frames, Dm] fp32 pinned: separate motion stream, None = `frames`
+    motion: Optional[torch.Tensor] = None  # [n_frames, Dm] fp32 or fp16 pinned: separate motion stream, None = `frames`
 
     def h2d_bytes(self) -> int:
-        return self.frames.numel() * 4 + self.qb.h2d_bytes() + (self.motion.numel() * 4 if self.motion is not None else 0)
+        return (self.frames.numel() * self.frames.element_size() + self.qb.h2d_bytes() +
+                (self.motion.numel() * self.motion.element_size() if self.motion is not None else 0))
 
 
 def plan_steps(video_lengths: Sequence[int], queries, max_frames_per_step: int) -> List[List[int]]:
@@ -44,7 +45,11 @@ def plan_steps(video_lengths: Sequence[int], queries, max_frames_per_step: int) 
 def stage_step(cfg: ConeConfig, videos: Sequence[np.ndarray], queries, video_ids: Sequence[int], pin: bool = True,
                motion_videos: Optional[Sequence[np.ndarray]] = None) -> HostStep:
     """Concatenate the step's videos (and their motion features, when a separate motion stream is given) and pack
-    its queries (dataset order preserved within the step)."""
+    its queries (dataset order preserved within the step).  float16 features stay float16, each stream on its own;
+    a stream that mixes float16 with other types raises ValueError."""
+    host_feature_dtype([videos[v] for v in video_ids], "videos")
+    if motion_videos is not None:
+        host_feature_dtype([motion_videos[v] for v in video_ids], "motion features")
     vid_set = {v: i for i, v in enumerate(video_ids)}
     sel = [(i, q) for i, q in enumerate(queries) if q.video_idx in vid_set]
     local = [dataclasses.replace(q, video_idx=vid_set[q.video_idx]) for _, q in sel]
@@ -107,8 +112,10 @@ def ground_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, ma
     reference pools proposals over windows padded to the longest window of each `eval_bsz` batch of queries
     (SURVEY.md §8 A9), which is reproduced exactly when a step holds whole eval batches (always true for a
     single step).  `motion_videos[v]` [L_v, Dm]: raw features of a separate motion stream (`--motion_feat_dir`), the
-    input of Moment-DETR; None = the appearance features serve both roles."""
-    _check_streams(videos, motion_videos)
+    input of Moment-DETR; None = the appearance features serve both roles.  Videos, motion features and queries may
+    each be float32 or float16 (one type per stream): float16 is staged, copied and read as such, and the results are
+    bitwise those of the float32 upcast."""
+    _check_streams(videos, motion_videos, queries)
     res: Dict[str, dict] = {}
     lens = [len(v) for v in videos]
     for ids in plan_steps(lens, queries, max_frames_per_step):
@@ -120,9 +127,13 @@ def ground_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, ma
     return res
 
 
-def _check_streams(videos, motion_videos) -> None:
+def _check_streams(videos, motion_videos, queries) -> None:
     if motion_videos is not None and len(motion_videos) != len(videos):
         raise ValueError(f"{len(motion_videos)} motion feature tensors for {len(videos)} videos")
+    host_feature_dtype(videos, "videos")  # before any step runs
+    if motion_videos is not None:
+        host_feature_dtype(motion_videos, "motion features")
+    host_feature_dtype([q.tokens for q in queries] + [q.cls for q in queries], "queries")
 
 
 def to_submission(results: Dict[str, dict], annotations: Sequence[dict], mode: str = "fusion") -> List[dict]:
@@ -207,7 +218,7 @@ def evaluate_dataset(engine: ConeEngine, videos: Sequence[np.ndarray], queries, 
                      motion_videos: Optional[Sequence[np.ndarray]] = None) -> MetricCounters:
     """Stages 0-3 + metric counters over (this rank's share of) a dataset; only the counters are read back.
     `motion_videos` as in `ground_dataset`."""
-    _check_streams(videos, motion_videos)
+    _check_streams(videos, motion_videos, queries)
     counters = new_counters(engine.device, topk, thresholds, window_topk)
     lens = [len(v) for v in videos]
     mine = None if video_ids is None else set(video_ids)

@@ -34,26 +34,44 @@ def encode_record(compress: bool = True, **arrays) -> bytes:
         return w.getvalue()
 
 
-def decode_video_record(buf) -> np.ndarray:
-    """bytes -> raw features [L, Dv] float32 (ego4d_mad_dataloader.py:294-302 returns them un-normalised)."""
+def _as_feature(a: np.ndarray, dtype, key: str) -> np.ndarray:
+    """`a` as a contiguous array of `dtype` (float32 or float16).  float16 records pass through unchanged; wider
+    records are rounded once, and a finite value beyond the float16 range raises instead of becoming inf."""
+    dtype = np.dtype(dtype)
+    if dtype not in (np.dtype(np.float32), np.dtype(np.float16)):
+        raise ValueError(f"feature dtype must be float32 or float16, got {dtype}")
+    with np.errstate(over="ignore"):
+        out = np.ascontiguousarray(a, dtype=dtype)
+    if dtype == np.float16 and a.dtype != np.float16:
+        bad = np.isinf(out) & np.isfinite(a)
+        if bad.any():
+            raise ValueError(f"{key}: {int(bad.sum())} finite values exceed the float16 range "
+                             f"(largest magnitude {float(np.abs(a[bad]).max()):.6g})")
+    return out
+
+
+def decode_video_record(buf, dtype=np.float32, key: str = "video record") -> np.ndarray:
+    """bytes -> raw features [L, Dv] (ego4d_mad_dataloader.py:294-302 returns them un-normalised) as `dtype`:
+    float32 (the reference's type) or float16 (half the host, pinned and HBM footprint; see `_as_feature`).
+    `key` names the record in errors."""
     with io.BytesIO(bytes(buf)) as r:
         dump = np.load(r, allow_pickle=False)
         if "features" not in dump:
             raise KeyError("video record has no 'features' array")
-        return np.ascontiguousarray(dump["features"], dtype=np.float32)
+        return _as_feature(dump["features"], dtype, key)
 
 
-def decode_query_record(buf) -> Tuple[np.ndarray, np.ndarray]:
-    """bytes -> (token_features [n_tok, Dt], holistic feature [Dv]) float32, raw (ego4d_mad_dataloader.py:258-282):
-    `cls_features` if present, else `eot_features`; a [1, Dv] holistic feature is squeezed."""
+def decode_query_record(buf, dtype=np.float32, key: str = "query record") -> Tuple[np.ndarray, np.ndarray]:
+    """bytes -> (token_features [n_tok, Dt], holistic feature [Dv]) as `dtype` (float32 or float16), raw
+    (ego4d_mad_dataloader.py:258-282): `cls_features` if present, else `eot_features`; a [1, Dv] holistic feature is
+    squeezed."""
     with io.BytesIO(bytes(buf)) as r:
         dump = np.load(r, allow_pickle=False)
-        tok = np.ascontiguousarray(dump["token_features"], dtype=np.float32)
-        cls = dump["cls_features"] if "cls_features" in dump else dump["eot_features"]
-        cls = np.asarray(cls, dtype=np.float32)
+        tok = _as_feature(dump["token_features"], dtype, key)
+        cls = np.asarray(dump["cls_features"] if "cls_features" in dump else dump["eot_features"])
         if cls.ndim == 2:
             cls = cls[0]
-    return tok, np.ascontiguousarray(cls)
+    return tok, _as_feature(cls, dtype, key)
 
 
 # ------------------------------------------------------------------------------------------------ stores
@@ -97,12 +115,13 @@ class LmdbStore:
 
 
 # ------------------------------------------------------------------------------------------------ staging
-def load_queries(query_store, annotations: Sequence[dict], video_index: Dict[str, int]) -> List[SynthQuery]:
+def load_queries(query_store, annotations: Sequence[dict], video_index: Dict[str, int],
+                 feature_dtype=np.float32) -> List[SynthQuery]:
     """Annotation rows (query_id, clip_id, timestamps — ego4d_mad_dataloader.py:19-29) -> query objects in DATASET
-    order, features decoded from `query_store`."""
+    order, features decoded from `query_store` as `feature_dtype` (float32 or float16, see `decode_query_record`)."""
     out = []
     for a in annotations:
-        tok, cls = decode_query_record(query_store.get(a["query_id"]))
+        tok, cls = decode_query_record(query_store.get(a["query_id"]), feature_dtype, key=a["query_id"])
         ts = a.get("timestamps", (0.0, 0.0))
         out.append(SynthQuery(a["query_id"], video_index[a["clip_id"]], tok, cls, (float(ts[0]), float(ts[1]))))
     return out
@@ -115,11 +134,14 @@ class StagedSteps:
     SURVEY.md §8 A1)."""
 
     def __init__(self, cfg: ConeConfig, video_store, video_ids: Sequence[str], video_lengths: Sequence[int], queries,
-                 max_frames_per_step: int = 1 << 20, depth: int = 2, pin: bool = True, motion_store=None):
+                 max_frames_per_step: int = 1 << 20, depth: int = 2, pin: bool = True, motion_store=None,
+                 feature_dtype=np.float32):
         """`motion_store`: records of a separate motion stream under the same keys (`--motion_feat_dir`); None = the
-        appearance records serve both roles."""
+        appearance records serve both roles.  `feature_dtype` (float32 or float16): the type video and motion records
+        are decoded to and staged in (see `decode_video_record`)."""
         self.cfg, self.store, self.video_ids, self.queries, self.pin = cfg, video_store, list(video_ids), queries, pin
         self.motion_store = motion_store
+        self.feature_dtype = feature_dtype
         self.plan = plan_steps(video_lengths, queries, max_frames_per_step)
         self._q: "queue.Queue" = queue.Queue(maxsize=max(1, depth))
         self._stop = threading.Event()
@@ -142,9 +164,12 @@ class StagedSteps:
                 if self._stop.is_set():
                     return
                 # stage_step only indexes videos[v] for v in ids: a dict of this step's decoded arrays is enough
-                vids: Dict[int, np.ndarray] = {v: decode_video_record(self.store.get(self.video_ids[v])) for v in ids}
+                dt = self.feature_dtype
+                vids: Dict[int, np.ndarray] = {v: decode_video_record(self.store.get(self.video_ids[v]), dt,
+                                                                      key=self.video_ids[v]) for v in ids}
                 mot = None if self.motion_store is None else \
-                    {v: decode_video_record(self.motion_store.get(self.video_ids[v])) for v in ids}
+                    {v: decode_video_record(self.motion_store.get(self.video_ids[v]), dt, key=self.video_ids[v])
+                     for v in ids}
                 step = stage_step(self.cfg, vids, self.queries, ids, pin=self.pin, motion_videos=mot)
                 if not self._put(step):
                     return
@@ -182,21 +207,25 @@ class StagedSteps:
 
 
 def ground_store(engine, video_store, query_store, annotations: Sequence[dict], video_lengths: Optional[Dict[str, int]] = None,
-                 max_frames_per_step: int = 1 << 20, full: bool = False, motion_store=None) -> Dict[str, dict]:
+                 max_frames_per_step: int = 1 << 20, full: bool = False, motion_store=None,
+                 feature_dtype=np.float32) -> Dict[str, dict]:
     """`eval_epoch` stages 0-3 straight from feature stores: decode -> pinned -> HBM -> kernels, the decoding of the
     next step overlapping the kernels of the current one.  `video_lengths` (frames per clip_id) avoids a first pass
     over the video records when the annotations do not carry it.  `motion_store` holds the records of a separate
     motion stream (`--motion_feat_dir`) under the same clip ids, `features [L, Dm]`; None = the reference's
-    same-directory case."""
+    same-directory case.  `feature_dtype=np.float16` keeps every feature in float16 from the decoded record to HBM
+    (float16 records pass through, wider ones are rounded once on the host); the results are bitwise those of
+    `ground_dataset` on the same float16 arrays.  numpy has no bfloat16: bf16 features are reachable only through
+    `ConeEngine` with torch tensors."""
     from .inference import output_to_host, run_step
     clip_ids = list(dict.fromkeys(a["clip_id"] for a in annotations))
     index = {c: i for i, c in enumerate(clip_ids)}
     if video_lengths is None:
         video_lengths = {c: int(decode_video_record(video_store.get(c)).shape[0]) for c in clip_ids}
-    queries = load_queries(query_store, annotations, index)
+    queries = load_queries(query_store, annotations, index, feature_dtype)
     res: Dict[str, dict] = {}
     steps = StagedSteps(engine.cfg, video_store, clip_ids, [video_lengths[c] for c in clip_ids], queries,
-                        max_frames_per_step, motion_store=motion_store)
+                        max_frames_per_step, motion_store=motion_store, feature_dtype=feature_dtype)
     for step in steps:
         if step.qb.tok_len.numel() == 0:
             continue

@@ -9,9 +9,11 @@ replace `make_dataset` by `ingest.load_queries` + feature stores.
 from __future__ import annotations
 
 import argparse
+import dataclasses
 import json
 import os
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -30,6 +32,8 @@ def main() -> None:
     ap.add_argument("--frames", type=int, nargs=2, default=(300, 1500))
     ap.add_argument("--queries", type=int, default=6, help="queries per video")
     ap.add_argument("--motion-dim", type=int, default=0, help="width of a separate motion stream (0 = none)")
+    ap.add_argument("--feature-dtype", default="float32", choices=["float32", "float16"],
+                    help="storage type of the videos, motion features and queries")
     ap.add_argument("--precision", default="fp32")
     ap.add_argument("--flavour", default="mad", choices=["mad", "ego4d"])
     ap.add_argument("--seed", type=int, default=0)
@@ -47,13 +51,17 @@ def main() -> None:
     # with `queries` per video a multiple of eval_bsz every video holds whole batches
     cfg = cfg.replace(eval_bsz=a.queries, v_motion_feat_dim=a.motion_dim)
     ds = make_dataset(cfg, a.videos, None, a.queries, seed=a.seed, frames_range=tuple(a.frames), motion_dim=a.motion_dim)
+    fdt = np.dtype(a.feature_dtype)
+    videos = [v.astype(fdt) for v in ds.videos]
+    motion = None if ds.motion is None else [m.astype(fdt) for m in ds.motion]
+    queries = [dataclasses.replace(q, tokens=q.tokens.astype(fdt), cls=q.cls.astype(fdt)) for q in ds.queries]
     gt = {q.query_id: q.timestamps for q in ds.queries}
     costs = [video_cost(len(v), a.queries, cfg.topk_window) for v in ds.videos]
     mine = lpt_assign(costs, world)[rank]
     eng = ConeEngine(cfg, init_state_dict(cfg, a.seed), device=dev, precision=a.precision, workspace_bytes=4 << 30)
     # one video per step keeps the reference's eval-batch boundaries identical for every sharding
-    c = evaluate_dataset(eng, ds.videos, ds.queries, gt, flavour=a.flavour, max_frames_per_step=1, video_ids=mine,
-                         motion_videos=ds.motion)
+    c = evaluate_dataset(eng, videos, queries, gt, flavour=a.flavour, max_frames_per_step=1, video_ids=mine,
+                         motion_videos=motion)
     reduce_counters(c)
     if rank == 0:
         out = {"world": world, "n_queries": int(c.n_queries.item()), "window_recall": c.window_recall().tolist()}

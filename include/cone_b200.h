@@ -41,6 +41,13 @@ extern "C" {
 #define CONE_PREC_TC_SPLIT 2 /* cone_linear only: 3-product split-fp16 GEMM on tcgen05, fp32-class accuracy (what
                                 CONE_PREC_TC uses for the input projections and the span head) */
 
+/* storage type of a raw feature tensor (frames, motion rows, tokens, CLS) passed to an _ex entry point.  fp16 and bf16
+ * values convert to fp32 exactly and the kernels that read raw rows keep their fp32 reduction order, so a call on 16-bit
+ * features gives the same bits as the same call on the fp32 upcast.  A 16-bit feature pointer must be 8-byte aligned. */
+#define CONE_DTYPE_F32 0
+#define CONE_DTYPE_F16 1
+#define CONE_DTYPE_BF16 2
+
 /* Model / window hyper-parameters (cone/config.py:73-125; values per dataset in
  * cone/scripts/train_{ego4d,mad}.sh). */
 typedef struct cone_dims {
@@ -88,6 +95,9 @@ size_t cone_prepare_workspace_bytes(const cone_dims* dims, int64_t n_frames);
  * torch's F.normalize form x / max(||x||, -eps) (run_on_video/cone_localizator.py:127, 131).
  * In place if out == x. */
 int cone_l2_normalize(const float* x, float* out, int64_t rows, int32_t dim, float eps, void* stream);
+/* Same on x of storage type x_dtype (CONE_DTYPE_*); out stays fp32 (so out == x only for fp32).
+ * cone_l2_normalize == cone_l2_normalize_ex(x_dtype CONE_DTYPE_F32). */
+int cone_l2_normalize_ex(const void* x, int32_t x_dtype, float* out, int64_t rows, int32_t dim, float eps, void* stream);
 
 /* ---- A2  stage 0 (cone/inference.py:250-260) + per-frame `input_vid_proj` (cone/model.py:100).
  * frames_raw [n_frames, Dv] raw features.  ctx_out [n_frames, Dv] = normalised adapted context
@@ -97,6 +107,11 @@ int cone_l2_normalize(const float* x, float* out, int64_t rows, int32_t dim, flo
  * m_dim != v_dim a non-NULL vidproj_out is CONE_ERR_INVALID (use cone_video_prepare_motion). */
 int cone_video_prepare(const cone_weights* w, const float* frames_raw, int64_t n_frames, float* ctx_out,
                        float* vidproj_out, void* workspace, size_t workspace_bytes, int precision, void* stream);
+/* Same on frames_raw of storage type frames_dtype (CONE_DTYPE_*); outputs stay fp32.
+ * cone_video_prepare == cone_video_prepare_ex(frames_dtype CONE_DTYPE_F32). */
+int cone_video_prepare_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t n_frames,
+                          float* ctx_out, float* vidproj_out, void* workspace, size_t workspace_bytes, int precision,
+                          void* stream);
 
 /* Per-frame `input_vid_proj` of a separate motion stream (--motion_feat_dir): motion_raw [n_frames, Dm] raw features
  * are L2-normalised per frame, x / (||x|| + 1e-5) (cone/ego4d_mad_dataloader.py:284-292), then projected:
@@ -104,6 +119,10 @@ int cone_video_prepare(const cone_weights* w, const float* frames_raw, int64_t n
  * (cone_prepare_workspace_bytes); the result does not depend on the slab size. */
 int cone_video_prepare_motion(const cone_weights* w, const float* motion_raw, int64_t n_frames, float* vidproj_out,
                               void* workspace, size_t workspace_bytes, int precision, void* stream);
+/* Same on motion_raw of storage type motion_dtype (CONE_DTYPE_*); vidproj_out stays fp32.
+ * cone_video_prepare_motion == cone_video_prepare_motion_ex(motion_dtype CONE_DTYPE_F32). */
+int cone_video_prepare_motion_ex(const cone_weights* w, const void* motion_raw, int32_t motion_dtype, int64_t n_frames,
+                                 float* vidproj_out, void* workspace, size_t workspace_bytes, int precision, void* stream);
 
 /* `adapter_layer(x) + x` on arbitrary rows (cone/model.py:80; inference.py:255): the
  * `model.adapter_layer` attribute of the drop-in surface. `residual` = 1 adds x. */
@@ -161,6 +180,11 @@ int cone_window_ranklist(const float* frame_score, const int64_t* score_offsets,
 size_t cone_prefilter_workspace_bytes(const cone_dims* dims, int64_t n_frames, int32_t n_queries);
 int cone_prefilter(const cone_weights* w, const float* frames_raw, int64_t n_frames, const float* cls_raw, int32_t n_queries,
                    int32_t topk, int32_t* win_idx, float* win_score, void* workspace, size_t workspace_bytes, void* stream);
+/* Same with frames_raw of storage type frames_dtype and cls_raw of storage type cls_dtype (CONE_DTYPE_*, independent).
+ * cone_prefilter == cone_prefilter_ex(both CONE_DTYPE_F32). */
+int cone_prefilter_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t n_frames,
+                      const void* cls_raw, int32_t cls_dtype, int32_t n_queries, int32_t topk, int32_t* win_idx,
+                      float* win_score, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- A4-A9  stage 2: slice the top-k windows of every query straight out of the frame tensors,
  * run Moment-DETR on them and score the proposals (cone/ego4d_mad_dataloader.py:144-159, 305-358;
@@ -184,6 +208,14 @@ int cone_ground_windows(const cone_weights* w, const float* frames_raw, int64_t 
                         const int32_t* q_batch, int32_t n_batches, int32_t n_queries, int32_t topk,
                         float* pred_spans, float* prob_fg, float* match, int32_t* win_start, int32_t* win_len,
                         void* workspace, size_t workspace_bytes, int precision, void* stream);
+/* Same with frames_raw (the rows pooled for matching) of storage type frames_dtype (CONE_DTYPE_*); every other
+ * input is fp32 as above.  cone_ground_windows == cone_ground_windows_ex(frames_dtype CONE_DTYPE_F32). */
+int cone_ground_windows_ex(const cone_weights* w, const void* frames_raw, int32_t frames_dtype, int64_t n_frames,
+                           const float* vidproj, const int64_t* q_video_start, const int32_t* q_video_len,
+                           const int32_t* ranklist, int32_t ranklist_stride, const float* tok, const int32_t* tok_len,
+                           const float* cls_norm, const int32_t* q_batch, int32_t n_batches, int32_t n_queries,
+                           int32_t topk, float* pred_spans, float* prob_fg, float* match, int32_t* win_start,
+                           int32_t* win_len, void* workspace, size_t workspace_bytes, int precision, void* stream);
 
 /* ---- A6-A8  reference-shaped forward: `model(src_txt, src_txt_mask, src_vid_motion,
  * src_vid_motion_mask)` (cone/model.py:82-128).  src_vid [B, Lv, Dm] (= src_vid_motion), src_txt [B, Lt, Dt], valid
