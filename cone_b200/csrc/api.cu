@@ -199,13 +199,14 @@ static int check_dims(const cone_dims* c) {
     CONE_REQUIRE(c->ffn > 0 && c->ffn % 16 == 0, "dim_feedforward must be a multiple of 16");
     CONE_REQUIRE(c->enc_layers >= 1 && c->dec_layers >= 1 && c->enc_layers <= 8 && c->dec_layers <= 8, "1..8 layers");
     CONE_REQUIRE(c->num_queries >= 1 && c->num_queries <= 8, "1..8 moment slots");
-    CONE_REQUIRE(c->max_v_l >= 2 && c->max_q_l >= 1 && c->max_v_l + c->max_q_l <= 256,
-                 "window (max_v_l + max_q_l) must fit 256 rows");
+    // windows of up to 256 rows run the short-window attention kernels, 257..512 rows their long-window variants
+    CONE_REQUIRE(c->max_v_l >= 2 && c->max_q_l >= 1 && c->max_v_l + c->max_q_l <= CONE_MAX_WINDOW_ROWS,
+                 "window (max_v_l + max_q_l = %d) must fit %d rows", c->max_v_l + c->max_q_l, CONE_MAX_WINDOW_ROWS);
     return CONE_OK;
 }
 
 extern "C" const char* cone_last_error(void) { return g_err; }
-extern "C" int cone_version(void) { return 3; }
+extern "C" int cone_version(void) { return 4; }
 extern "C" int64_t cone_launch_count(void) { return g_launches; }
 extern "C" void cone_launch_count_reset(void) { g_launches = 0; }
 
@@ -1371,7 +1372,8 @@ extern "C" int cone_forward(const cone_weights* w, const float* src_txt, const i
     CONE_TRY(check_prec(precision));
     const cone_dims& dm = w->dims;
     CONE_REQUIRE(Lv >= 1 && Lv <= dm.max_v_l, "cone_forward: L_vid=%d exceeds max_v_l=%d of the weights handle", Lv, dm.max_v_l);
-    CONE_REQUIRE(Lt >= 1 && Lv + Lt <= 256, "cone_forward: window of %d rows exceeds 256", Lv + Lt);
+    CONE_REQUIRE(Lt >= 1 && Lv + Lt <= CONE_MAX_WINDOW_ROWS, "cone_forward: window of %d rows exceeds %d", Lv + Lt,
+                 CONE_MAX_WINDOW_ROWS);
     if (B == 0) return CONE_OK;
     Ctx c{w, precision, (cudaStream_t)stream};
     CONE_TRY(ensure_tc(w, precision, c.s));

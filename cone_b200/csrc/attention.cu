@@ -1,4 +1,5 @@
-// Small-sequence multi-head attention for Moment-DETR windows (S = Lv + Lt <= 256 rows, head_dim 32).
+// Small-sequence multi-head attention for Moment-DETR windows (S = Lv + Lt <= 512 rows, head_dim 32).  Windows of up
+// to 256 rows run the kernels sized for them; longer windows (256 < S <= 512) run the long-window variants below.
 // Math follows torch.nn.functional.multi_head_attention_forward as called at cone/transformer.py:239,
 // 304, 308: q scaled by sqrt(1/head_dim) BEFORE the dot product, additive -inf key-padding mask,
 // softmax over keys, then P.V.  One CTA per (window, head); K and V of the head live in shared memory.
@@ -12,7 +13,8 @@ namespace cone {
 namespace {
 
 constexpr int HD = 32;            // head dim (hidden 256 / 8 heads)
-constexpr int MAX_S = 256;        // max keys per window
+constexpr int MAX_S = 256;        // max keys per window of the short-window kernels
+constexpr int MAX_S_LONG = 512;   // max keys per window of the long-window variants
 constexpr int ENC_WARPS = 4;
 
 __device__ __forceinline__ float fast_exp2(float x) {
@@ -23,6 +25,8 @@ __device__ __forceinline__ float fast_exp2(float x) {
 
 __device__ __forceinline__ bool key_valid(int j, int Lv, int vl, int tl) { return j < Lv ? (j < vl) : ((j - Lv) < tl); }
 
+// KPL = keys per lane: MAX_S / 32, or MAX_S_LONG / 32 for long windows
+template <int KPL>
 __global__ void __launch_bounds__(ENC_WARPS * 32)
 enc_self_attention_kernel(const float* __restrict__ qk, int64_t ldqk, const float* __restrict__ v, int64_t ldv,
                           float* __restrict__ o, int64_t ldo, const int32_t* __restrict__ vlen,
@@ -47,7 +51,6 @@ enc_self_attention_kernel(const float* __restrict__ qk, int64_t ldqk, const floa
     }
     __syncthreads();
 
-    constexpr int KPL = MAX_S / 32;  // keys per lane
     for (int i = warp; i < S; i += ENC_WARPS) {
         Qs[warp * HD + lane] = qk[(row0 + i) * ldqk + h * HD + lane] * scale;
         __syncwarp();
@@ -201,7 +204,8 @@ struct XChunk<float> {
     }
 };
 
-template <typename KV, int NQ>
+// KPL = scores per lane in phase 2: MAX_S / 32, or MAX_S_LONG / 32 for long windows
+template <typename KV, int NQ, int KPL>
 __global__ void __launch_bounds__(256, 2)
 dec_cross_attention_kernel(const float* __restrict__ q, int64_t ldq, const KV* __restrict__ k, int64_t ldk,
                            const KV* __restrict__ v, int64_t ldv, float* __restrict__ o, int64_t ldo,
@@ -278,10 +282,10 @@ dec_cross_attention_kernel(const float* __restrict__ q, int64_t ldq, const KV* _
     // phase 2: each lane keeps its (at most 8) scores of the row in registers
     for (int r = warp; r < H * NQ; r += 8) {
         float* row = Ps + r * Sp;
-        float a[MAX_S / 32];
+        float a[KPL];
         float mx = -CUDART_INF_F;
 #pragma unroll
-        for (int t = 0; t < MAX_S / 32; ++t) {
+        for (int t = 0; t < KPL; ++t) {
             const int j = lane + 32 * t;
             a[t] = j < S ? row[j] : -CUDART_INF_F;
             mx = fmaxf(mx, a[t]);
@@ -289,7 +293,7 @@ dec_cross_attention_kernel(const float* __restrict__ q, int64_t ldq, const KV* _
         mx = warp_max(mx);
         float sum = 0.f;
 #pragma unroll
-        for (int t = 0; t < MAX_S / 32; ++t) {
+        for (int t = 0; t < KPL; ++t) {
             const int j = lane + 32 * t;
             float e;
             if (sizeof(KV) == 2) {  // reduced-precision mode: exp2 with the hardware approximation (2^-22 relative)
@@ -628,6 +632,226 @@ enc_attention_f16_kernel(const __half* __restrict__ qk, int64_t ldqk, const __ha
     }
 }
 
+// Long windows (256 < S <= 512 keys): the kernel above issues the loads of the whole tile before the first use and keeps
+// half a score row block in registers, and neither fits at 64 key blocks.  Same inputs (dense rows or the layer-0 row
+// tables, the per-layer position table) and the same arithmetic per key block; what changes:
+//   - 16 warps, the tile loaded in rounds of LA_ROUND rows per thread (3 x LA_ROUND 16-byte loads in flight);
+//   - online softmax over chunks of LA_CH key blocks (64 keys): a running (max, sum) per row, the accumulators of P.V and
+//     of the row sums rescaled when the maximum grows;
+//   - only the key blocks that hold a valid-length key are visited (the others are text padding: their P is exactly 0).
+// Shared memory is the same [Sp][QK_PAD] x 3 tile (123 KB at S = 512): one CTA per SM at 512 rows.
+constexpr int LA_WARPS = 16;
+constexpr int LA_ROUND = 4;  // load iterations per round
+constexpr int LA_CH = 8;     // key blocks per chunk of the online softmax
+
+__global__ void __launch_bounds__(LA_WARPS * 32, 1)
+enc_attention_f16_long_kernel(const __half* __restrict__ qk, int64_t ldqk, const __half* __restrict__ v, int64_t ldv,
+                              __half* __restrict__ o, int64_t ldo, const int32_t* __restrict__ vlen,
+                              const int32_t* __restrict__ tlen, int Lv, int Lt, int d_model,
+                              const __half* __restrict__ posqk, int table_lv, EncRowSource src) {
+    extern __shared__ __align__(16) unsigned char att_smem[];
+    const int S = Lv + Lt;
+    const int Sp = (S + 15) & ~15;
+    __half* Qs = reinterpret_cast<__half*>(att_smem);  // [Sp][QK_PAD]
+    __half* Ks = Qs + Sp * QK_PAD;                      // [Sp][QK_PAD]
+    __half* Vs = Ks + Sp * QK_PAD;                      // [Sp][QK_PAD]
+    float* mbias = reinterpret_cast<float*>(Vs + Sp * QK_PAD);  // [Sp]
+    const int nheads = d_model / HD;
+    const int64_t b = blockIdx.x / nheads;
+    const int h = blockIdx.x % nheads;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t row0 = b * S;
+    const int vl = vlen[b], tl = tlen[b];
+
+    constexpr int ROWS_PER_IT = LA_WARPS * 32 / 4;  // 4 threads per row
+    const int r0 = threadIdx.x >> 2, c8 = (threadIdx.x & 3) * 8 + h * HD;
+    const bool indirect = src.frames != nullptr;
+    const int64_t vbase = indirect ? src.vid_base[b] : 0;
+    const int64_t tbase = indirect ? src.txt_base[b] : 0;
+    const __half* qp = qk + (row0 + r0) * ldqk + c8;
+    const __half* vp = v + (row0 + r0) * ldv + c8;
+    const __half* pp = posqk + ((int64_t)vl * table_lv + r0) * (2 * d_model) + c8;
+    unsigned char* sbase = att_smem + (r0 * QK_PAD + (threadIdx.x & 3) * 8) * 2;
+    const int mat_bytes = Sp * QK_PAD * 2;
+    for (int it0 = 0; it0 * ROWS_PER_IT < Sp; it0 += LA_ROUND) {
+        uint4 q4[LA_ROUND], k4[LA_ROUND], v4[LA_ROUND];
+#pragma unroll
+        for (int u = 0; u < LA_ROUND; ++u) {
+            const int it = it0 + u;
+            const int r = r0 + it * ROWS_PER_IT;
+            q4[u] = make_uint4(0, 0, 0, 0);
+            k4[u] = q4[u];
+            v4[u] = q4[u];
+            if (r < S) {
+                if (indirect) {
+                    const __half* row;
+                    if (r < Lv) {
+                        int64_t fr = vbase + r;  // rows past the tensor end belong to masked keys: never read out of bounds
+                        fr = fr < src.n_frames ? fr : src.n_frames - 1;
+                        row = src.frames + fr * (3 * d_model) + c8;
+                    } else {
+                        row = src.tokens + (tbase + (r - Lv)) * (3 * d_model) + c8;
+                    }
+                    q4[u] = *reinterpret_cast<const uint4*>(row);
+                    k4[u] = *reinterpret_cast<const uint4*>(row + d_model);
+                    v4[u] = *reinterpret_cast<const uint4*>(row + 2 * d_model);
+                } else {
+                    q4[u] = *reinterpret_cast<const uint4*>(qp + (int64_t)it * ROWS_PER_IT * ldqk);
+                    k4[u] = *reinterpret_cast<const uint4*>(qp + (int64_t)it * ROWS_PER_IT * ldqk + d_model);
+                    v4[u] = *reinterpret_cast<const uint4*>(vp + (int64_t)it * ROWS_PER_IT * ldv);
+                }
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < LA_ROUND; ++u) {
+            const int it = it0 + u;
+            const int r = r0 + it * ROWS_PER_IT;
+            if (r < Sp) {
+                if (posqk != nullptr && r < Lv) {  // q | k + pos . [Wq; Wk]^T, one fp16 rounding (as the kernel above)
+                    const __half* pr = pp + (int64_t)it * ROWS_PER_IT * 2 * d_model;
+                    const uint4 pq = __ldg(reinterpret_cast<const uint4*>(pr));
+                    const uint4 pk = __ldg(reinterpret_cast<const uint4*>(pr + d_model));
+                    __half2* qh = reinterpret_cast<__half2*>(&q4[u]);
+                    __half2* kh = reinterpret_cast<__half2*>(&k4[u]);
+                    const __half2* pqh = reinterpret_cast<const __half2*>(&pq);
+                    const __half2* pkh = reinterpret_cast<const __half2*>(&pk);
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) {
+                        qh[e] = __hadd2(qh[e], pqh[e]);
+                        kh[e] = __hadd2(kh[e], pkh[e]);
+                    }
+                }
+                unsigned char* sp = sbase + it * ROWS_PER_IT * QK_PAD * 2;
+                *reinterpret_cast<uint4*>(sp) = q4[u];
+                *reinterpret_cast<uint4*>(sp + mat_bytes) = k4[u];
+                *reinterpret_cast<uint4*>(sp + 2 * mat_bytes) = v4[u];
+            }
+        }
+    }
+    for (int key = threadIdx.x; key < Sp; key += blockDim.x)
+        mbias[key] = (key < S && key_valid(key, Lv, vl, tl)) ? 0.f : -CUDART_INF_F;
+    __syncthreads();
+
+    const int nrb = Sp >> 4;
+    const int g = lane >> 2, t4 = lane & 3;
+    const int l8 = lane & 7, lq = lane >> 3;
+    const float sl2 = 0.17677669529663687f * 1.4426950408889634f;
+    // bit jb of word jb / 32 set = key block jb touches a padded key (64 blocks: two ballots)
+    uint32_t blkflags[2];
+#pragma unroll
+    for (int w = 0; w < 2; ++w) {
+        const int k0 = (w * 32 + lane) * 8, k1 = k0 + 8;
+        const bool all_valid = (k1 <= vl) || (k1 <= Lv + tl && (vl == Lv || k0 >= Lv));
+        blkflags[w] = __ballot_sync(0xffffffffu, !all_valid);
+    }
+    const int nrb_live = (Lv + tl + 15) >> 4;
+    const int nkb_live = (Lv + tl + 7) >> 3;  // key blocks from here on hold only padding
+    const int nch = (nkb_live + LA_CH - 1) / LA_CH;
+    for (int rb = warp; rb < nrb; rb += LA_WARPS) {
+        const int r_lo = rb * 16 + g, r_hi = r_lo + 8;
+        if (rb >= nrb_live) {  // warp-uniform: text padding rows, zeros
+#pragma unroll
+            for (int nb = 0; nb < 4; ++nb) {
+                if (r_lo < S) *reinterpret_cast<uint32_t*>(o + (row0 + r_lo) * ldo + h * HD + nb * 8 + t4 * 2) = 0u;
+                if (r_hi < S) *reinterpret_cast<uint32_t*>(o + (row0 + r_hi) * ldo + h * HD + nb * 8 + t4 * 2) = 0u;
+            }
+            continue;
+        }
+        uint32_t aq[2][4];
+#pragma unroll
+        for (int ks = 0; ks < 2; ++ks)
+            ldsm_x4(aq[ks], Qs + (rb * 16 + l8 + (lq & 1) * 8) * QK_PAD + ks * 16 + (lq >> 1) * 8);
+        float m_lo = -CUDART_INF_F, m_hi = -CUDART_INF_F;
+        float rs[4] = {0.f, 0.f, 0.f, 0.f};
+        const uint32_t ones = g == 0 ? 0x3C003C00u : 0u;
+        float out[4][4];
+#pragma unroll
+        for (int nb = 0; nb < 4; ++nb) out[nb][0] = out[nb][1] = out[nb][2] = out[nb][3] = 0.f;
+        for (int ch = 0; ch < nch; ++ch) {
+            const int jb0 = ch * LA_CH;
+            const uint32_t fl = (jb0 < 32 ? blkflags[0] : blkflags[1]) >> (jb0 & 31);  // a chunk lies within one word
+            float sc[LA_CH][4];
+            float c_lo = -CUDART_INF_F, c_hi = -CUDART_INF_F;
+#pragma unroll
+            for (int jj = 0; jj < LA_CH; ++jj) {
+                const int jb = jb0 + jj;
+                sc[jj][0] = sc[jj][1] = sc[jj][2] = sc[jj][3] = -CUDART_INF_F;
+                if (jb < nkb_live) {  // warp-uniform
+                    sc[jj][0] = sc[jj][1] = sc[jj][2] = sc[jj][3] = 0.f;
+                    uint32_t bk[4];
+                    ldsm_x4(bk, Ks + (jb * 8 + l8) * QK_PAD + lq * 8);
+                    mma_16816(sc[jj], aq[0], bk[0], bk[1]);
+                    mma_16816(sc[jj], aq[1], bk[2], bk[3]);
+                    if (fl & (1u << jj)) {
+                        const float2 mb = *reinterpret_cast<const float2*>(mbias + jb * 8 + t4 * 2);
+                        sc[jj][0] += mb.x; sc[jj][1] += mb.y;
+                        sc[jj][2] += mb.x; sc[jj][3] += mb.y;
+                    }
+                    c_lo = fmaxf(c_lo, fmaxf(sc[jj][0], sc[jj][1]));
+                    c_hi = fmaxf(c_hi, fmaxf(sc[jj][2], sc[jj][3]));
+                }
+            }
+            c_lo = fmaxf(c_lo, __shfl_xor_sync(0xffffffffu, c_lo, 1));
+            c_lo = fmaxf(c_lo, __shfl_xor_sync(0xffffffffu, c_lo, 2));
+            c_hi = fmaxf(c_hi, __shfl_xor_sync(0xffffffffu, c_hi, 1));
+            c_hi = fmaxf(c_hi, __shfl_xor_sync(0xffffffffu, c_hi, 2));
+            const float n_lo = fmaxf(m_lo, c_lo), n_hi = fmaxf(m_hi, c_hi);
+            const float o_lo = n_lo == -CUDART_INF_F ? 0.f : -n_lo * sl2;
+            const float o_hi = n_hi == -CUDART_INF_F ? 0.f : -n_hi * sl2;
+            if (ch > 0) {  // exp2(-inf) = 0: a row with no valid key so far has nothing to rescale
+                const float f_lo = fast_exp2(fmaf(m_lo, sl2, o_lo)), f_hi = fast_exp2(fmaf(m_hi, sl2, o_hi));
+                rs[0] *= f_lo;
+                rs[2] *= f_hi;
+#pragma unroll
+                for (int nb = 0; nb < 4; ++nb) {
+                    out[nb][0] *= f_lo; out[nb][1] *= f_lo;
+                    out[nb][2] *= f_hi; out[nb][3] *= f_hi;
+                }
+            }
+            m_lo = n_lo;
+            m_hi = n_hi;
+#pragma unroll
+            for (int jj = 0; jj < LA_CH; ++jj) {
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    sc[jj][e] = fast_exp2(fmaf(sc[jj][e], sl2, o_lo));
+                    sc[jj][2 + e] = fast_exp2(fmaf(sc[jj][2 + e], sl2, o_hi));
+                }
+            }
+#pragma unroll
+            for (int kk = 0; kk < LA_CH / 2; ++kk) {
+                const int kb = jb0 / 2 + kk;  // k-step of 16 keys
+                if (kb * 2 < nkb_live) {
+                    uint32_t ap[4];
+                    ap[0] = pack_half2(sc[2 * kk][0], sc[2 * kk][1]);
+                    ap[1] = pack_half2(sc[2 * kk][2], sc[2 * kk][3]);
+                    ap[2] = pack_half2(sc[2 * kk + 1][0], sc[2 * kk + 1][1]);
+                    ap[3] = pack_half2(sc[2 * kk + 1][2], sc[2 * kk + 1][3]);
+#pragma unroll
+                    for (int np = 0; np < 2; ++np) {
+                        uint32_t bv[4];
+                        ldsm_x4_trans(bv, Vs + (kb * 16 + l8 + (lq & 1) * 8) * QK_PAD + (np * 2 + (lq >> 1)) * 8);
+                        mma_16816(out[np * 2], ap, bv[0], bv[1]);
+                        mma_16816(out[np * 2 + 1], ap, bv[2], bv[3]);
+                    }
+                    mma_16816(rs, ap, ones, ones);  // row sums over the fp16 values of P
+                }
+            }
+        }
+        const float s_lo = __shfl_sync(0xffffffffu, rs[0], lane & ~3), s_hi = __shfl_sync(0xffffffffu, rs[2], lane & ~3);
+        const float i_lo = 1.f / s_lo, i_hi = 1.f / s_hi;
+#pragma unroll
+        for (int nb = 0; nb < 4; ++nb) {
+            if (r_lo < S)
+                *reinterpret_cast<uint32_t*>(o + (row0 + r_lo) * ldo + h * HD + nb * 8 + t4 * 2) =
+                    pack_half2(out[nb][0] * i_lo, out[nb][1] * i_lo);
+            if (r_hi < S)
+                *reinterpret_cast<uint32_t*>(o + (row0 + r_hi) * ldo + h * HD + nb * 8 + t4 * 2) =
+                    pack_half2(out[nb][2] * i_hi, out[nb][3] * i_hi);
+        }
+    }
+}
+
 
 // ------------------------------------------------------------------------------------------------
 // Memory-direct decoder cross-attention (CONE_PREC_TC).  The K and V projections of the memory are never formed:
@@ -850,6 +1074,217 @@ dec_cross_attention_mem_kernel(const __half* __restrict__ mem, int64_t ldm, cons
     }
 }
 
+// Long windows (256 < S <= 512): 512 memory rows at 528 B would need 270 KB of shared memory.  This variant streams the
+// memory through two buffers of XL_KC rows (cp.async: chunk c + 1 is in flight while chunk c is multiplied), with an
+// online softmax across chunks: an fp32 running maximum per score row (shared by the two warps of a row block through
+// shared memory), fp32 partial row sums and P.M accumulators rescaled whenever the maximum grows.  Per chunk the
+// arithmetic is that of the kernel above: content term over the 256 channels, position term through the pos.Wk^T
+// table, masked exp2 softmax with P rounded to fp16 and the row sums taken over the rounded values, P.M with
+// transposing ldmatrix.  The qt rows stay in shared memory (their fragments are re-read per chunk) and P has its own
+// buffer.  Shared memory at MT = 4: 2 x 66 KB (memory) + 33 KB (qt) + 17 KB (P) = 183 KB, one CTA per SM.
+constexpr int XL_KC = 128;  // memory rows per chunk
+
+template <int MT>
+__global__ void __launch_bounds__(MT * 64, 1)
+dec_cross_attention_mem_long_kernel(const __half* __restrict__ mem, int64_t ldm, const __half* __restrict__ qqt, int64_t ldq,
+                                    __half* __restrict__ pm, int64_t ldp, const int32_t* __restrict__ vlen,
+                                    const int32_t* __restrict__ tlen, int nq, int Lv, int Lt,
+                                    const __half* __restrict__ posk, int64_t ldposk, int table_lv, int q_bcast) {
+    constexpr int D = 256;
+    constexpr int NW = MT * 2;         // warps
+    constexpr int NJ = XL_KC / 16;     // key blocks of a chunk per warp (the two warps of a row block: even / odd)
+    constexpr int PS_PAD = XL_KC + 8;  // halves per row of P (272-byte stride: conflict-free stores and ldmatrix)
+    extern __shared__ __align__(16) unsigned char xsm[];
+    __half* Ms = reinterpret_cast<__half*>(xsm);          // [2][XL_KC][XM_PAD] memory chunks (rows >= S are zero)
+    __half* Qt = Ms + 2 * XL_KC * XM_PAD;                 // [MT * 16][XM_PAD] qt rows, row = head * nq + slot
+    __half* Ps = Qt + MT * 16 * XM_PAD;                   // [MT * 16][PS_PAD] P of the current chunk
+    float* red = reinterpret_cast<float*>(Ps + MT * 16 * PS_PAD);  // [MT][2 halves][16 rows][max, sum]
+    const int64_t b = blockIdx.x;
+    const int S = Lv + Lt;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int mt = warp >> 1, half = warp & 1;
+    const int64_t row0 = b * S;
+    const int R = 8 * nq;
+    const int nch = (S + XL_KC - 1) / XL_KC;
+
+    auto load_chunk = [&](int c) {  // one row per warp and iteration, 32 chunks of 16 bytes per row
+        const int k0 = c * XL_KC;
+        const __half* src = mem + (row0 + k0 + warp) * ldm + lane * 8;
+        __half* dst = Ms + (c & 1) * XL_KC * XM_PAD + warp * XM_PAD + lane * 8;
+#pragma unroll 4
+        for (int r = warp; r < XL_KC; r += NW) {
+            if (k0 + r < S) cp_async16(dst, src);
+            else *reinterpret_cast<uint4*>(dst) = make_uint4(0u, 0u, 0u, 0u);
+            src += (int64_t)NW * ldm;
+            dst += NW * XM_PAD;
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");
+    };
+    for (int r = warp; r < MT * 16; r += NW) {
+        __half* qd = Qt + r * XM_PAD + lane * 8;
+        if (r < R) {
+            const int hh = r / nq, slot = r - hh * nq;
+            cp_async16(qd, qqt + ((q_bcast ? 0 : b * nq) + slot) * ldq + D + hh * D + lane * 8);
+        } else {
+            *reinterpret_cast<uint4*>(qd) = make_uint4(0u, 0u, 0u, 0u);
+        }
+    }
+    load_chunk(0);  // the same commit group as the qt rows
+
+    const int vl = vlen[b], tl = tlen[b];
+    const int g = lane >> 2, t4 = lane & 3;
+    const int l8 = lane & 7, lq = lane >> 3;
+    const int r_lo = mt * 16 + g, r_hi = r_lo + 8;
+    const int h_lo = r_lo < R ? r_lo / nq : -1, h_hi = r_hi < R ? r_hi / nq : -1;
+    const int64_t q_lo = r_lo < R ? (b * nq + (r_lo - h_lo * nq)) : 0, q_hi = r_hi < R ? (b * nq + (r_hi - h_hi * nq)) : 0;
+    const int64_t qs_lo = (q_bcast && r_lo < R) ? q_lo - b * nq : q_lo, qs_hi = (q_bcast && r_hi < R) ? q_hi - b * nq : q_hi;
+    const int h_first = (mt * 16) / nq;
+    const int h_last = min(7, (mt * 16 + 15) / nq);
+    float* my_red = red + ((mt * 2 + half) * 16) * 2;
+    const float* other_red = red + ((mt * 2 + (half ^ 1)) * 16) * 2;
+
+    float m_lo = -CUDART_INF_F, m_hi = -CUDART_INF_F;  // running maxima (the same in both warps of the row block)
+    float s_lo = 0.f, s_hi = 0.f;                      // this lane's part of the row sums, against the running maxima
+    float out[16][4];
+#pragma unroll
+    for (int nt = 0; nt < 16; ++nt) out[nt][0] = out[nt][1] = out[nt][2] = out[nt][3] = 0.f;
+    for (int c = 0; c < nch; ++c) {
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
+        __syncthreads();  // chunk c is in place; every warp is done with chunk c - 1 (its buffer, P and the maxima)
+        if (c + 1 < nch) load_chunk(c + 1);
+        const __half* Mc = Ms + (c & 1) * XL_KC * XM_PAD;
+        const int k0 = c * XL_KC;
+        float sc[NJ][4];  // key block jb = 2 j + half of the chunk
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) sc[j][0] = sc[j][1] = sc[j][2] = sc[j][3] = 0.f;
+#pragma unroll
+        for (int ks = 0; ks < 16; ++ks) {  // content term: 16 k-steps over the 256 channels
+            uint32_t aq[4];
+            ldsm_x4(aq, Qt + (mt * 16 + l8 + (lq & 1) * 8) * XM_PAD + ks * 16 + (lq >> 1) * 8);
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) {
+                uint32_t b0, b1;
+                ldsm_x2(b0, b1, Mc + ((2 * j + half) * 8 + l8) * XM_PAD + ks * 16 + (lq & 1) * 8);
+                mma_16816(sc[j], aq, b0, b1);
+            }
+        }
+        if (posk != nullptr && k0 < Lv) {  // position term of the video keys of this chunk, two heads per pass
+            for (int hh = h_first; hh <= h_last; hh += 2) {
+                uint32_t a[2][2][4];
+                uint4 pf[2][NJ];
+#pragma unroll
+                for (int u = 0; u < 2; ++u) {
+                    const int hu = hh + u;
+                    uint4 xl = make_uint4(0u, 0u, 0u, 0u), xh = xl;
+                    if (h_lo == hu) xl = *reinterpret_cast<const uint4*>(qqt + qs_lo * ldq + hu * HD + t4 * 8);
+                    if (h_hi == hu) xh = *reinterpret_cast<const uint4*>(qqt + qs_hi * ldq + hu * HD + t4 * 8);
+                    a[u][0][0] = xl.x; a[u][0][1] = xh.x; a[u][0][2] = xl.y; a[u][0][3] = xh.y;
+                    a[u][1][0] = xl.z; a[u][1][1] = xh.z; a[u][1][2] = xl.w; a[u][1][3] = xh.w;
+                    const __half* pbase = posk + ((int64_t)vl * table_lv + k0 + half * 8 + g) * ldposk + hu * HD + t4 * 8;
+#pragma unroll
+                    for (int j = 0; j < NJ; ++j) {
+                        pf[u][j] = make_uint4(0u, 0u, 0u, 0u);
+                        if (hu <= h_last && k0 + (2 * j + half) * 8 + g < Lv)
+                            pf[u][j] = __ldg(reinterpret_cast<const uint4*>(pbase + (int64_t)j * 16 * ldposk));
+                    }
+                }
+#pragma unroll
+                for (int u = 0; u < 2; ++u) {
+                    if (hh + u <= h_last) {  // warp-uniform
+#pragma unroll
+                        for (int j = 0; j < NJ; ++j) mma_16816(sc[j], a[u][0], pf[u][j].x, pf[u][j].y);
+#pragma unroll
+                        for (int j = 0; j < NJ; ++j) mma_16816(sc[j], a[u][1], pf[u][j].z, pf[u][j].w);
+                    }
+                }
+            }
+        }
+        // mask, chunk maxima of rows g and g + 8 over both warps' key blocks
+        float c_lo = -CUDART_INF_F, c_hi = -CUDART_INF_F;
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) {
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int key = k0 + (2 * j + half) * 8 + t4 * 2 + e;
+                const bool ok = key < S && key_valid(key, Lv, vl, tl);
+                sc[j][e] = ok ? sc[j][e] : -CUDART_INF_F;
+                sc[j][2 + e] = ok ? sc[j][2 + e] : -CUDART_INF_F;
+                c_lo = fmaxf(c_lo, sc[j][e]);
+                c_hi = fmaxf(c_hi, sc[j][2 + e]);
+            }
+        }
+        c_lo = fmaxf(c_lo, __shfl_xor_sync(0xffffffffu, c_lo, 1));
+        c_lo = fmaxf(c_lo, __shfl_xor_sync(0xffffffffu, c_lo, 2));
+        c_hi = fmaxf(c_hi, __shfl_xor_sync(0xffffffffu, c_hi, 1));
+        c_hi = fmaxf(c_hi, __shfl_xor_sync(0xffffffffu, c_hi, 2));
+        if (t4 == 0) {
+            my_red[g * 2] = c_lo;
+            my_red[(g + 8) * 2] = c_hi;
+        }
+        asm volatile("bar.sync %0, 64;" ::"r"(1 + mt) : "memory");  // the two warps of this row block
+        c_lo = fmaxf(c_lo, other_red[g * 2]);
+        c_hi = fmaxf(c_hi, other_red[(g + 8) * 2]);
+        const float n_lo = fmaxf(m_lo, c_lo), n_hi = fmaxf(m_hi, c_hi);
+        // a row with no valid key so far keeps offset 0: exp2(-inf) = 0 for its P and its rescale factor
+        const float o_lo = n_lo == -CUDART_INF_F ? 0.f : n_lo, o_hi = n_hi == -CUDART_INF_F ? 0.f : n_hi;
+        if (c > 0) {
+            const float f_lo = fast_exp2(m_lo - o_lo), f_hi = fast_exp2(m_hi - o_hi);
+            s_lo *= f_lo;
+            s_hi *= f_hi;
+#pragma unroll
+            for (int nt = 0; nt < 16; ++nt) {
+                out[nt][0] *= f_lo; out[nt][1] *= f_lo;
+                out[nt][2] *= f_hi; out[nt][3] *= f_hi;
+            }
+        }
+        m_lo = n_lo;
+        m_hi = n_hi;
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) {
+            const uint32_t pl = pack_half2(fast_exp2(sc[j][0] - o_lo), fast_exp2(sc[j][1] - o_lo));
+            const uint32_t ph = pack_half2(fast_exp2(sc[j][2] - o_hi), fast_exp2(sc[j][3] - o_hi));
+            const float2 fl = __half22float2(*reinterpret_cast<const __half2*>(&pl));
+            const float2 fh = __half22float2(*reinterpret_cast<const __half2*>(&ph));
+            s_lo += fl.x + fl.y;
+            s_hi += fh.x + fh.y;
+            const int key = (2 * j + half) * 8 + t4 * 2;
+            *reinterpret_cast<uint32_t*>(Ps + r_lo * PS_PAD + key) = pl;
+            *reinterpret_cast<uint32_t*>(Ps + r_hi * PS_PAD + key) = ph;
+        }
+        asm volatile("bar.sync %0, 64;" ::"r"(1 + mt) : "memory");  // both halves of P are visible
+#pragma unroll
+        for (int kb = 0; kb < NJ; ++kb) {  // out[16 rows x this warp's 128 channels] += P . M over the chunk
+            uint32_t ap[4];
+            ldsm_x4(ap, Ps + (mt * 16 + l8 + (lq & 1) * 8) * PS_PAD + kb * 16 + (lq >> 1) * 8);
+#pragma unroll
+            for (int np = 0; np < 8; ++np) {
+                uint32_t bv[4];
+                ldsm_x4_trans(bv, Mc + (kb * 16 + l8 + (lq & 1) * 8) * XM_PAD + half * 128 + (np * 2 + (lq >> 1)) * 8);
+                mma_16816(out[np * 2], ap, bv[0], bv[1]);
+                mma_16816(out[np * 2 + 1], ap, bv[2], bv[3]);
+            }
+        }
+    }
+    s_lo += __shfl_xor_sync(0xffffffffu, s_lo, 1);
+    s_lo += __shfl_xor_sync(0xffffffffu, s_lo, 2);
+    s_hi += __shfl_xor_sync(0xffffffffu, s_hi, 1);
+    s_hi += __shfl_xor_sync(0xffffffffu, s_hi, 2);
+    if (t4 == 0) {
+        my_red[g * 2 + 1] = s_lo;
+        my_red[(g + 8) * 2 + 1] = s_hi;
+    }
+    asm volatile("bar.sync %0, 64;" ::"r"(1 + mt) : "memory");
+    // all keys masked -> sum 0 -> NaN, like torch's softmax of all -inf
+    const float i_lo = 1.f / (s_lo + other_red[g * 2 + 1]), i_hi = 1.f / (s_hi + other_red[(g + 8) * 2 + 1]);
+    __half* o_lo_p = pm + q_lo * ldp + (h_lo < 0 ? 0 : h_lo) * D + half * 128 + t4 * 2;
+    __half* o_hi_p = pm + q_hi * ldp + (h_hi < 0 ? 0 : h_hi) * D + half * 128 + t4 * 2;
+#pragma unroll
+    for (int nt = 0; nt < 16; ++nt) {
+        if (h_lo >= 0) *reinterpret_cast<uint32_t*>(o_lo_p + nt * 8) = pack_half2(out[nt][0] * i_lo, out[nt][1] * i_lo);
+        if (h_hi >= 0) *reinterpret_cast<uint32_t*>(o_hi_p + nt * 8) = pack_half2(out[nt][2] * i_hi, out[nt][3] * i_hi);
+    }
+}
+
 }  // namespace
 
 int enc_self_attention(const float* qk, int64_t ldqk, const float* v, int64_t ldv, float* o, int64_t ldo,
@@ -857,17 +1292,30 @@ int enc_self_attention(const float* qk, int64_t ldqk, const float* v, int64_t ld
                        cudaStream_t s) {
     if (B == 0) return CONE_OK;
     const int S = Lv + Lt;
-    CONE_REQUIRE(S <= MAX_S, "enc_self_attention: window of %d rows exceeds %d", S, MAX_S);
+    CONE_REQUIRE(S <= MAX_S_LONG, "enc_self_attention: window of %d rows exceeds %d", S, MAX_S_LONG);
     const size_t smem = sizeof(float) * ((size_t)S * (HD + 1) + (size_t)S * HD + ENC_WARPS * HD + (size_t)ENC_WARPS * S);
-    static bool attr_set = false;
-    if (!attr_set) {
-        CONE_CUDA(cudaFuncSetAttribute(enc_self_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set = true;
-    }
     dim3 grid((unsigned)B, (unsigned)nheads);
     ProfScope ps(s, P_ENC_ATTN, 4.0 * (double)B * nheads * S * S * HD, 16.0 * (double)B * S * nheads * HD);
-    enc_self_attention_kernel<<<grid, ENC_WARPS * 32, smem, s>>>(qk, ldqk, v, ldv, o, ldo, vlen, tlen, Lv, Lt,
-                                                               nheads * HD);
+    if (S <= MAX_S) {
+        static bool attr_set = false;
+        if (!attr_set) {
+            CONE_CUDA(cudaFuncSetAttribute(enc_self_attention_kernel<MAX_S / 32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           100 * 1024));
+            attr_set = true;
+        }
+        enc_self_attention_kernel<MAX_S / 32><<<grid, ENC_WARPS * 32, smem, s>>>(qk, ldqk, v, ldv, o, ldo, vlen, tlen, Lv, Lt,
+                                                                                nheads * HD);
+    } else {  // long windows: 16 keys per lane, up to 139 KB of shared memory at 512 rows
+        static bool attr_set = false;
+        if (!attr_set) {
+            const size_t smem_max = sizeof(float) * ((size_t)MAX_S_LONG * (2 * HD + 1) + ENC_WARPS * HD + (size_t)ENC_WARPS * MAX_S_LONG);
+            CONE_CUDA(cudaFuncSetAttribute(enc_self_attention_kernel<MAX_S_LONG / 32>,
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max));
+            attr_set = true;
+        }
+        enc_self_attention_kernel<MAX_S_LONG / 32><<<grid, ENC_WARPS * 32, smem, s>>>(qk, ldqk, v, ldv, o, ldo, vlen, tlen, Lv,
+                                                                                     Lt, nheads * HD);
+    }
     CONE_LAUNCH_CHECK("enc_self_attention");
     return CONE_OK;
 }
@@ -901,28 +1349,34 @@ int dec_cross_attention(const void* q_any, int64_t ldq, const void* k, int64_t l
     float* o = static_cast<float*>(o_any);
     if (B == 0) return CONE_OK;
     const int S = Lv + Lt;
-    CONE_REQUIRE(nq >= 1 && nq <= 8 && S <= MAX_S && nheads == 8, "dec_cross_attention: unsupported nq=%d S=%d heads=%d", nq,
-                 S, nheads);
+    CONE_REQUIRE(nq >= 1 && nq <= 8 && S <= MAX_S_LONG && nheads == 8, "dec_cross_attention: unsupported nq=%d S=%d heads=%d",
+                 nq, S, nheads);
     CONE_REQUIRE((ldk & 7) == 0, "dec_cross_attention: ldk must be a multiple of 8");
     const int NQ = nq <= 5 ? 5 : 8;
     const int Sp = (S + 3) & ~3;
     const size_t smem = sizeof(float) * ((size_t)8 * NQ * Sp + 8 * NQ + (size_t)8 * NQ * 8 * 32);
     ProfScope ps(s, P_DEC_ATTN, 4.0 * (double)B * nheads * nq * S * HD, (kv_f16 ? 4.0 : 8.0) * (double)B * S * nheads * HD);
     const unsigned grid = (unsigned)B;
-#define CONE_XATT(KV, NQV)                                                                                              \
+    // long windows (S > 256): 16 scores per lane in the softmax phase, up to 192 KB of shared memory at 512 rows
+#define CONE_XATT(KV, NQV, KPL, SMEM_MAX)                                                                               \
     do {                                                                                                                \
         static bool attr = false;                                                                                       \
         if (!attr) {                                                                                                    \
-            CONE_CUDA(cudaFuncSetAttribute(dec_cross_attention_kernel<KV, NQV>,                                         \
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));                   \
+            CONE_CUDA(cudaFuncSetAttribute(dec_cross_attention_kernel<KV, NQV, KPL>,                                    \
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SMEM_MAX)));              \
             attr = true;                                                                                                \
         }                                                                                                               \
-        dec_cross_attention_kernel<KV, NQV><<<grid, 256, smem, s>>>(q, ldq, static_cast<const KV*>(k), ldk,             \
-                                                                    static_cast<const KV*>(v), ldv, o, ldo, vlen, tlen, \
-                                                                    nq, Lv, Lt, posk, ldposk, table_lv);                \
+        dec_cross_attention_kernel<KV, NQV, KPL><<<grid, 256, smem, s>>>(q, ldq, static_cast<const KV*>(k), ldk,        \
+                                                                         static_cast<const KV*>(v), ldv, o, ldo, vlen,  \
+                                                                         tlen, nq, Lv, Lt, posk, ldposk, table_lv);     \
     } while (0)
     CONE_REQUIRE(!kv_f16, "dec_cross_attention: the tensor-core decoder uses dec_cross_attention_mem");
-    if (NQ == 5) CONE_XATT(float, 5); else CONE_XATT(float, 8);
+    const size_t smem_long = sizeof(float) * ((size_t)8 * NQ * MAX_S_LONG + 8 * NQ + (size_t)8 * NQ * 8 * 32);
+    if (S <= MAX_S) {
+        if (NQ == 5) CONE_XATT(float, 5, MAX_S / 32, 160 * 1024); else CONE_XATT(float, 8, MAX_S / 32, 160 * 1024);
+    } else {
+        if (NQ == 5) CONE_XATT(float, 5, MAX_S_LONG / 32, smem_long); else CONE_XATT(float, 8, MAX_S_LONG / 32, smem_long);
+    }
 
 #undef CONE_XATT
     CONE_LAUNCH_CHECK("dec_cross_attention");
@@ -935,7 +1389,7 @@ int enc_self_attention_f16(const void* qk, int64_t ldqk, const void* v, int64_t 
                            const void* token_qkv, const int64_t* vid_base, const int64_t* txt_base, int64_t n_frames) {
     if (B == 0) return CONE_OK;
     const int S = Lv + Lt;
-    CONE_REQUIRE(S <= MAX_S, "enc_self_attention_f16: window of %d rows exceeds %d", S, MAX_S);
+    CONE_REQUIRE(S <= MAX_S_LONG, "enc_self_attention_f16: window of %d rows exceeds %d", S, MAX_S_LONG);
     CONE_REQUIRE((ldqk % 8) == 0 && (ldv % 8) == 0 && (ldo % 2) == 0, "enc_self_attention_f16: leading dims must keep 16-byte rows");
     const int Sp = (S + 15) & ~15;
     const size_t smem = sizeof(__half) * (size_t)3 * Sp * QK_PAD + sizeof(float) * Sp;
@@ -954,16 +1408,53 @@ int enc_self_attention_f16(const void* qk, int64_t ldqk, const void* v, int64_t 
         CONE_ENC_ATT(20, true);
     } else if (Sp <= 160) {
         CONE_ENC_ATT(20, false);
-    } else {
+    } else if (Sp <= MAX_S) {
         static bool attr = false;
         if (!attr) {
             CONE_CUDA(cudaFuncSetAttribute(enc_attention_f16_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
             attr = true;
         }
         CONE_ENC_ATT(32, false);
+    } else {  // long windows: 16 warps, tile loaded in rounds, online softmax over 64-key chunks (123 KB at 512 rows)
+        static bool attr = false;
+        if (!attr) {
+            const int smem_max = (int)(sizeof(__half) * (size_t)3 * MAX_S_LONG * QK_PAD + sizeof(float) * MAX_S_LONG);
+            CONE_CUDA(cudaFuncSetAttribute(enc_attention_f16_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+            attr = true;
+        }
+        enc_attention_f16_long_kernel<<<grid, LA_WARPS * 32, smem, s>>>(qk16, ldqk, v16, ldv, o16, ldo, vlen, tlen, Lv, Lt,
+                                                                        nheads * HD, static_cast<const __half*>(posqk16),
+                                                                        table_lv, rs);
     }
 #undef CONE_ENC_ATT
     CONE_LAUNCH_CHECK("enc_self_attention_f16");
+    return CONE_OK;
+}
+
+// long windows (256 < S <= 512): the memory streamed in chunks of XL_KC rows (see the kernel's comment)
+static int dec_cross_attention_mem_long(const void* mem, int64_t ldm, const void* qqt, int64_t ldq, void* pm, int64_t ldp,
+                                        const int32_t* vlen, const int32_t* tlen, int64_t B, int nq, int Lv, int Lt,
+                                        const void* posk, int64_t ldposk, int table_lv, cudaStream_t s, int q_bcast, int MT) {
+    const int S = Lv + Lt;
+    const size_t smem = ((size_t)(2 * XL_KC + MT * 16) * XM_PAD + (size_t)MT * 16 * (XL_KC + 8)) * sizeof(__half) +
+                        (size_t)MT * 2 * 16 * 2 * sizeof(float);
+    ProfScope ps(s, P_DEC_ATTN, 2.0 * 2.0 * (double)B * 8 * nq * S * 256, 2.0 * (double)B * S * 256 + 2.0 * 2.0 * (double)B * nq * 9 * 256);
+#define CONE_XMEM_LONG(MTV)                                                                                             \
+    do {                                                                                                                \
+        static bool attr = false;                                                                                       \
+        if (!attr) {                                                                                                    \
+            CONE_CUDA(cudaFuncSetAttribute(dec_cross_attention_mem_long_kernel<MTV>,                                    \
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                    \
+            attr = true;                                                                                                \
+        }                                                                                                               \
+        dec_cross_attention_mem_long_kernel<MTV><<<(unsigned)B, MTV * 64, smem, s>>>(                                   \
+            static_cast<const __half*>(mem), ldm, static_cast<const __half*>(qqt), ldq, static_cast<__half*>(pm), ldp,  \
+            vlen, tlen, nq, Lv, Lt, static_cast<const __half*>(posk), ldposk, table_lv, q_bcast);                       \
+    } while (0)
+    if (MT == 3) CONE_XMEM_LONG(3);
+    else CONE_XMEM_LONG(4);
+#undef CONE_XMEM_LONG
+    CONE_LAUNCH_CHECK("dec_cross_attention_mem");
     return CONE_OK;
 }
 
@@ -973,10 +1464,12 @@ int dec_cross_attention_mem(const void* mem, int64_t ldm, const void* qqt, int64
                             int64_t ldposk, int table_lv, cudaStream_t s, int q_bcast) {
     if (B == 0) return CONE_OK;
     const int S = Lv + Lt;
-    CONE_REQUIRE(nq >= 1 && nq <= 8 && S <= MAX_S, "dec_cross_attention_mem: unsupported nq=%d S=%d", nq, S);
+    CONE_REQUIRE(nq >= 1 && nq <= 8 && S <= MAX_S_LONG, "dec_cross_attention_mem: unsupported nq=%d S=%d", nq, S);
     CONE_REQUIRE((ldm & 7) == 0 && (ldq & 7) == 0 && (ldp & 1) == 0 && (ldposk & 7) == 0,
                  "dec_cross_attention_mem: rows must be 16-byte aligned");
     const int MT = nq <= 6 ? 3 : 4;  // warps = 16-row blocks of the 8 nq score rows (rows past 8 nq are zero)
+    if (S > MAX_S) return dec_cross_attention_mem_long(mem, ldm, qqt, ldq, pm, ldp, vlen, tlen, B, nq, Lv, Lt, posk, ldposk,
+                                                       table_lv, s, q_bcast, MT);
     const int NB = S <= 112 ? 14 : (S <= 160 ? 20 : (S <= 208 ? 26 : 32));  // key blocks of 8, all processed
     const size_t smem = (size_t)(NB * 8 + MT * 16) * XM_PAD * sizeof(__half) + (size_t)MT * 2 * 16 * 2 * sizeof(float);
     // algorithmic work: both products over the raw memory, which is read once

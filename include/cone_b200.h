@@ -48,6 +48,13 @@ extern "C" {
 #define CONE_DTYPE_F16 1
 #define CONE_DTYPE_BF16 2
 
+/* Longest window the library runs: max_v_l + max_q_l (and Lv + Lt of cone_forward) <= 512 rows.  Windows of up to 256
+ * rows run the short-window attention kernels; 257..512 rows run their long-window variants, chosen per call from the
+ * row count with the same accuracy contract.  Longer windows are refused (CONE_ERR_INVALID, the message names the
+ * limit).  The handle's position tables grow as (max_v_l + 1) * max_v_l rows: about 2.4 GB at max_v_l = 480 in
+ * CONE_PREC_TC mode (DESIGN.md §4). */
+#define CONE_MAX_WINDOW_ROWS 512
+
 /* Model / window hyper-parameters (cone/config.py:73-125; values per dataset in
  * cone/scripts/train_{ego4d,mad}.sh). */
 typedef struct cone_dims {
@@ -60,7 +67,7 @@ typedef struct cone_dims {
     int32_t dec_layers;  /* 2                                            --dec_layers        */
     int32_t num_queries; /* 5 moment slots per window                    --num_queries       */
     int32_t max_v_l;     /* window length in frames                      --max_v_l           */
-    int32_t max_q_l;     /* max text tokens                              --max_q_l           */
+    int32_t max_q_l;     /* max text tokens (max_v_l + max_q_l <= 512)   --max_q_l           */
     int32_t m_dim;       /* Dm: motion feature dim, the input width of   --v_motion_feat_dim
                             input_vid_proj; 0 = Dv (one feature source for both roles) */
 } cone_dims;
@@ -219,7 +226,8 @@ int cone_ground_windows_ex(const cone_weights* w, const void* frames_raw, int32_
 
 /* ---- A6-A8  reference-shaped forward: `model(src_txt, src_txt_mask, src_vid_motion,
  * src_vid_motion_mask)` (cone/model.py:82-128).  src_vid [B, Lv, Dm] (= src_vid_motion), src_txt [B, Lt, Dt], valid
- * lengths vid_len / txt_len [B] int32.  Outputs: pred_logits [B,nq,2], pred_spans [B,nq,2];
+ * lengths vid_len / txt_len [B] int32, Lv <= max_v_l of the handle, Lv + Lt <= CONE_MAX_WINDOW_ROWS.
+ * Outputs: pred_logits [B,nq,2], pred_spans [B,nq,2];
  * nullable: saliency [B,Lv], aux_logits / aux_spans [dec_layers-1, B, nq, 2]. */
 int cone_forward(const cone_weights* w, const float* src_txt, const int32_t* txt_len, const float* src_vid,
                  const int32_t* vid_len, int32_t B, int32_t Lt, int32_t Lv, float* pred_logits, float* pred_spans,
