@@ -931,6 +931,15 @@ int check_prec(int prec) {
     return CONE_OK;
 }
 
+// The tensor-core transformer runs its FFN GEMMs (N = ffn, and K = ffn for linear2) on tcgen05 tiles of 128 columns;
+// check_dims accepts any multiple of 16, so a handle with another width is refused here, before any work, rather than
+// by a GEMM partway through the call.  fp32 mode runs every width.
+int check_tc_ffn(const cone_dims& dm, int prec, const char* who) {
+    CONE_REQUIRE(prec != CONE_PREC_TC || dm.ffn % 128 == 0,
+                 "%s: tensor-core mode needs dim_feedforward to be a multiple of 128 (got %d); use fp32 mode", who, dm.ffn);
+    return CONE_OK;
+}
+
 // a raw feature tensor of an _ex entry point: known storage type; 16-bit rows are read 4 elements (8 bytes) at a time,
 // and a sliced view can start at any element
 int check_feature(const char* who, const char* name, const void* p, int32_t dtype) {
@@ -1263,6 +1272,7 @@ extern "C" int cone_ground_windows_ex(const cone_weights* w, const void* frames_
     CONE_TRY(check_feature("cone_ground_windows", "frames_raw", frames_raw, frames_dtype));
     CONE_REQUIRE(topk >= 1 && n_batches >= 1 && n_queries >= 0, "bad sizes");
     CONE_TRY(check_prec(precision));
+    CONE_TRY(check_tc_ffn(w->dims, precision, "cone_ground_windows"));
     Ctx c{w, precision, (cudaStream_t)stream};
     CONE_TRY(ensure_tc(w, precision, c.s));
     const cone_dims& dm = w->dims;
@@ -1371,6 +1381,7 @@ extern "C" int cone_forward(const cone_weights* w, const float* src_txt, const i
     CONE_REQUIRE(w && src_txt && txt_len && src_vid && vid_len && pred_logits && pred_spans && workspace, "null argument");
     CONE_TRY(check_prec(precision));
     const cone_dims& dm = w->dims;
+    CONE_TRY(check_tc_ffn(dm, precision, "cone_forward"));
     CONE_REQUIRE(Lv >= 1 && Lv <= dm.max_v_l, "cone_forward: L_vid=%d exceeds max_v_l=%d of the weights handle", Lv, dm.max_v_l);
     CONE_REQUIRE(Lt >= 1 && Lv + Lt <= CONE_MAX_WINDOW_ROWS, "cone_forward: window of %d rows exceeds %d", Lv + Lt,
                  CONE_MAX_WINDOW_ROWS);

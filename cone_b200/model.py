@@ -110,8 +110,8 @@ class CONE(nn.Module):
         logits, spans, sal, aux_l, aux_s = eng.forward(src_txt.float(), tl, src_vid_motion.float(), vl,
                                                        want_saliency=True, want_aux=self.aux_loss)
         out = {"pred_logits": logits, "pred_spans": spans, "saliency_scores": sal}
-        if self.aux_loss and aux_l is not None:
-            out["aux_outputs"] = [{"pred_logits": a, "pred_spans": b} for a, b in zip(aux_l, aux_s)]
+        if self.aux_loss:  # one entry per decoder layer but the last, as cone/model.py builds it: empty with one layer
+            out["aux_outputs"] = [] if aux_l is None else [{"pred_logits": a, "pred_spans": b} for a, b in zip(aux_l, aux_s)]
         return out
 
     @torch.no_grad()

@@ -37,7 +37,10 @@ extern "C" {
 
 /* compute precision of the dense projections */
 #define CONE_PREC_FP32 0 /* fp32 CUDA-core GEMMs: parity mode, 1e-5 vs the reference */
-#define CONE_PREC_TC 1   /* tcgen05 tensor-core GEMMs (fp16 operands, fp32 accumulate): 1e-3 */
+#define CONE_PREC_TC 1   /* tcgen05 tensor-core GEMMs (fp16 operands, fp32 accumulate): 1e-3.  cone_forward and
+                            cone_ground_windows(_ex) need dims.ffn to be a multiple of 128 in this mode and refuse
+                            any other width (CONE_ERR_INVALID, the message names dim_feedforward); fp32 mode and the
+                            calls that do not run the transformer take any multiple of 16 */
 #define CONE_PREC_TC_SPLIT 2 /* cone_linear only: 3-product split-fp16 GEMM on tcgen05, fp32-class accuracy (what
                                 CONE_PREC_TC uses for the input projections and the span head) */
 

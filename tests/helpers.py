@@ -4,6 +4,7 @@ import os
 
 import numpy as np
 
+from cone_b200.inference import MODES, recall_at_k
 from cone_b200.synth import make_dataset
 from cone_b200.weights import init_state_dict
 from oracle.make_golden import E2E_CASES, GOLDEN, dense_case  # noqa: F401  (no reference import at module load)
@@ -134,3 +135,136 @@ def oracle_window_scores(sd, cfg, ds, q):
         ctx = O.stage0_video_context(sd, torch.from_numpy(O.l2_normalize_np(ds.videos[q.video_idx])))
         _, fs = O.stage1_ranklist(ctx, torch.from_numpy(O.l2_normalize_np(q.cls)), cfg.max_v_l)
         return O.window_scores(fs, cfg.max_v_l).numpy()
+
+
+def pooled_bounds(spans, dur):
+    """[start, end) pooled-row bounds as model.py:186-192 computes them in fp32 (clipping aside)."""
+    sp = np.asarray(spans, dtype=np.float32)
+    x1 = (sp[..., 0] - np.float32(0.5) * sp[..., 1]) * dur
+    x2 = (sp[..., 0] + np.float32(0.5) * sp[..., 1]) * dur
+    return np.stack([np.maximum(np.floor(x1), 0), np.ceil(x2)])
+
+
+def check_grounding_fp32(cfg, ds, res, ora, name):
+    """fp32 mode against the oracle's `eval_pipeline`: rank-lists and windows exact, raw outputs within 1e-5, R@K
+    identical, NMS'd lists equal up to the 4-decimal rounding.  A query whose matching score crossed a floor/ceil pooling
+    boundary may differ; so may, counted, one other query per case: the candidates are sorted on scores rounded to 4
+    decimals (inference.py:83), a 1e-7 difference that moves one rounding reorders rounded ties, and NMS then keeps
+    another row."""
+    from oracle import cone_oracle as O
+    span_tol = ROUND_TOL + 2e-5 * max(len(v) for v in ds.videos) * cfg.clip_length
+    hatch = Hatch(name, "NMS'd list differs from the oracle's with no pooling-boundary flip", 1)
+    flips = n_same = 0
+    for q in ds.queries:
+        r, o = res[q.query_id], ora[q.query_id]
+        assert r["ranklist"] == o["ranklist"], q.query_id
+        assert r["windows"] == o["windows"], q.query_id
+        assert_close(r["pred_spans"], np.stack(o["pred_spans"]), FP32_TOL, "pred_spans")
+        assert_close(r["prob_fg"], np.stack(o["prob_fg"]), FP32_TOL, "prob_fg")
+        f = assert_match_close(r["match"], np.stack(o["match"]), np.stack(o["pred_spans"]),
+                               [n for _, n in r["windows"]], FP32_TOL)
+        flips += f
+        diff = [m for m in MODES if not rows_close(r[m], o[m], span_tol)]
+        n_same += not diff
+        if diff and not f:
+            hatch.use(f"{q.query_id} {diff}")
+    used = hatch.close(len(ds.queries))
+    assert n_same >= len(ds.queries) - flips - used, (n_same, len(ds.queries), flips)
+    gt = {q.query_id: list(q.timestamps) for q in ds.queries}
+    for mode in MODES:
+        want = O.recall_at_k_iou({q.query_id: ora[q.query_id][mode] for q in ds.queries}, gt)
+        assert np.array_equal(np.round(recall_at_k(res, gt, mode=mode) * len(ds.queries)),
+                              np.round(want * len(ds.queries))), mode
+
+
+def check_grounding_tc(cfg, ds, res, ora, name):
+    """Tensor-core mode against the oracle's `eval_pipeline`, the criteria of tests/test_gpu_tc.py: identical top-k
+    windows (the ranking is fp32 in every mode), spans and probabilities within TC_TOL, matching scores within TC_TOL
+    where both sides pool the same rows, at most 8 % of the proposals with moved pooling bounds, R@K hit counts equal up
+    to max(1, 0.5 % of the queries).  Returns the largest span / probability error."""
+    from oracle import cone_oracle as O
+    errs, n_prop, n_flip = [], 0, 0
+    for q in ds.queries:
+        r, o = res[q.query_id], ora[q.query_id]
+        assert r["ranklist"][: cfg.topk_window] == o["ranklist"][: cfg.topk_window], q.query_id
+        assert r["windows"] == o["windows"], q.query_id
+        osp = np.stack(o["pred_spans"])
+        errs.append(np.abs(r["pred_spans"] - osp).ravel())
+        errs.append(np.abs(r["prob_fg"] - np.stack(o["prob_fg"])).ravel())
+        dur = np.asarray([n for _, n in r["windows"]], dtype=np.float32)[:, None]
+        same = np.all(pooled_bounds(r["pred_spans"], dur) == pooled_bounds(osp, dur), axis=0)
+        dm = np.abs(r["match"] - np.stack(o["match"]))
+        assert dm[same].max() <= TC_TOL, f"{q.query_id}: match differs by {dm[same].max():.3e} on identical pooled rows"
+        n_prop += same.size
+        n_flip += int((~same).sum())
+    err = np.concatenate(errs)
+    print(f"[tc-long] {name}: n {err.size} max {err.max():.3e} rms {np.sqrt(np.mean(err ** 2)):.3e}; "
+          f"pooled-row bounds differ for {n_flip} of {n_prop} proposals")
+    assert err.max() <= TC_TOL, f"{name}: max error {err.max():.3e} > {TC_TOL}"
+    assert n_flip <= 0.08 * n_prop
+    gt = {q.query_id: list(q.timestamps) for q in ds.queries}
+    n = len(ds.queries)
+    for mode in MODES:
+        want = O.recall_at_k_iou({q.query_id: ora[q.query_id][mode] for q in ds.queries}, gt)
+        dev = np.abs(np.round(recall_at_k(res, gt, mode=mode) * n) - np.round(want * n)).max()
+        assert dev <= max(1, 0.005 * n), (name, mode)
+    return float(err.max())
+
+
+# ---- the configuration matrix of tests/test_config_matrix.py (CPU) and tests/test_gpu_config_matrix.py (GPU) ----------
+# (Lv, Lt) of dense windows of S = Lv + Lt rows, chosen at the boundaries of the attention dispatch (attention.cu):
+# S 3 / 16 / 17, the NB 14|20 (112/113), <20, true> (145..160), <32, false> (161..), NB 26|32 (208/209), short|long
+# (256/257) switches, the long memory kernel's 128-row chunks (384/385), and 511 / 512.  One handle with max_v_l 480
+# and max_q_l 32 runs all of them: cone_forward takes any Lv <= max_v_l with Lv + Lt <= 512.
+SWEEP_ROWS = [(2, 1), (8, 8), (9, 8), (90, 22), (90, 23), (120, 24), (120, 25), (125, 25), (128, 32), (130, 31),
+              (180, 28), (180, 29), (224, 32), (232, 25), (300, 20), (352, 32), (384, 1), (440, 9), (480, 31), (480, 32)]
+# fp32 decoder NQ 5 / 8, memory-direct cross-attention MT 3 / 4
+SWEEP_NQ = (1, 6, 8)
+# model-configuration axes, on 90 + 20 row windows unless stated
+AXES = {
+    "layers1_nq8": dict(enc_layers=1, dec_layers=1, num_queries=8),
+    "layers3_nq6_ffn2048": dict(enc_layers=3, dec_layers=3, num_queries=6, dim_feedforward=2048),
+    "layers8": dict(enc_layers=8, dec_layers=8),
+    "ffn128": dict(dim_feedforward=128),
+    "odd_dims": dict(v_feat_dim=48, t_feat_dim=16, v_motion_feat_dim=80),
+    "dims320_192": dict(v_feat_dim=320, t_feat_dim=192),
+    "window3": dict(max_v_l=2, max_q_l=1, num_queries=1),
+    "ffn1040": dict(dim_feedforward=1040),
+}
+
+
+def sweep_cfg(nq):
+    from cone_b200.config import EGO4D
+    return EGO4D.replace(max_v_l=480, max_q_l=32, num_queries=nq)
+
+
+def axis_cfg(name):
+    from cone_b200.config import EGO4D
+    return EGO4D.replace(**dict(dict(max_v_l=90, max_q_l=20), **AXES[name]))
+
+
+def dense_batch(cfg, lv, lt, seed):
+    """B = 5 padded windows as start_end_collate emits them: valid lengths vlen = [Lv, 1, ceil(Lv/2), Lv-1, random],
+    tlen = [Lt, Lt, 1, Lt//2, random] (at least 1), padding zeroed.  Returns (motion rows [B, Lv, motion_dim], appearance
+    rows [B, Lv, v_feat_dim], vid mask, tokens, token mask, normalised CLS); the two row tensors are one tensor when the
+    model has no separate motion stream."""
+    import torch
+    g = torch.Generator().manual_seed(seed)
+    r = lambda n: int(torch.randint(1, n + 1, (1,), generator=g))
+    vlen = [max(1, x) for x in (lv, 1, -(-lv // 2), lv - 1, r(lv))]
+    tlen = [max(1, x) for x in (lt, lt, 1, lt // 2, r(lt))]
+    B = len(vlen)
+    mot = torch.randn(B, lv, cfg.motion_dim, generator=g)
+    app = torch.randn(B, lv, cfg.v_feat_dim, generator=g) if cfg.v_motion_feat_dim else mot
+    txt = torch.randn(B, lt, cfg.t_feat_dim, generator=g)
+    txt = txt / (txt.norm(dim=-1, keepdim=True) + 1e-5)
+    cls = torch.randn(B, cfg.v_feat_dim, generator=g)
+    cls = cls / (cls.norm(dim=-1, keepdim=True) + 1e-5)
+    vm, tm = torch.zeros(B, lv), torch.zeros(B, lt)
+    for i in range(B):
+        vm[i, : vlen[i]] = 1
+        tm[i, : tlen[i]] = 1
+        mot[i, vlen[i]:] = 0
+        app[i, vlen[i]:] = 0
+        txt[i, tlen[i]:] = 0
+    return mot, app, vm, txt, tm, cls

@@ -17,14 +17,14 @@ import torch
 from cone_b200._lib import ConeError
 from cone_b200.config import EGO4D, MAD512
 from cone_b200.engine import ConeEngine
-from cone_b200.inference import MODES, ground_dataset, recall_at_k
+from cone_b200.inference import ground_dataset
 from cone_b200.model import CONE
 from cone_b200.synth import make_dataset
 from cone_b200.weights import init_state_dict
 from oracle import cone_oracle as O
 from oracle.make_golden_localizer import localizer_case
 import motion_oracle as MO
-from helpers import FP32_TOL, ROUND_TOL, TC_TOL, Hatch, assert_close, assert_match_close, rows_close
+from helpers import FP32_TOL, TC_TOL, assert_close, check_grounding_fp32, check_grounding_tc
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -58,76 +58,6 @@ def _case(lv, lt):
     return _cache[lv, lt]
 
 
-def _check_fp32(cfg, ds, res, ora, name):
-    """rank-lists and windows exact, raw outputs within 1e-5, R@K identical, NMS'd lists equal up to the 4-decimal rounding.
-    A query whose matching score crossed a floor/ceil pooling boundary may differ; so may, counted, one other query per
-    case: the candidates are sorted on scores rounded to 4 decimals (inference.py:83), a 1e-7 difference that moves one
-    rounding reorders rounded ties, and NMS then keeps another row.  The (231, 25) case, which runs the short-window
-    kernels, has one such query."""
-    span_tol = ROUND_TOL + 2e-5 * max(len(v) for v in ds.videos) * cfg.clip_length
-    hatch = Hatch(name, "NMS'd list differs from the oracle's with no pooling-boundary flip", 1)
-    flips = n_same = 0
-    for q in ds.queries:
-        r, o = res[q.query_id], ora[q.query_id]
-        assert r["ranklist"] == o["ranklist"], q.query_id
-        assert r["windows"] == o["windows"], q.query_id
-        assert_close(r["pred_spans"], np.stack(o["pred_spans"]), FP32_TOL, "pred_spans")
-        assert_close(r["prob_fg"], np.stack(o["prob_fg"]), FP32_TOL, "prob_fg")
-        f = assert_match_close(r["match"], np.stack(o["match"]), np.stack(o["pred_spans"]),
-                               [n for _, n in r["windows"]], FP32_TOL)
-        flips += f
-        diff = [m for m in MODES if not rows_close(r[m], o[m], span_tol)]
-        n_same += not diff
-        if diff and not f:
-            hatch.use(f"{q.query_id} {diff}")
-    used = hatch.close(len(ds.queries))
-    assert n_same >= len(ds.queries) - flips - used, (n_same, len(ds.queries), flips)
-    gt = {q.query_id: list(q.timestamps) for q in ds.queries}
-    for mode in MODES:
-        want = O.recall_at_k_iou({q.query_id: ora[q.query_id][mode] for q in ds.queries}, gt)
-        assert np.array_equal(np.round(recall_at_k(res, gt, mode=mode) * len(ds.queries)),
-                              np.round(want * len(ds.queries))), mode
-
-
-def _bounds(spans, dur):
-    """[start, end) pooled-row bounds as model.py:186-192 computes them in fp32 (clipping aside)."""
-    sp = np.asarray(spans, dtype=np.float32)
-    x1 = (sp[..., 0] - np.float32(0.5) * sp[..., 1]) * dur
-    x2 = (sp[..., 0] + np.float32(0.5) * sp[..., 1]) * dur
-    return np.stack([np.maximum(np.floor(x1), 0), np.ceil(x2)])
-
-
-def _check_tc(cfg, ds, res, ora, name):
-    """The criteria of tests/test_gpu_tc.py: identical top-k windows (the ranking is fp32 in every mode), spans and
-    probabilities within TC_TOL, matching scores within TC_TOL where both sides pool the same rows, at most 8 % of the
-    proposals with moved pooling bounds, R@K hit counts equal up to max(1, 0.5 % of the queries)."""
-    errs, n_prop, n_flip = [], 0, 0
-    for q in ds.queries:
-        r, o = res[q.query_id], ora[q.query_id]
-        assert r["ranklist"][: cfg.topk_window] == o["ranklist"][: cfg.topk_window], q.query_id
-        assert r["windows"] == o["windows"], q.query_id
-        osp = np.stack(o["pred_spans"])
-        errs.append(np.abs(r["pred_spans"] - osp).ravel())
-        errs.append(np.abs(r["prob_fg"] - np.stack(o["prob_fg"])).ravel())
-        dur = np.asarray([n for _, n in r["windows"]], dtype=np.float32)[:, None]
-        same = np.all(_bounds(r["pred_spans"], dur) == _bounds(osp, dur), axis=0)
-        dm = np.abs(r["match"] - np.stack(o["match"]))
-        assert dm[same].max() <= TC_TOL, f"{q.query_id}: match differs by {dm[same].max():.3e} on identical pooled rows"
-        n_prop += same.size
-        n_flip += int((~same).sum())
-    err = np.concatenate(errs)
-    print(f"[tc-long] {name}: n {err.size} max {err.max():.3e} rms {np.sqrt(np.mean(err ** 2)):.3e}; "
-          f"pooled-row bounds differ for {n_flip} of {n_prop} proposals")
-    assert err.max() <= TC_TOL, f"{name}: max error {err.max():.3e} > {TC_TOL}"
-    assert n_flip <= 0.08 * n_prop
-    gt = {q.query_id: list(q.timestamps) for q in ds.queries}
-    n = len(ds.queries)
-    for mode in MODES:
-        want = O.recall_at_k_iou({q.query_id: ora[q.query_id][mode] for q in ds.queries}, gt)
-        dev = np.abs(np.round(recall_at_k(res, gt, mode=mode) * n) - np.round(want * n)).max()
-        assert dev <= max(1, 0.005 * n), (name, mode)
-
-
 def _assert_results_equal(a, b):
     assert a.keys() == b.keys()
     for k in a:
@@ -144,14 +74,14 @@ def _assert_results_equal(a, b):
 def test_long_windows_fp32_vs_oracle(lv, lt):
     cfg, sd, ds, ora = _case(lv, lt)
     eng = ConeEngine(cfg, sd, device=DEV, precision="fp32", workspace_bytes=2 << 30)
-    _check_fp32(cfg, ds, ground_dataset(eng, ds.videos, ds.queries), ora, f"fp32 {lv}+{lt}")
+    check_grounding_fp32(cfg, ds, ground_dataset(eng, ds.videos, ds.queries), ora, f"fp32 {lv}+{lt}")
 
 
 @pytest.mark.parametrize("lv,lt", SHAPES)
 def test_long_windows_tc_vs_oracle(lv, lt):
     cfg, sd, ds, ora = _case(lv, lt)
     eng = ConeEngine(cfg, sd, device=DEV, precision="tc", workspace_bytes=2 << 30)
-    _check_tc(cfg, ds, ground_dataset(eng, ds.videos, ds.queries), ora, f"{lv}+{lt}")
+    check_grounding_tc(cfg, ds, ground_dataset(eng, ds.videos, ds.queries), ora, f"{lv}+{lt}")
 
 
 def _dense(cfg, lt, seed):
@@ -238,7 +168,7 @@ def test_motion_stream_fp32_vs_oracle():
     ds = make_dataset(cfg, 3, _lengths(300), [2, 2, 1], seed=12, motion_dim=1024)
     ora = MO.eval_pipeline(sd, cfg, ds.videos, ds.queries, motion_videos=ds.motion)
     eng = ConeEngine(cfg, sd, device=DEV, precision="fp32", workspace_bytes=2 << 30)
-    _check_fp32(cfg, ds, ground_dataset(eng, ds.videos, ds.queries, motion_videos=ds.motion), ora, "fp32 motion 300+77")
+    check_grounding_fp32(cfg, ds, ground_dataset(eng, ds.videos, ds.queries, motion_videos=ds.motion), ora, "fp32 motion 300+77")
 
 
 @pytest.mark.parametrize("precision", ["fp32", "tc"])

@@ -17,7 +17,7 @@ from cone_b200.synth import make_dataset
 from cone_b200.weights import init_state_dict
 from oracle import cone_oracle as O
 import motion_oracle as MO
-from helpers import FP32_TOL, ROUND_TOL, TC_TOL, assert_close, assert_match_close, dense_case, rows_close
+from helpers import FP32_TOL, ROUND_TOL, TC_TOL, assert_close, assert_match_close, dense_case, pooled_bounds, rows_close
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -39,14 +39,6 @@ def _case(name):
         ds = make_dataset(cfg, motion_dim=cfg.v_motion_feat_dim, **dkw)
         _cache[name] = (cfg, sd, ds, MO.eval_pipeline(sd, cfg, ds.videos, ds.queries, motion_videos=ds.motion))
     return _cache[name]
-
-
-def _bounds(spans, dur):
-    """[start, end) pooled-row bounds as model.py:186-192 computes them in fp32 (clipping aside)."""
-    sp = np.asarray(spans, dtype=np.float32)
-    x1 = (sp[..., 0] - np.float32(0.5) * sp[..., 1]) * dur
-    x2 = (sp[..., 0] + np.float32(0.5) * sp[..., 1]) * dur
-    return np.stack([np.maximum(np.floor(x1), 0), np.ceil(x2)])
 
 
 @pytest.mark.parametrize("name", list(CASES))
@@ -97,7 +89,7 @@ def test_two_streams_tc_vs_oracle(name):
         errs.append(np.abs(r["prob_fg"] - np.stack(o["prob_fg"])).ravel())
         # matching scores where both sides pool the same rows; proposals whose floor/ceil bounds moved are counted
         dur = np.asarray([n for _, n in r["windows"]], dtype=np.float32)[:, None]
-        same = np.all(_bounds(r["pred_spans"], dur) == _bounds(osp, dur), axis=0)
+        same = np.all(pooled_bounds(r["pred_spans"], dur) == pooled_bounds(osp, dur), axis=0)
         dm = np.abs(r["match"] - np.stack(o["match"]))
         assert dm[same].max() <= TC_TOL, f"{q.query_id}: match differs by {dm[same].max():.3e} on identical pooled rows"
         n_prop += same.size

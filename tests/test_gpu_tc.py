@@ -13,7 +13,7 @@ from cone_b200.inference import ground_dataset, recall_at_k
 from cone_b200.synth import make_dataset
 from cone_b200.weights import init_state_dict
 from oracle import cone_oracle as O
-from helpers import TC_TOL, Hatch, assert_close, assert_match_close, dense_case, oracle_window_scores, ranklist_near_tie
+from helpers import TC_TOL, Hatch, assert_close, assert_match_close, dense_case, oracle_window_scores, pooled_bounds, ranklist_near_tie
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -130,7 +130,7 @@ def _tc_vs_oracle(cfg, sd, ds, name, workspace=3 << 30, hatch_limit=0):
         # then moves by ~1e-2.  Where both sides pool the SAME rows the scores must agree within TC_TOL; the proposals
         # whose bounds differ are counted.
         dur = np.asarray([n for _, n in r["windows"]], dtype=np.float32)[:, None]
-        b_got, b_ref = _bounds(r["pred_spans"], dur), _bounds(osp, dur)
+        b_got, b_ref = pooled_bounds(r["pred_spans"], dur), pooled_bounds(osp, dur)
         same = np.all(b_got == b_ref, axis=0)
         dm = np.abs(r["match"] - np.stack(o["match"]))
         assert dm[same].max() <= TC_TOL, f"{q.query_id}: match differs by {dm[same].max():.3e} on identical pooled rows"
@@ -156,14 +156,6 @@ def _tc_vs_oracle(cfg, sd, ds, name, workspace=3 << 30, hatch_limit=0):
             print(f"[tc-vs-oracle] {name}: R@K hit counts ({mode}) differ from the oracle's by at most {int(dev)} of {n} queries")
             assert dev <= max(1, 0.005 * n), (name, mode, got, want)
     return err
-
-
-def _bounds(spans, dur):
-    """[start, end) pooled-row bounds as model.py:186-192 computes them in fp32 (clipping aside)."""
-    sp = np.asarray(spans, dtype=np.float32)
-    x1 = (sp[..., 0] - np.float32(0.5) * sp[..., 1]) * dur
-    x2 = (sp[..., 0] + np.float32(0.5) * sp[..., 1]) * dur
-    return np.stack([np.maximum(np.floor(x1), 0), np.ceil(x2)])
 
 
 @pytest.mark.parametrize("wseed,dseed", [(21, 33), (5, 7), (9, 11)])
