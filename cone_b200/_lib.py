@@ -18,6 +18,10 @@ DTYPE_F32 = 0
 DTYPE_F16 = 1
 DTYPE_BF16 = 2
 
+# include/cone_b200.h: most candidates per query of cone_fuse_nms(_ex) (shared memory) and of cone_fuse_nms_ws
+FUSE_NMS_MAX_SHARED_CANDIDATES = 2201
+FUSE_NMS_MAX_CANDIDATES = 131072
+
 
 class ConeDims(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("v_dim", "t_dim", "hidden", "nheads", "ffn", "enc_layers", "dec_layers",
@@ -67,6 +71,9 @@ SIGNATURES = {
     "cone_fuse_nms": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _f32, _f64, _i32, _i32, _p, _p, _p, _p, _p]),
     "cone_fuse_nms_ex": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _f32, _f64, _i32, _i32, _i32, _i32, _p, _p, _p, _p,
                                    _p]),
+    "cone_fuse_nms_workspace_bytes": (_sz, [_i32, _i32, _i32]),
+    "cone_fuse_nms_ws": (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _i32, _f32, _f64, _i32, _i32, _i32, _i32, _p, _p, _p, _p,
+                                   _p, _sz, _p]),
     "cone_temporal_nms": (C.c_int, [_p, _p, _p, _i32, _f64, _i32, _p, _p, _p]),
     "cone_eval_recall": (C.c_int, [_p, _p, _p, _i32, _i32, _p, _i32, _p, _i32, _i32, _p, _p, _p]),
     "cone_eval_window_recall": (C.c_int, [_p, _i32, _p, _i32, _f64, _i32, _p, _i32, _p, _p]),

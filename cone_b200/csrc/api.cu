@@ -1219,9 +1219,9 @@ extern "C" int cone_prefilter_ex(const cone_weights* w, const void* frames_raw, 
 }
 
 namespace {
-size_t ground_chunk_bytes(const cone_dims& dm, int64_t nqc, int topk, int Lv, int Lt, int prec) {
+// workspace of one stage-2 chunk: B windows of nqc queries
+size_t ground_chunk_bytes(const cone_dims& dm, int64_t nqc, int64_t B, int Lv, int Lt, int prec) {
     Arena a(nullptr, 0);
-    const int64_t B = nqc * topk;
     plan_core(a, dm, B, Lv, Lt, prec);
     plan_match(a, dm, B, nqc);
     a.get<float>(nqc * Lt * dm.hidden);  // txtproj
@@ -1316,16 +1316,21 @@ extern "C" int cone_ground_windows_ex(const cone_weights* w, const void* frames_
     }
 
     const size_t avail = workspace_bytes - head.used;
+    // chunks of whole queries, halved until one fits; when one query's k windows do not fit, each query runs in chunks
+    // of nwc contiguous windows instead (every window's result is independent of the chunk it runs in)
     int64_t nqc = n_queries;
-    while (nqc > 1 && ground_chunk_bytes(dm, nqc, topk, Lv, Lt, precision) > avail) nqc = (nqc + 1) / 2;
-    if (ground_chunk_bytes(dm, nqc, topk, Lv, Lt, precision) > avail) {
-        set_error("cone_ground_windows: workspace of %zu bytes cannot hold one query (%zu needed)", workspace_bytes,
-                  ground_chunk_bytes(dm, 1, topk, Lv, Lt, precision) + head.used);
-        return CONE_ERR_WORKSPACE;
+    while (nqc > 1 && ground_chunk_bytes(dm, nqc, nqc * topk, Lv, Lt, precision) > avail) nqc = (nqc + 1) / 2;
+    int nwc = topk;
+    if (ground_chunk_bytes(dm, nqc, nqc * topk, Lv, Lt, precision) > avail) {
+        while (nwc > 1 && ground_chunk_bytes(dm, 1, nwc, Lv, Lt, precision) > avail) nwc = (nwc + 1) / 2;
+        if (ground_chunk_bytes(dm, 1, nwc, Lv, Lt, precision) > avail) {
+            set_error("cone_ground_windows: workspace of %zu bytes cannot hold one window (%zu needed)", workspace_bytes,
+                      ground_chunk_bytes(dm, 1, 1, Lv, Lt, precision) + head.used);
+            return CONE_ERR_WORKSPACE;
+        }
     }
-    for (int64_t q0 = 0; q0 < n_queries; q0 += nqc) {
-        const int64_t n = (n_queries - q0) < nqc ? (n_queries - q0) : nqc;
-        const int64_t B = n * topk;
+    // windows g0 .. g0+B of the flat [n_queries, topk] list, which belong to the n queries from q0
+    auto run_chunk = [&](int64_t q0, int64_t n, int64_t g0, int64_t B) -> int {
         Arena a((char*)workspace + head.used, avail);
         CoreBuffers cb = plan_core(a, dm, B, Lv, Lt, precision);
         MatchBuffers mb = plan_match(a, dm, B, n);
@@ -1354,7 +1359,7 @@ extern "C" int cone_ground_windows_ex(const cone_weights* w, const void* frames_
                 cb.g_src_lo = vidproj16lo;
             }
         }
-        CONE_TRY(fill_window_desc_chunk(q_video_start, win_start, win_len, tok_len, q_batch, batch_max, (int)q0, (int)n,
+        CONE_TRY(fill_window_desc_chunk(q_video_start, win_start, win_len, tok_len, q_batch, batch_max, g0, (int)B, (int)q0,
                                         topk, Lt, Lv, cb.vid_base, cb.vlen, cb.txt_base, cb.tlen, cb.pad_len, cb.qidx, c.s));
         if (tail_gather) {
             // nothing to copy: layer 0 reads q|k|v and its residual rows through the window descriptors
@@ -1367,9 +1372,19 @@ extern "C" int cone_ground_windows_ex(const cone_weights* w, const void* frames_
         } else {
             CONE_TRY(gather_window_rows(vidproj, n_frames, cb.vid_base, txtproj, cb.txt_base, cb.src, B, Lv, Lt, dm.hidden, c.s));
         }
-        float* spans_c = pred_spans + q0 * topk * nq * 2;
-        CONE_TRY(transformer_core(c, cb, nullptr, prob_fg + q0 * topk * nq, spans_c, nullptr, nullptr, nullptr));
-        CONE_TRY(match_core(c, frames_raw, frames_dtype, n_frames, cb, spans_c, cls_norm + q0 * dm.v_dim, n, mb, match + q0 * topk * nq, nq));
+        float* spans_c = pred_spans + g0 * nq * 2;
+        CONE_TRY(transformer_core(c, cb, nullptr, prob_fg + g0 * nq, spans_c, nullptr, nullptr, nullptr));
+        CONE_TRY(match_core(c, frames_raw, frames_dtype, n_frames, cb, spans_c, cls_norm + q0 * dm.v_dim, n, mb, match + g0 * nq, nq));
+        return CONE_OK;
+    };
+    if (nwc == topk) {
+        for (int64_t q0 = 0; q0 < n_queries; q0 += nqc) {
+            const int64_t n = (n_queries - q0) < nqc ? (n_queries - q0) : nqc;
+            CONE_TRY(run_chunk(q0, n, q0 * topk, n * topk));
+        }
+    } else {
+        for (int64_t q = 0; q < n_queries; ++q)
+            for (int j0 = 0; j0 < topk; j0 += nwc) CONE_TRY(run_chunk(q, 1, q * topk + j0, topk - j0 < nwc ? topk - j0 : nwc));
     }
     return CONE_OK;
 }
@@ -1467,6 +1482,24 @@ extern "C" int cone_fuse_nms_ex(const float* pred_spans, const float* prob_fg, c
     return fuse_nms(pred_spans, prob_fg, match, win_start, win_len, n_queries, topk, nq, clip_length, nms_thd,
                     max_before_nms, max_after_nms, out, out_count, rows_out, rows_count, (cudaStream_t)stream,
                     fixed_duration, sort_within_window != 0);
+}
+
+extern "C" size_t cone_fuse_nms_workspace_bytes(int32_t n_queries, int32_t topk, int32_t nq) {
+    return fuse_nms_workspace_bytes(n_queries, topk, nq);
+}
+
+extern "C" int cone_fuse_nms_ws(const float* pred_spans, const float* prob_fg, const float* match,
+                                const int32_t* win_start, const int32_t* win_len, int32_t n_queries, int32_t topk, int32_t nq,
+                                float clip_length, double nms_thd, int32_t max_before_nms, int32_t max_after_nms,
+                                int32_t fixed_duration, int32_t sort_within_window, double* out, int32_t* out_count,
+                                double* rows_out, int32_t* rows_count, void* workspace, size_t workspace_bytes,
+                                void* stream) {
+    CONE_REQUIRE(n_queries == 0 || (pred_spans && prob_fg && match && win_start && win_len && out && out_count),
+                 "null argument");
+    CONE_REQUIRE(fixed_duration >= 0, "cone_fuse_nms_ws: fixed_duration must be >= 0");
+    return fuse_nms_ws(pred_spans, prob_fg, match, win_start, win_len, n_queries, topk, nq, clip_length, nms_thd,
+                       max_before_nms, max_after_nms, out, out_count, rows_out, rows_count, workspace, workspace_bytes,
+                       (cudaStream_t)stream, fixed_duration, sort_within_window != 0);
 }
 
 extern "C" int cone_temporal_nms(const double* st, const double* ed, const double* score, int32_t n, double nms_thd,

@@ -129,9 +129,10 @@ int build_windows(const int32_t* ranklist, int ranklist_stride, const int32_t* q
 int batch_max_len(const int32_t* win_len, const int32_t* q_batch, int n_queries, int topk, int32_t* batch_max,
                   int n_batches, cudaStream_t s);
 // per-chunk descriptors for queries [q0, q0+nq)
+// windows g0 .. g0+nw of the flat [n_queries, topk] list; txt_base / qidx count queries from q_lo
 int fill_window_desc_chunk(const int64_t* q_video_start, const int32_t* win_start, const int32_t* win_len,
-                           const int32_t* tok_len, const int32_t* q_batch, const int32_t* batch_max, int q0, int nqc,
-                           int topk, int Lt, int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base,
+                           const int32_t* tok_len, const int32_t* q_batch, const int32_t* batch_max, int64_t g0, int nw,
+                           int q_lo, int topk, int Lt, int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base,
                            int32_t* tlen, int32_t* pad_len, int32_t* qidx, cudaStream_t s);  // q_batch null: pad_len = fixed_pad
 
 // ---------------------------------------------------------------- pool_match.cu
@@ -149,6 +150,13 @@ int fuse_nms(const float* pred_spans, const float* prob_fg, const float* match, 
              const int32_t* win_len, int n_queries, int topk, int nq, float clip_length, double nms_thd,
              int max_before_nms, int max_after_nms, double* out, int32_t* out_count, double* rows_out,
              int32_t* rows_count, cudaStream_t s, int fixed_duration = 0, int sort_windows = 1);
+// the workspace path: up to 16384 * 8 candidates per query, queries in chunks sized to the workspace
+size_t fuse_nms_workspace_bytes(int n_queries, int topk, int nq);  // 0 + error message when refused
+int fuse_nms_ws(const float* pred_spans, const float* prob_fg, const float* match, const int32_t* win_start,
+                const int32_t* win_len, int n_queries, int topk, int nq, float clip_length, double nms_thd,
+                int max_before_nms, int max_after_nms, double* out, int32_t* out_count, double* rows_out,
+                int32_t* rows_count, void* workspace, size_t workspace_bytes, cudaStream_t s, int fixed_duration,
+                int sort_windows);
 int temporal_nms_single(const double* st, const double* ed, const double* score, int n, double nms_thd,
                         int max_after_nms, int32_t* keep_out, int32_t* n_keep_out, cudaStream_t s);
 

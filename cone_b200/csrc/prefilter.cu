@@ -96,17 +96,18 @@ __global__ void batch_max_len_kernel(const int32_t* __restrict__ win_len, const 
     atomicMax(&batch_max[q_batch[i / topk]], win_len[i]);
 }
 
+// descriptors of the flat windows g0 .. g0+nw of [n_queries, topk]; query indices relative to q_lo (the chunk's first query)
 __global__ void fill_window_desc_chunk_kernel(const int64_t* __restrict__ q_video_start,
                                               const int32_t* __restrict__ win_start, const int32_t* __restrict__ win_len,
                                               const int32_t* __restrict__ tok_len, const int32_t* __restrict__ q_batch,
-                                              const int32_t* __restrict__ batch_max, int q0, int nqc, int topk, int Lt,
-                                              int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base, int32_t* tlen,
-                                              int32_t* pad_len, int32_t* qidx) {
+                                              const int32_t* __restrict__ batch_max, int64_t g0, int nw, int q_lo, int topk,
+                                              int Lt, int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base,
+                                              int32_t* tlen, int32_t* pad_len, int32_t* qidx) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nqc * topk) return;
-    const int ql = i / topk;
-    const int q = q0 + ql;
-    const int64_t g = (int64_t)q * topk + (i % topk);
+    if (i >= nw) return;
+    const int64_t g = g0 + i;
+    const int q = (int)(g / topk);
+    const int ql = q - q_lo;
     vid_base[i] = q_video_start[q] + win_start[g];
     vlen[i] = win_len[g];
     txt_base[i] = (int64_t)ql * Lt;
@@ -198,13 +199,13 @@ int batch_max_len(const int32_t* win_len, const int32_t* q_batch, int n_queries,
 }
 
 int fill_window_desc_chunk(const int64_t* q_video_start, const int32_t* win_start, const int32_t* win_len,
-                           const int32_t* tok_len, const int32_t* q_batch, const int32_t* batch_max, int q0, int nqc,
-                           int topk, int Lt, int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base,
+                           const int32_t* tok_len, const int32_t* q_batch, const int32_t* batch_max, int64_t g0, int nw,
+                           int q_lo, int topk, int Lt, int fixed_pad, int64_t* vid_base, int32_t* vlen, int64_t* txt_base,
                            int32_t* tlen, int32_t* pad_len, int32_t* qidx, cudaStream_t s) {
-    if (nqc == 0) return CONE_OK;
-    fill_window_desc_chunk_kernel<<<cdiv(nqc * topk, 256), 256, 0, s>>>(q_video_start, win_start, win_len, tok_len,
-                                                                       q_batch, batch_max, q0, nqc, topk, Lt, fixed_pad, vid_base,
-                                                                       vlen, txt_base, tlen, pad_len, qidx);
+    if (nw == 0) return CONE_OK;
+    fill_window_desc_chunk_kernel<<<cdiv(nw, 256), 256, 0, s>>>(q_video_start, win_start, win_len, tok_len, q_batch,
+                                                                batch_max, g0, nw, q_lo, topk, Lt, fixed_pad, vid_base,
+                                                                vlen, txt_base, tlen, pad_len, qidx);
     CONE_LAUNCH_CHECK("fill_window_desc_chunk");
     return CONE_OK;
 }

@@ -386,7 +386,9 @@ class ConeEngine:
     def fuse_nms(self, pred_spans, prob_fg, match, win_start, win_len, want_rows=False, cfg: Optional[ConeConfig] = None,
                  fixed_duration: int = 0, sort_within_window: bool = True):
         """Stage 3.  `fixed_duration` / `sort_within_window` select the single-video front end's variant
-        (run_on_video/cone_localizator.py:183-219); the defaults are eval_epoch's."""
+        (run_on_video/cone_localizator.py:183-219); the defaults are eval_epoch's.  Up to
+        FUSE_NMS_MAX_SHARED_CANDIDATES candidates per query (topk_window x num_queries) run the shared-memory kernel,
+        more (up to every window of a video) the workspace kernel; both give the same bits."""
         cfg = cfg or self.cfg
         nq_, k, nslot = prob_fg.shape
         dev = prob_fg.device
@@ -394,15 +396,19 @@ class ConeEngine:
         cnt = torch.zeros((nq_, 3), dtype=torch.int32, device=dev)
         rows = torch.zeros((nq_, k * nslot, 4), dtype=torch.float64, device=dev) if want_rows else None
         rcnt = torch.zeros((nq_,), dtype=torch.int32, device=dev) if want_rows else None
-        _lib.check(self.lib.cone_fuse_nms_ex(_ptr(_need(pred_spans, torch.float32, "pred_spans")),
-                                             _ptr(_need(prob_fg, torch.float32, "prob_fg")),
-                                             _ptr(_need(match, torch.float32, "match")),
-                                             _ptr(_need(win_start, torch.int32, "win_start")),
-                                             _ptr(_need(win_len, torch.int32, "win_len")), nq_, k, nslot,
-                                             float(np.float32(cfg.clip_length)), float(cfg.nms_thd), cfg.max_before_nms,
-                                             cfg.max_after_nms, int(fixed_duration), int(bool(sort_within_window)),
-                                             _ptr(out), _ptr(cnt), _ptr(rows), _ptr(rcnt), _stream()),
-                   "cone_fuse_nms_ex")
+        args = (_ptr(_need(pred_spans, torch.float32, "pred_spans")), _ptr(_need(prob_fg, torch.float32, "prob_fg")),
+                _ptr(_need(match, torch.float32, "match")), _ptr(_need(win_start, torch.int32, "win_start")),
+                _ptr(_need(win_len, torch.int32, "win_len")), nq_, k, nslot, float(np.float32(cfg.clip_length)),
+                float(cfg.nms_thd), cfg.max_before_nms, cfg.max_after_nms, int(fixed_duration),
+                int(bool(sort_within_window)), _ptr(out), _ptr(cnt), _ptr(rows), _ptr(rcnt))
+        if k * nslot <= _lib.FUSE_NMS_MAX_SHARED_CANDIDATES:
+            _lib.check(self.lib.cone_fuse_nms_ex(*args, _stream()), "cone_fuse_nms_ex")
+        else:  # more candidates than shared memory holds: the workspace path, as many queries per launch as fit
+            one = self.lib.cone_fuse_nms_workspace_bytes(1, k, nslot)
+            if one == 0:
+                _lib.check(-1, "cone_fuse_nms_workspace_bytes")
+            ws, nb = self._wsargs(one)
+            _lib.check(self.lib.cone_fuse_nms_ws(*args, ws, nb, _stream()), "cone_fuse_nms_ws")
         return out, cnt, rows, rcnt
 
     # ---- metric counters (SURVEY.md §8(f)1) ---------------------------------------------------

@@ -25,6 +25,17 @@ from ..synth import make_dataset
 from ..weights import init_state_dict
 
 
+def resolve_topk_window(value: str, cfg, video_lengths) -> int:
+    """`--topk-window`: a positive count, or "all" = every window of the longest video (num_window of its length), the
+    exhaustive grounding that the pre-filter is measured against."""
+    if value == "all":
+        return cfg.num_window(max(video_lengths))
+    k = int(value)
+    if k < 1:
+        raise ValueError(f"--topk-window must be >= 1 or 'all', got {value}")
+    return k
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--config", default="ego4d", choices=sorted(PRESETS))
@@ -34,6 +45,8 @@ def main() -> None:
     ap.add_argument("--motion-dim", type=int, default=0, help="width of a separate motion stream (0 = none)")
     ap.add_argument("--feature-dtype", default="float32", choices=["float32", "float16"],
                     help="storage type of the videos, motion features and queries")
+    ap.add_argument("--topk-window", default="", help="windows grounded per query: a count, or 'all' for every window "
+                    "of the longest video (default: the config's topk_window)")
     ap.add_argument("--precision", default="fp32")
     ap.add_argument("--flavour", default="mad", choices=["mad", "ego4d"])
     ap.add_argument("--seed", type=int, default=0)
@@ -51,6 +64,8 @@ def main() -> None:
     # with `queries` per video a multiple of eval_bsz every video holds whole batches
     cfg = cfg.replace(eval_bsz=a.queries, v_motion_feat_dim=a.motion_dim)
     ds = make_dataset(cfg, a.videos, None, a.queries, seed=a.seed, frames_range=tuple(a.frames), motion_dim=a.motion_dim)
+    if a.topk_window:
+        cfg = cfg.replace(topk_window=resolve_topk_window(a.topk_window, cfg, [len(v) for v in ds.videos]))
     fdt = np.dtype(a.feature_dtype)
     videos = [v.astype(fdt) for v in ds.videos]
     motion = None if ds.motion is None else [m.astype(fdt) for m in ds.motion]

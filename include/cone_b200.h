@@ -266,6 +266,25 @@ int cone_fuse_nms_ex(const float* pred_spans, const float* prob_fg, const float*
                      int32_t sort_within_window, double* out, int32_t* out_count, double* rows_out,
                      int32_t* rows_count, void* stream);
 
+/* Largest topk * nq that cone_fuse_nms and cone_fuse_nms_ex take: they hold every candidate of a query in shared memory
+ * and refuse more (CONE_ERR_INVALID).  cone_fuse_nms_ws has no such limit below CONE_FUSE_NMS_MAX_CANDIDATES. */
+#define CONE_FUSE_NMS_MAX_SHARED_CANDIDATES 2201
+/* Largest topk * nq of cone_fuse_nms_ws: 16384 windows (the longest rank-list of cone_window_ranklist) x 8 slots. */
+#define CONE_FUSE_NMS_MAX_CANDIDATES 131072
+
+/* Stage 3 for any topk up to every window of a video: the arguments and results of cone_fuse_nms_ex, computed in
+ * `workspace` instead of shared memory, in O(N log N) per query (N = topk * nq <= CONE_FUSE_NMS_MAX_CANDIDATES).  At any N
+ * both give the same bits.  Queries run in chunks sized to the workspace; a workspace smaller than one query needs is
+ * CONE_ERR_WORKSPACE, a larger N is CONE_ERR_INVALID.  No allocation and no host synchronisation: capturable in a graph.
+ * cone_fuse_nms_workspace_bytes gives the bytes for all n_queries at once (any multiple of the one-query size runs
+ * that many queries per launch), or 0 when the arguments are refused (cone_last_error names the limit). */
+size_t cone_fuse_nms_workspace_bytes(int32_t n_queries, int32_t topk, int32_t nq);
+int cone_fuse_nms_ws(const float* pred_spans, const float* prob_fg, const float* match, const int32_t* win_start,
+                     const int32_t* win_len, int32_t n_queries, int32_t topk, int32_t nq, float clip_length,
+                     double nms_thd, int32_t max_before_nms, int32_t max_after_nms, int32_t fixed_duration,
+                     int32_t sort_within_window, double* out, int32_t* out_count, double* rows_out,
+                     int32_t* rows_count, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- A13  `temporal_nms(predictions, nms_thd, max_after_nms)` (utils/temporal_nms.py:25-74) on
  * one list: st/ed/score [n] fp64 in input order; keep_out [max_after_nms] indices into the input in
  * output order; n_keep_out [1]. */
