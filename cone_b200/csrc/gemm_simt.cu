@@ -24,7 +24,10 @@ struct TileArgs {
     int N, K, relu;
 };
 
-__device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0) {
+// kRowOffsets = false: row m of C starts at C + m * ldc.  true: at C + row_off[m] (ldc unused), and each row takes the
+// float4 epilogue only where its own start is 16-byte aligned.
+template <bool kRowOffsets>
+__device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0, const int64_t* row_off = nullptr) {
     __shared__ __align__(16) float As[2][BK][BM + 4];
     __shared__ __align__(16) float Ws[2][BK][BN + 4];
     const int tid = threadIdx.x;
@@ -92,12 +95,22 @@ __device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0
     }
 
     // epilogue: bias -> residual -> relu
-    const bool vec_ok = ((p.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0) &&
-                        (p.R == nullptr || (((p.ldr & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.R) & 15) == 0)));
+    const bool r_ok = p.R == nullptr || (((p.ldr & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.R) & 15) == 0));
+    const bool vec_all = ((p.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0) &&
+                         (p.R == nullptr || (((p.ldr & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.R) & 15) == 0)));
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
         const int64_t m = m0 + (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
         if (m >= p.M) continue;
+        float* crow;
+        bool vec_ok;
+        if constexpr (kRowOffsets) {
+            crow = p.C + row_off[m];
+            vec_ok = ((reinterpret_cast<uintptr_t>(crow) & 15) == 0) && r_ok;
+        } else {
+            crow = p.C + m * p.ldc;
+            vec_ok = vec_all;
+        }
 #pragma unroll
         for (int jb = 0; jb < 2; ++jb) {
             const int n = n0 + (jb == 0 ? tx * 4 : 64 + tx * 4);
@@ -116,7 +129,7 @@ __device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0
 #pragma unroll
                     for (int t = 0; t < 4; ++t) v[t] = fmaxf(v[t], 0.f);
                 }
-                *reinterpret_cast<float4*>(p.C + m * p.ldc + n) = make_float4(v[0], v[1], v[2], v[3]);
+                *reinterpret_cast<float4*>(crow + n) = make_float4(v[0], v[1], v[2], v[3]);
             } else {
 #pragma unroll
                 for (int t = 0; t < 4; ++t) {
@@ -125,7 +138,7 @@ __device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0
                     if (p.bias) x += __ldg(p.bias + n + t);
                     if (p.R) x += p.R[m * p.ldr + n + t];
                     if (p.relu) x = fmaxf(x, 0.f);
-                    p.C[m * p.ldc + n + t] = x;
+                    crow[n + t] = x;
                 }
             }
         }
@@ -133,7 +146,7 @@ __device__ __forceinline__ void sgemm_tile(const TileArgs& p, int64_t m0, int n0
 }
 
 __global__ void __launch_bounds__(NTHREADS, 2) sgemm_nt_kernel(TileArgs p) {
-    sgemm_tile(p, (int64_t)blockIdx.x * BM, (int)blockIdx.y * BN);
+    sgemm_tile<false>(p, (int64_t)blockIdx.x * BM, (int)blockIdx.y * BN);
 }
 
 // one z-slice per video: A = the video's query CLS rows, W = the video's context frames
@@ -154,8 +167,8 @@ frame_scores_kernel(const float* __restrict__ ctx, const float* __restrict__ cls
     p.lda = K;
     p.W = ctx + f0 * K;
     p.ldw = K;
-    p.C = score + score_offsets[q0];
-    p.ldc = N;  // every query of this video owns N consecutive scores
+    p.C = score;
+    p.ldc = 0;
     p.bias = nullptr;
     p.R = nullptr;
     p.ldr = 0;
@@ -163,7 +176,7 @@ frame_scores_kernel(const float* __restrict__ ctx, const float* __restrict__ cls
     p.N = N;
     p.K = K;
     p.relu = 0;
-    sgemm_tile(p, m0, n0);
+    sgemm_tile<true>(p, m0, n0, score_offsets + q0);  // query q's N scores start at score_offsets[q]
 }
 
 // tiny-N linear heads: one warp per row

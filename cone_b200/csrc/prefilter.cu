@@ -33,6 +33,13 @@ window_ranklist_kernel(const float* __restrict__ frame_score, const int64_t* __r
     const int stride = max_v_l / 2;
     const int nw = (L + stride - 1) / stride + 1;
     const float* fs = frame_score + score_offsets[q];
+    if (nw > npad) {  // windows past npad cannot enter the sort: no rank-list rather than the best of a prefix
+        for (int i = threadIdx.x; i < ranklist_stride; i += blockDim.x) {
+            ranklist[(int64_t)q * ranklist_stride + i] = -1;
+            if (winscore) winscore[(int64_t)q * ranklist_stride + i] = CUDART_NAN_F;
+        }
+        return;
+    }
     for (int i = threadIdx.x; i < npad; i += blockDim.x) {
         unsigned long long key = ~0ull;
         if (i < nw) {
@@ -43,7 +50,7 @@ window_ranklist_kernel(const float* __restrict__ frame_score, const int64_t* __r
                 m = fs[s];
                 for (int f = s + 1; f < e; ++f) m = nanmax(m, fs[f]);
             }
-            if (winscore) winscore[(int64_t)q * ranklist_stride + i] = m;
+            if (winscore && i < ranklist_stride) winscore[(int64_t)q * ranklist_stride + i] = m;
             key = ((unsigned long long)(~orderable(m)) << 32) | (unsigned)i;
         }
         keys[i] = key;

@@ -313,12 +313,29 @@ class ConeEngine:
         return scores, score_offsets
 
     def window_ranklist(self, frame_score: torch.Tensor, score_offsets: torch.Tensor, frame_count: torch.Tensor,
-                        ranklist_stride: Optional[int] = None, want_scores: bool = False, max_v_l: Optional[int] = None):
-        """Full window rank-list per query from (ragged) frame scores (cone/inference.py:286-299)."""
+                        ranklist_stride: Optional[int] = None, want_scores: bool = False, max_v_l: Optional[int] = None,
+                        max_frame_count: Optional[int] = None):
+        """Full window rank-list per query from (ragged) frame scores (cone/inference.py:286-299).
+
+        An explicit `ranklist_stride` must hold every window of the longest query: it is checked (ValueError) against
+        `max_frame_count` when given, else against `frame_count` when that is a CPU tensor (it is then copied to the
+        device).  A device `frame_count` is not read back; the library writes -1 over the row of a query whose windows
+        do not fit the sort that the stride sizes."""
+        max_v_l = max_v_l or self.cfg.max_v_l
+        if ranklist_stride is not None:
+            longest = max_frame_count
+            if longest is None and not frame_count.is_cuda and frame_count.numel():
+                longest = int(frame_count.max())
+            if longest is not None:
+                need = math.ceil(int(longest) / int(max_v_l / 2)) + 1
+                if ranklist_stride < need:
+                    raise ValueError(f"ranklist_stride {ranklist_stride} is shorter than the rank-list of a {longest}-frame "
+                                     f"video ({need} windows at max_v_l {max_v_l})")
+        if not frame_count.is_cuda:
+            frame_count = frame_count.to(frame_score.device)
         frame_score = _need(frame_score, torch.float32, "frame_score")
         score_offsets = _need(score_offsets, torch.int64, "score_offsets")
         frame_count = _need(frame_count, torch.int32, "frame_count")
-        max_v_l = max_v_l or self.cfg.max_v_l
         nq = frame_count.numel()
         if ranklist_stride is None:
             ranklist_stride = math.ceil(int(frame_count.max().item()) / int(max_v_l / 2)) + 1

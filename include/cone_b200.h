@@ -163,7 +163,8 @@ int cone_encoder_tail(const cone_weights* w, int32_t layer, const float* att, co
  * [n_videos+1] int64 frame offsets; q_first [n_videos+1] int32 = first query of each video;
  * cls_norm [n_queries, Dv] normalised CLS (all device arrays).  max_video_frames /
  * max_video_queries size the launch grid.  score_out is ragged: query q's scores are
- * score_out[score_offsets[q] ... + L_video(q)), score_offsets [n_queries] int64.
+ * score_out[score_offsets[q] ... + L_video(q)), score_offsets [n_queries] int64, per query: rows may be padded or
+ * ordered freely (they must not overlap); nothing outside them is written.
  * Always fp32: the window ranking must be bit-stable (precision is accepted for symmetry). */
 int cone_frame_scores(const float* ctx, int32_t v_dim, const int64_t* video_offsets, const int32_t* q_first,
                       int32_t n_videos, int32_t max_video_frames, int32_t max_video_queries, const float* cls_norm,
@@ -173,6 +174,9 @@ int cone_frame_scores(const float* ctx, int32_t v_dim, const int64_t* video_offs
  * torch.sort orders it).  frame_score ragged as above (device), score_offsets / frame_count
  * [n_queries] device arrays.  ranklist_out [n_queries, ranklist_stride] int32, filled up to
  * num_window(q) = ceil(L/stride)+1, rest -1; winscore_out (nullable) same shape fp32.
+ * ranklist_stride must be >= num_window(q) for every query, and <= 16384 (else CONE_ERR_INVALID).  The sort holds the
+ * next power of two >= ranklist_stride windows: a query with more windows than that gets a row of -1 (winscore NaN),
+ * never the best of a prefix.  The frame counts live on the device, so the first condition is not checked here.
  * Also the parity surface of the function form `compute_window_ranklist`
  * (run_on_video/cone_localizator.py:83-100). */
 int cone_window_ranklist(const float* frame_score, const int64_t* score_offsets, const int32_t* frame_count,
