@@ -17,8 +17,9 @@ namespace {
 // One CTA per (window, slot).  Bounds follow the reference's fp32 operation order exactly:
 //   x1 = cx - 0.5*w ; x2 = cx + 0.5*w                     (span_cxw_to_xx, cone/span_utils.py:39-40)
 //   start = relu(int(floor(x1 * dur))) ; end = int(ceil(x2 * dur))          (model.py:187-192)
-// `feat[start:end]` is a Python slice of the window zero-padded to pad_len rows: `end` clips to pad_len,
-// pad rows inside the slice are averaged in (they are zeros), an empty slice gives NaN.
+// `feat[start:end]` is a Python slice of the window zero-padded to pad_len rows: a negative `end` counts back from
+// pad_len (and stops at 0), `end` clips to pad_len, pad rows inside the slice are averaged in (they are zeros), an empty
+// slice gives NaN.
 template <class T>
 __global__ void __launch_bounds__(256)
 span_mean_pool_kernel(const T* __restrict__ frames, int64_t n_frames, const int64_t* __restrict__ vid_base,
@@ -36,7 +37,8 @@ span_mean_pool_kernel(const T* __restrict__ frames, int64_t n_frames, const int6
     start = start < 0 ? 0 : start;
     int end = (int)ceilf(x2);
     const int pl = pad_len[b];
-    if (end > pl) end = pl;
+    if (end < 0) end += pl;  // a negative end counts back from pad_len, as a Python slice's does
+    end = end < 0 ? 0 : (end > pl ? pl : end);
     const int n = end - start;            // rows in the slice, pad rows included
     const int vend = end < len ? end : len;  // rows that hold data
     const int64_t base = vid_base[b];
@@ -97,7 +99,8 @@ span_mean_pool_window_kernel(const T* __restrict__ frames, int64_t n_frames, con
             int start = (int)floorf(x1);
             start = start < 0 ? 0 : start;
             int end = (int)ceilf(x2);
-            if (end > pl) end = pl;
+            if (end < 0) end += pl;  // a negative end counts back from pad_len, as above
+            end = end < 0 ? 0 : (end > pl ? pl : end);
             cnt[j] = end - start;
             int vend = end < len ? end : len;                                  // rows that hold data
             const int64_t room = n_frames - base;                              // rows past the tensor end: none

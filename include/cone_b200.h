@@ -243,7 +243,8 @@ int cone_forward(const cone_weights* w, const float* src_txt, const int32_t* txt
 
 /* ---- A9  `model.forward_clip_matching(src_cls_txt, src_vid_appear, src_vid_appear_mask,
  * proposal=pred_spans)` (cone/model.py:130-152, 178-210).  src_vid_appear [B, Lv, Dv] zero padded,
- * vid_len [B]; spans [B, nq, 2]; out [B, nq]. */
+ * vid_len [B]; spans [B, nq, 2]; out [B, nq].  Each proposal pools rows feat[start:end] as a Python slice of the Lv
+ * padded rows: a negative end counts back from Lv, an empty slice gives NaN; rows >= vid_len are read as zeros. */
 int cone_clip_matching(const cone_weights* w, const float* src_cls_txt, const float* src_vid_appear,
                        const int32_t* vid_len, const float* spans, int32_t B, int32_t Lv, int32_t nq, float* out,
                        void* workspace, size_t workspace_bytes, int precision, void* stream);

@@ -35,3 +35,25 @@ def clip_matching(sd, cls, vid, vmask, spans, dtype=torch.float64) -> torch.Tens
     c = lambda x: torch.as_tensor(x).to("cpu", dtype)
     with torch.no_grad():
         return O.clip_matching(cast_state_dict(sd, dtype), c(cls), c(vid), c(vmask), c(spans))
+
+
+def pool_slices(vid, start, end) -> torch.Tensor:
+    """[B * nq, Dv] means of `vid[b][start[b, j]:end[b, j]]`, Python slices of the padded rows (a negative end counts back
+    from the padded length; an empty slice gives NaN), in the dtype of `vid`: the pooling lines of `O.clip_matching`."""
+    return torch.vstack([feat[s:e].mean(axis=0) for feat, ss, ee in zip(vid, start, end) for s, e in zip(ss, ee)])
+
+
+def clip_matching_exact_bounds(sd, cls, vid, vmask, spans, dtype=torch.float64) -> torch.Tensor:
+    """`O.clip_matching` with the [start, end) bounds computed as the fp32 reference computes them (`O.proposal_bounds` on
+    the fp32 spans and mask), and the pooling, adapter, normalisation and dot product in `dtype`.  `clip_matching` above
+    casts the spans first, so at a floor/ceil boundary it can pool other rows than the fp32 reference; this one pools the
+    same rows.  In float32 it returns exactly `O.clip_matching`'s bits."""
+    c = lambda x: torch.as_tensor(x).to("cpu", dtype)
+    f32 = lambda x: torch.as_tensor(x).to("cpu", torch.float32)
+    with torch.no_grad():
+        start, end = O.proposal_bounds(f32(spans), f32(vmask))
+        cls = c(cls)
+        t = cls / cls.norm(dim=1, keepdim=True)
+        p = O.adapter(cast_state_dict(sd, dtype), pool_slices(c(vid), start, end)).reshape(*start.shape, -1)
+        p = p / p.norm(dim=2, keepdim=True)
+        return torch.einsum("bld,bd->bl", p, t)

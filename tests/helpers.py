@@ -268,3 +268,78 @@ def dense_batch(cfg, lv, lt, seed):
         app[i, vlen[i]:] = 0
         txt[i, tlen[i]:] = 0
     return mot, app, vm, txt, tm, cls
+
+
+# ---- proposals at the pooling edges of A9 (tests/test_matching.py on the CPU, tests/test_gpu_matching.py on the GPU) ----
+def span_products(spans, dur):
+    """fp32 (x1 * dur, x2 * dur) of proposals (cx, w), in the operation order of `O.proposal_bounds`."""
+    import torch
+    from oracle import cone_oracle as O
+    xx = O.span_cxw_to_xx(torch.as_tensor(np.asarray(spans, np.float32))) * torch.tensor(float(dur), dtype=torch.float32)
+    return xx[..., 0].numpy(), xx[..., 1].numpy()
+
+
+def boundary_spans(dur, ks=(1, 3, 6), a_values=None, n_ulps=8, reach=4096):
+    """fp32 proposals whose floor(x1 * dur) or ceil(x2 * dur) sits on an integer boundary: exact widths w = 2^-k, and cx
+    scanned over +-n_ulps ulps (np.nextafter) around a/dur + w/2 (x1 * dur near the integer a) and a/dur - w/2
+    (x2 * dur near a), then at +-16, 32, ... `reach` ulps: where dur times an ulp of x is below an ulp of a, several cx
+    give the same product, and the wider steps reach the products on both sides of it.
+    Returns (spans [M, 2] float32, group [M]): each group is one scan, in increasing cx."""
+    if a_values is None:
+        a_values = sorted({0, 1, dur // 2, dur - 1, dur})
+    spans, group = [], []
+    for k in ks:
+        w = np.float32(2.0 ** -k)
+        for a in a_values:
+            for sign in (1, -1):
+                c = np.float32(a / dur + sign * float(w) / 2)
+                lo, hi = [c], [c]
+                dn, up = c, c
+                for i in range(1, reach + 1):
+                    dn, up = np.nextafter(dn, np.float32(-np.inf)), np.nextafter(up, np.float32(np.inf))
+                    if i <= n_ulps or (i & (i - 1)) == 0:
+                        lo.append(dn)
+                        hi.append(up)
+                cx = np.asarray(lo[::-1] + hi[1:], np.float32)
+                spans.append(np.stack([cx, np.full_like(cx, w)], 1))
+                group.append(np.full(len(cx), len(group)))
+    return np.concatenate(spans).astype(np.float32), np.concatenate(group)
+
+
+def boundary_hits(spans, group, dur):
+    """Indices of the proposals of `boundary_spans` whose x1 * dur or x2 * dur is an exact fp32 integer, and of their
+    scan neighbours (one cx ulp away), which miss it."""
+    x1, x2 = span_products(spans, dur)
+    exact = (x1 == np.floor(x1)) | (x2 == np.floor(x2))
+    keep = exact.copy()
+    for i in np.nonzero(exact)[0]:
+        for j in (i - 1, i + 1):
+            if 0 <= j < len(spans) and group[j] == group[i]:
+                keep[j] = True
+    return np.nonzero(keep)[0]
+
+
+def edge_spans(dur, pad, seed):
+    """fp32 proposals of one window of `dur` data rows zero padded to `pad` rows, at every edge of the pooling: random
+    spans, x1 < 0, ends past `dur` inside the pad, ends past `pad`, empty slices (w = 0 on an integer), start >= pad,
+    negative ends (-1, -pad, -pad - 1, -0.0), a negative width, NaN, and the floor/ceil boundary spans of
+    `boundary_spans` (exact hits and their 1-ulp misses)."""
+    rng = np.random.default_rng(seed)
+    d = float(max(dur, 1))
+    neg_end = lambda e: ((e - 0.5) / d, 0.0)  # x1 = x2 = (e - 0.5) / dur: start 0, end e
+    x2_in_pad = (dur + pad) / 2 / d  # [0.5 dur, (dur + pad) / 2)
+    rows = [(0.05, 0.5), (0.1, 0.9), (-0.2, 0.3),  # x1 < 0
+            ((0.5 + x2_in_pad) / 2, x2_in_pad - 0.5),  # end past dur, inside the pad
+            (pad / d, 1.0), (2.0 * pad / d, 0.5), (0.9, 0.6),  # end past pad
+            (0.0, 0.0), (1.0, 0.0), (0.5, 0.0),  # empty slices
+            (3.0 * pad / d + 0.1, 0.1), (pad / d + 0.5 / d, 1.0 / d),  # start >= pad
+            neg_end(-1), neg_end(-pad), neg_end(-pad - 1), (-0.4 / d, 0.0), (-0.5, 0.4), (0.3, -0.8),  # negative ends
+            (0.5, -1.5),  # negative width: start > 0 > end
+            (np.nan, 0.3), (0.5, np.nan), (np.nan, np.nan)]
+    sp = [np.asarray(rows, np.float32),
+          rng.uniform(0, 1, (12, 2)).astype(np.float32),
+          np.stack([rng.uniform(-0.3, 1.3, 8), rng.uniform(0, 1.2, 8)], 1).astype(np.float32)]
+    if dur > 0:
+        b, g = boundary_spans(dur, ks=(1, 6), a_values=sorted({0, 1, dur // 2, dur}))
+        sp.append(b[boundary_hits(b, g, dur)])
+    return np.concatenate(sp).astype(np.float32)
